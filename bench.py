@@ -24,13 +24,19 @@ Keys beyond the base contract:
                image) timed on this host, bounded sample.
   e2e          same metric through the public host API (`mynimize_repeated` with HOST buffers):
                pinned H2D of the initial angles and D2H of the result arrays inside the timing.
+
+--dump-outputs DIR writes what the last timed step computed (the AdamState arrays a caller of `adam_run`
+receives) for a fixed, seeded sample of the samples, one DIR/<name>.npy per array, so that two builds run with
+the same arguments can be compared output for output.
 """
 import argparse
 import json
+import math
 import os
 import statistics
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
@@ -41,6 +47,9 @@ METRIC = "loss+grad evals/sec (4q Toffoli, 40 CP gates)"
 UNIT = "evals/s"
 R_WEIGHT = 0.001476          # the reference's stored K=40 trial point (SURVEY.md §8d C3)
 LR = 0.1
+# --dump-outputs: the AdamState arrays written, and the byte budget that bounds the sampled rows (48 MiB)
+DUMP_FIELDS = ("angles", "best_params", "best_regloss", "best_reg", "init_regloss", "init_reg")
+DUMP_BYTES = 48 << 20
 
 
 def parse():
@@ -61,7 +70,13 @@ def parse():
     ap.add_argument("--no-extras", action="store_true", help="skip the complex128 / 5-qubit / other-loss roofline extras")
     ap.add_argument("--cpu-samples", type=int, default=1024)
     ap.add_argument("--cpu-iters", type=int, default=30)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write a seeded sample of the last timed step's results to DIR/<name>.npy")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "b200":
+        ap.error("--dump-outputs writes the CUDA engine's results: it needs --impl b200")
     if a.samples_per_gpu is not None:
         a.scaling, a.samples = "weak", a.samples_per_gpu
     return a
@@ -204,10 +219,12 @@ def measure_fp32_peak():
     exe = os.path.join(ROOT, "tools", "fp32_peak")
     src = exe + ".cu"
     try:
-        if not os.path.exists(exe):
-            subprocess.run(["nvcc", "-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-o", exe, src],
-                           check=True, capture_output=True)
-        out = subprocess.run([exe, "--quick"], capture_output=True, text=True, timeout=120).stdout
+        with tempfile.TemporaryDirectory() as tmp:
+            if not os.path.exists(exe):     # the tree may be read-only: compile a private copy instead
+                exe = os.path.join(tmp, "fp32_peak")
+                subprocess.run(["nvcc", "-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-o", exe, src],
+                               check=True, capture_output=True)
+            out = subprocess.run([exe, "--quick"], capture_output=True, text=True, timeout=120).stdout
         best = {}
         for ln in out.splitlines():
             if ln.startswith("{"):
@@ -334,6 +351,26 @@ def other_rooflines(peak_tf, peak_detail):
     return out
 
 
+def dump_outputs(out_dir, st, first, B, B_total, world, rank):
+    """DIR/<field>.npy for every DUMP_FIELDS array of `st`, restricted to a seeded sample of global sample indices
+    (ascending), so that the rows are the same for any split of the batch over ranks.  Rank 0 gathers and writes."""
+    import numpy as np
+    import torch
+    import torch.distributed as dist
+    row_bytes = sum(getattr(st, f).element_size() * math.prod(getattr(st, f).shape[1:]) for f in DUMP_FIELDS)
+    idx = np.sort(np.random.default_rng(0).choice(B_total, min(B_total, DUMP_BYTES // row_bytes), replace=False))
+    rows = torch.as_tensor(idx[(idx >= first) & (idx < first + B)] - first, device=st.angles.device)
+    parts = [{f: getattr(st, f).index_select(0, rows).cpu().numpy() for f in DUMP_FIELDS}]
+    if world > 1:
+        gathered = [None] * world
+        dist.all_gather_object(gathered, parts[0])
+        parts = gathered
+    if rank == 0:
+        os.makedirs(out_dir, exist_ok=True)
+        for f in DUMP_FIELDS:
+            np.save(os.path.join(out_dir, f + ".npy"), np.concatenate([p[f] for p in parts]))
+
+
 def run_b200(args):
     import numpy as np
     import torch
@@ -436,6 +473,8 @@ def run_b200(args):
     best = st.best_regloss
     assert bool(torch.isfinite(best).all()) and bool((best <= st.init_regloss).all())
     frac_converged = float((best - st.best_reg < 1e-3).float().mean())
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, st, first, B, B_total, world, rank)
 
     # ---- e2e: the public host API with HOST buffers (pinned H2D of inputs, D2H of results) ----
     a0_host = a0.cpu().pin_memory()

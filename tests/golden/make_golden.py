@@ -1,8 +1,8 @@
 """Extract known-answer fixtures from the reference's stored result files.
 
-Run ONCE in the build container (where /root/reference exists):
+Run once, given a checkout of the reference project (argument, or CPFLOW_REFERENCE_DIR):
 
-    python tests/golden/make_golden.py
+    python tests/golden/make_golden.py /path/to/cpflow
 
 It reads cpflow's dill `Results` pickles (paper/results, paper/results/benchmarks,
 tutorial/results — SURVEY.md §4.3 / Appendix A) with the stub unpickler and writes small,
@@ -15,7 +15,7 @@ dependency-free fixtures next to this file:
 * ``trials.json`` — hyperopt trial records (num_cp_gates, r, random_seed, cz_counts) used as
   statistical pins and as threefry `split` known answers (main.py:741-749, 798-799).
 
-Nothing at test time reads /root/reference; only these committed fixtures are used.
+Nothing at test time reads the reference checkout; only these committed fixtures are used.
 """
 import glob
 import json
@@ -28,7 +28,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, HERE)
 import stub_unpickle as su  # noqa: E402
 
-REF = "/root/reference"
+REF = sys.argv[1] if len(sys.argv) > 1 else os.environ.get("CPFLOW_REFERENCE_DIR", "")
 FILES = (sorted(glob.glob(f"{REF}/tutorial/results/*"))
          + sorted(f for f in glob.glob(f"{REF}/paper/results/*") if os.path.isfile(f))
          + sorted(glob.glob(f"{REF}/paper/results/benchmarks/*")))
@@ -93,6 +93,8 @@ def circuit_gates(circ):
 
 
 def main():
+    if not (REF and os.path.isdir(os.path.join(REF, "tutorial", "results"))):
+        raise SystemExit("usage: make_golden.py /path/to/cpflow  (a checkout of the reference project)")
     ans_meta, ans_arrays = [], {}
     gl_meta, gl_arrays = [], {}
     trials_out = {}

@@ -1,7 +1,7 @@
 """cpflow_b200.legacy: reading the reference's stored `Results` files (SURVEY.md §8f N5) without cpflow, qiskit,
 hyperopt, jax or dill.  CPU only.  The first test builds a file with the reference's class paths from scratch;
-the second reads the reference's own files when the reference tree is mounted (build container) and checks them
-against the committed golden fixtures."""
+the second reads the reference's own files when CPFLOW_REFERENCE_DIR names a checkout of the reference project
+(the files are not part of this repository) and checks them against the committed golden fixtures."""
 import json
 import os
 import pickle
@@ -15,7 +15,7 @@ from cpflow_b200.legacy import load_reference_results
 from oracle import cpflow_oracle as O
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = "/root/reference"
+REF = os.environ.get("CPFLOW_REFERENCE_DIR", "")
 
 
 def _fake_class(path):
@@ -103,7 +103,8 @@ def test_rejects_other_pickles(tmp_path):
         load_reference_results(str(p))
 
 
-@pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "tutorial", "results")), reason="reference tree not mounted")
+@pytest.mark.skipif(not (REF and os.path.isdir(os.path.join(REF, "tutorial", "results"))),
+                    reason="CPFLOW_REFERENCE_DIR does not name a checkout of the reference project")
 def test_reference_files_against_golden_fixtures():
     """Every stored file loads; trials match tests/golden/trials.json; the stored circuits reproduce their stored
     unitaries up to a global phase (the property tests/golden/gatelist_kats pins for a subset; a few refined
