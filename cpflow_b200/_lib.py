@@ -53,6 +53,10 @@ class CpfAdamBuffers(C.Structure):
                 ("workspace_bytes", C.c_int64)]
 
 
+class CpfTargetTable(C.Structure):
+    _fields_ = [("kind", C.c_int32), ("n_targets", C.c_int32), ("targets", C.c_void_p), ("target_index", C.c_void_p)]
+
+
 EXPORTS = {
     "cpf_version": (C.c_int, []),
     "cpf_last_error": (C.c_char_p, []),
@@ -68,6 +72,13 @@ EXPORTS = {
                                C.POINTER(CpfAdamSpec), C.c_int32, C.c_int64, C.c_int64, C.c_int64,
                                C.POINTER(CpfAdamBuffers), C.c_void_p]),
     "cpf_workspace_bytes": (C.c_int, [C.c_void_p, C.c_int32, C.c_int32, C.c_int64, C.POINTER(C.c_int64)]),
+    "cpf_loss_grad_multi": (C.c_int, [C.c_void_p, C.POINTER(CpfTargetTable), C.POINTER(CpfPenaltySpec), C.c_int32,
+                                      C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "cpf_adam_run_multi": (C.c_int, [C.c_void_p, C.POINTER(CpfTargetTable), C.POINTER(CpfPenaltySpec),
+                                     C.POINTER(CpfAdamSpec), C.c_int32, C.c_int64, C.c_int64, C.c_int64,
+                                     C.POINTER(CpfAdamBuffers), C.c_void_p]),
+    "cpf_workspace_bytes_multi": (C.c_int, [C.c_void_p, C.c_int32, C.c_int32, C.c_int64, C.c_int32,
+                                            C.POINTER(C.c_int64)]),
     "cpf_adam_step": (C.c_int, [C.c_void_p, C.POINTER(CpfPenaltySpec), C.POINTER(CpfAdamSpec), C.c_int32, C.c_int64,
                                 C.c_int64, C.c_void_p, C.c_void_p, C.POINTER(CpfAdamBuffers), C.c_void_p]),
     "cpf_count_cz": (C.c_int, [C.c_void_p, C.c_int32, C.c_int64, C.c_void_p, C.c_double, C.c_void_p,

@@ -249,6 +249,9 @@ void heis_scratch_sizes(const cpf::Program* prog, int64_t batch, size_t* target_
 }
 
 template <typename R>
+int stage_heis_state(const cpf::Program* prog, cpf::KParams<R>& p, Scratch& sc);
+
+template <typename R>
 int stage_heis(const cpf::Program* prog, const cpf_loss_spec* loss, cpf::KParams<R>& p, Scratch& sc) {
   cudaStream_t st = sc.st;
   if (!sc.base) keep_pool_memory();
@@ -256,21 +259,30 @@ int stage_heis(const cpf::Program* prog, const cpf_loss_spec* loss, cpf::KParams
   const int words = cpf::heis_target_words<R>(prog->n_qubits, cpt);
   size_t bytes, aux_pad, pk_bytes;
   heis_scratch_sizes<R>(prog, p.B, &bytes, &aux_pad, &pk_bytes);
-  R* packed_v = nullptr; R* aux_v = nullptr;
-  R** packed = &packed_v; R** aux = &aux_v;
-  int rc = sc.get((void**)packed, bytes);
+  R* packed = nullptr;
+  int rc = sc.get((void**)&packed, bytes);
   if (rc) return rc;
-  if (bytes != (size_t)words * sizeof(R)) CPF_CUDA(cudaMemsetAsync(*packed, 0, bytes, st));
-  rc = cpf::launch_pack_target_heis<R>((const R*)loss->target, *packed, prog->n_qubits, cpt, st);
+  if (bytes != (size_t)words * sizeof(R)) CPF_CUDA(cudaMemsetAsync(packed, 0, bytes, st));
+  rc = cpf::launch_pack_target_heis<R>((const R*)loss->target, packed, prog->n_qubits, cpt, st);
   if (rc) return fail(rc, "pack_target_heis launch failed");
-  // one block: per-gate scratch, then the packed optimiser state (32-byte aligned)
-  rc = sc.get((void**)aux, aux_pad + pk_bytes);
-  if (rc) return rc;
-  p.pk = reinterpret_cast<char*>(*aux) + aux_pad;
-  p.target_packed = *packed;
+  p.target_packed = packed;
   p.target_bytes = (int)bytes;
   p.loss_kind = loss->kind;
-  p.aux = *aux;
+  return stage_heis_state(prog, p, sc);
+}
+
+// the target-independent part of the heis set-up: per-gate scratch and packed optimiser state, gate-pattern flags
+template <typename R>
+int stage_heis_state(const cpf::Program* prog, cpf::KParams<R>& p, Scratch& sc) {
+  const int cpt = cpf::heis_cpt<R>(prog->n_qubits);
+  size_t bytes, aux_pad, pk_bytes;
+  heis_scratch_sizes<R>(prog, p.B, &bytes, &aux_pad, &pk_bytes);
+  R* aux = nullptr;
+  // one block: per-gate scratch, then the packed optimiser state (32-byte aligned)
+  int rc = sc.get((void**)&aux, aux_pad + pk_bytes);
+  if (rc) return rc;
+  p.pk = reinterpret_cast<char*>(aux) + aux_pad;
+  p.aux = aux;
   // rotation-axis pattern shared by the surface gates (slots < n) and by the block gates (the rest)
   auto pattern = [&](size_t lo, size_t hi) {
     int pat = -1;
@@ -310,6 +322,76 @@ int check_loss(const cpf_loss_spec* loss) {
   return CPF_OK;
 }
 
+// Everything a multi-target call needs to know is checked here, before any CUDA call.
+int check_table(const cpf::Program* prog, const cpf_target_table* tt, int64_t batch) {
+  if (!tt) return fail(CPF_ERR_INVALID, "target table is NULL");
+  if (tt->kind < CPF_LOSS_HS || tt->kind > CPF_LOSS_RELPHASE) return fail(CPF_ERR_INVALID, "unknown loss kind");
+  if (tt->n_targets < 1) return fail(CPF_ERR_INVALID, "target table: n_targets must be >= 1");
+  if (!tt->targets) return fail(CPF_ERR_INVALID, "target table: targets is NULL");
+  if (batch > 0 && !tt->target_index) return fail(CPF_ERR_INVALID, "target table: target_index is NULL");
+  if (tt->kind != CPF_LOSS_STATE && prog->n_qubits > 5)
+    return fail(CPF_ERR_UNSUPPORTED, "full-unitary losses need n <= 5 qubits (6-7 qubits: state preparation and "
+                                     "cpf_unitary only)");
+  for (int64_t b = 0; b < batch; ++b) {
+    const int32_t t = tt->target_index[b];
+    if (t < 0 || t >= tt->n_targets)
+      return fail(CPF_ERR_INVALID, "target_index[" + std::to_string(b) + "] = " + std::to_string(t) +
+                                       " is outside [0, n_targets = " + std::to_string(tt->n_targets) + ")");
+  }
+  return CPF_OK;
+}
+
+// bytes of the multi-target table of the kernel a call runs on (targets back to back in the kernel's packed layout)
+template <typename R>
+size_t multi_table_bytes(const cpf::Program* prog, int32_t kind, bool heis, int32_t n_targets) {
+  const bool single = kind == CPF_LOSS_STATE;
+  const int n = prog->n_qubits;
+  const int words = heis ? cpf::heis_target_words<R>(n, cpf::heis_cpt<R>(n))
+                         : cpf::target_words<R>(n, single ? 1 : cpf::cpt_for<R>(n), single);
+  return (size_t)n_targets * (size_t)words * sizeof(R);
+}
+
+// Multi-target staging: the index array (host, checked by check_table) goes to the device, all targets are packed in
+// one launch; the kernels read both from global memory (p.target_bytes = 0: no shared-memory copy).
+template <typename R>
+int stage_multi(const cpf::Program* prog, const cpf_target_table* tt, cpf::KParams<R>& p, bool heis, Scratch& sc) {
+  cudaStream_t st = sc.st;
+  if (heis && !sc.base) keep_pool_memory();
+  const bool single = tt->kind == CPF_LOSS_STATE;
+  const int n = prog->n_qubits;
+  int32_t* idx = nullptr;
+  R* table = nullptr;
+  int rc = sc.get((void**)&idx, (size_t)p.B * sizeof(int32_t));
+  if (!rc) rc = sc.get((void**)&table, multi_table_bytes<R>(prog, tt->kind, heis, tt->n_targets));
+  if (rc) return rc;
+  // pageable source: the runtime stages the bytes before returning
+  CPF_CUDA(cudaMemcpyAsync(idx, tt->target_index, (size_t)p.B * sizeof(int32_t), cudaMemcpyHostToDevice, st));
+  rc = heis ? cpf::launch_pack_targets_heis<R>((const R*)tt->targets, table, n, cpf::heis_cpt<R>(n), tt->n_targets, st)
+            : cpf::launch_pack_targets<R>((const R*)tt->targets, table, n, single ? 1 : cpf::cpt_for<R>(n), single,
+                                          tt->n_targets, st);
+  if (rc) return fail(rc, "pack_targets launch failed");
+  p.target_packed = table;
+  p.target_bytes = 0;
+  p.target_index = idx;
+  p.loss_kind = tt->kind;
+  return heis ? stage_heis_state(prog, p, sc) : CPF_OK;
+}
+
+// Launch of a staged call: the single-target kernels, or (table != NULL) their multi-target variants.
+template <typename R>
+int launch_staged(const cpf::KParams<R>& p, const cpf::Program* prog, const cpf_target_table* table, bool heis,
+                  bool single, cudaStream_t st, std::string& err) {
+  int rc = CPF_OK;
+  if (table) {
+    if (heis) cpf::launch_heis_multi<R>(p, *prog, st, err, rc);
+    else rc = cpf::launch_engine_multi<R>(p, prog->n_qubits, single, st, err);
+  } else {
+    if (heis) cpf::launch_heis<R>(p, *prog, st, err, rc, false);
+    else rc = launch_any<R>(p, prog, single, st, err);
+  }
+  return rc;
+}
+
 template <typename R>
 int run_unitary(const cpf::Program* prog, int64_t batch, const void* angles, void* u_out, cudaStream_t st) {
   cpf::KParams<R> p;
@@ -325,10 +407,11 @@ int run_unitary(const cpf::Program* prog, int64_t batch, const void* angles, voi
   return rc ? fail(rc, err) : CPF_OK;
 }
 
+// table != NULL: multi-target call (loss->kind = table->kind, loss->target unused)
 template <typename R>
 int run_loss_grad(const cpf::Program* prog, const cpf_loss_spec* loss, const cpf_penalty_spec* pen,
                   int64_t batch, const void* angles, void* loss_out, void* reg_out, void* grad_out,
-                  cudaStream_t st) {
+                  cudaStream_t st, const cpf_target_table* table = nullptr) {
   cpf::KParams<R> p;
   const bool single = loss->kind == CPF_LOSS_STATE;
   int rc = fill_common(prog, p, batch, single);
@@ -339,15 +422,15 @@ int run_loss_grad(const cpf::Program* prog, const cpf_loss_spec* loss, const cpf
   sc.st = st;
   const bool heis = use_heis<R>(prog, loss) && (unsigned long long)batch * (unsigned long long)prog->n_params < (1ull << 32);
   rc = fill_penalty(prog, pen, p, sc);
-  if (!rc) rc = heis ? stage_heis(prog, loss, p, sc) : stage_target(prog, loss, p, single, sc);
+  if (!rc && table) rc = stage_multi(prog, table, p, heis, sc);
+  else if (!rc) rc = heis ? stage_heis(prog, loss, p, sc) : stage_target(prog, loss, p, single, sc);
   if (!rc && grad_out) {
     cudaError_t e = cudaMemsetAsync(grad_out, 0, (size_t)batch * prog->n_params * sizeof(R), st);
     if (e != cudaSuccess) rc = cuda_fail("cudaMemsetAsync(grad)", e);
   }
   std::string err;
   if (!rc) {
-    if (heis) cpf::launch_heis<R>(p, *prog, st, err, rc, false);
-    else rc = launch_any<R>(p, prog, single, st, err);
+    rc = launch_staged<R>(p, prog, table, heis, single, st, err);
     if (rc) fail(rc, err);
   }
   return rc;
@@ -370,7 +453,7 @@ int run_cotangent(const cpf::Program* prog, int64_t batch, const void* angles, c
 template <typename R>
 int run_adam(const cpf::Program* prog, const cpf_loss_spec* loss, const cpf_penalty_spec* pen,
              const cpf_adam_spec* adam, int64_t batch, int64_t step0, int64_t num_steps,
-             const cpf_adam_buffers* buf, cudaStream_t st) {
+             const cpf_adam_buffers* buf, cudaStream_t st, const cpf_target_table* table = nullptr) {
   cpf::KParams<R> p;
   const bool single = loss->kind == CPF_LOSS_STATE;
   int rc = fill_common(prog, p, batch, single);
@@ -392,11 +475,11 @@ int run_adam(const cpf::Program* prog, const cpf_loss_spec* loss, const cpf_pena
   }
   const bool heis = use_heis<R>(prog, loss) && (unsigned long long)batch * (unsigned long long)prog->n_params < (1ull << 32);
   rc = fill_penalty(prog, pen, p, sc);
-  if (!rc) rc = heis ? stage_heis(prog, loss, p, sc) : stage_target(prog, loss, p, single, sc);
+  if (!rc && table) rc = stage_multi(prog, table, p, heis, sc);
+  else if (!rc) rc = heis ? stage_heis(prog, loss, p, sc) : stage_target(prog, loss, p, single, sc);
   std::string err;
   if (!rc) {
-    if (heis) cpf::launch_heis<R>(p, *prog, st, err, rc, false);
-    else rc = launch_any<R>(p, prog, single, st, err);
+    rc = launch_staged<R>(p, prog, table, heis, single, st, err);
     if (rc) fail(rc, err);
   }
   return rc;
@@ -417,6 +500,22 @@ int64_t workspace_bytes_t(const cpf::Program* prog, int32_t loss_kind, int64_t b
   } else {
     const int cpt = single ? 1 : cpf::cpt_for<R>(prog->n_qubits);
     total += Scratch::align((((size_t)cpf::target_words<R>(prog->n_qubits, cpt, single) * sizeof(R)) + 15) & ~(size_t)15);
+  }
+  return (int64_t)total;
+}
+
+template <typename R>
+int64_t workspace_bytes_multi_t(const cpf::Program* prog, int32_t loss_kind, int64_t batch, int32_t n_targets) {
+  cpf_loss_spec ls{};
+  ls.kind = loss_kind;
+  const bool heis = use_heis<R>(prog, &ls) && (unsigned long long)batch * (unsigned long long)prog->n_params < (1ull << 32);
+  size_t total = Scratch::align(prog->cp.empty() ? 1 : prog->cp.size());          // penalty mask
+  total += Scratch::align((size_t)batch * sizeof(int32_t));                         // target_index
+  total += Scratch::align(multi_table_bytes<R>(prog, loss_kind, heis, n_targets));  // target table
+  if (heis) {
+    size_t tb, ap, pk;
+    heis_scratch_sizes<R>(prog, batch, &tb, &ap, &pk);
+    total += Scratch::align(ap + pk);
   }
   return (int64_t)total;
 }
@@ -819,6 +918,53 @@ int cpf_workspace_bytes(const cpf_program* prog, int32_t loss_kind, int32_t dtyp
   if (loss_kind < CPF_LOSS_HS || loss_kind > CPF_LOSS_RELPHASE) return fail(CPF_ERR_INVALID, "unknown loss kind");
   const cpf::Program* p = reinterpret_cast<const cpf::Program*>(prog);
   *bytes = dtype == CPF_F64 ? workspace_bytes_t<double>(p, loss_kind, batch) : workspace_bytes_t<float>(p, loss_kind, batch);
+  return CPF_OK;
+}
+
+int cpf_loss_grad_multi(const cpf_program* prog, const cpf_target_table* table, const cpf_penalty_spec* penalty,
+                        int32_t dtype, int64_t batch, const void* angles, void* loss_out, void* reg_out,
+                        void* grad_out, void* stream) {
+  if (!prog || batch < 0) return fail(CPF_ERR_INVALID, "NULL program / bad batch");
+  const cpf::Program* p = reinterpret_cast<const cpf::Program*>(prog);
+  int rc = check_table(p, table, batch);
+  if (rc) return rc;
+  if (batch == 0) return CPF_OK;
+  if (!loss_out) return fail(CPF_ERR_INVALID, "loss_out is NULL");
+  if (!angles && p->n_params > 0) return fail(CPF_ERR_INVALID, "angles is NULL");
+  const cpf_loss_spec loss{table->kind, table->targets};
+  CPF_DISPATCH(dtype, (run_loss_grad<R>(p, &loss, penalty, batch, angles, loss_out, reg_out, grad_out,
+                                        (cudaStream_t)stream, table)));
+}
+
+int cpf_adam_run_multi(const cpf_program* prog, const cpf_target_table* table, const cpf_penalty_spec* penalty,
+                       const cpf_adam_spec* adam, int32_t dtype, int64_t batch, int64_t step0, int64_t num_steps,
+                       const cpf_adam_buffers* buf, void* stream) {
+  if (!prog || !adam || !buf || batch < 0 || step0 < 0 || num_steps < 0)
+    return fail(CPF_ERR_INVALID, "NULL argument / negative size");
+  const cpf::Program* p = reinterpret_cast<const cpf::Program*>(prog);
+  int rc = check_table(p, table, batch);
+  if (rc) return rc;
+  if (batch == 0 || num_steps == 0) return CPF_OK;
+  if (!buf->angles || !buf->m || !buf->v || !buf->best_params || !buf->best_regloss || !buf->best_reg ||
+      !buf->init_regloss || !buf->init_reg)
+    return fail(CPF_ERR_INVALID, "a required cpf_adam_buffers pointer is NULL");
+  if ((buf->hist_params || buf->hist_regloss) && buf->hist_len <= 0)
+    return fail(CPF_ERR_INVALID, "history buffers given with hist_len <= 0");
+  if (num_steps > 2000000000LL) return fail(CPF_ERR_INVALID, "num_steps too large");
+  const cpf_loss_spec loss{table->kind, table->targets};
+  CPF_DISPATCH(dtype, (run_adam<R>(p, &loss, penalty, adam, batch, step0, num_steps, buf, (cudaStream_t)stream,
+                                   table)));
+}
+
+int cpf_workspace_bytes_multi(const cpf_program* prog, int32_t loss_kind, int32_t dtype, int64_t batch,
+                              int32_t n_targets, int64_t* bytes) {
+  if (!prog || !bytes || batch < 0) return fail(CPF_ERR_INVALID, "NULL argument / negative batch");
+  if (loss_kind < CPF_LOSS_HS || loss_kind > CPF_LOSS_RELPHASE) return fail(CPF_ERR_INVALID, "unknown loss kind");
+  if (n_targets < 1) return fail(CPF_ERR_INVALID, "n_targets must be >= 1");
+  if (dtype != CPF_F32 && dtype != CPF_F64) return fail(CPF_ERR_INVALID, "unknown dtype");
+  const cpf::Program* p = reinterpret_cast<const cpf::Program*>(prog);
+  *bytes = dtype == CPF_F64 ? workspace_bytes_multi_t<double>(p, loss_kind, batch, n_targets)
+                            : workspace_bytes_multi_t<float>(p, loss_kind, batch, n_targets);
   return CPF_OK;
 }
 

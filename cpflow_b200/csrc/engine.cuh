@@ -76,6 +76,9 @@ struct KParams {
   int pk_stride;                // heis_kernel: words of R per sample in the packed optimiser state (heis_pk_stride)
   int last_slot[8];             // heis_kernel: slot of the last fused gate on each qubit
   PenaltyT<R> pen;
+  // multi-target kernels (sweep types with MULTI_TARGET, engine_impl.cuh): device [B], sample b is scored against the
+  // packed target target_index[b] of the table at target_packed (nothing is staged: target_bytes = 0)
+  const int32_t* target_index;
 };
 
 // ------------------------------------------------------------------------------------------

@@ -1,5 +1,7 @@
 // Kernel body of the cpflow_b200 engine (see engine.cuh for the design notes).
 #pragma once
+#include <type_traits>
+
 #include "engine.cuh"
 
 namespace cpf {
@@ -107,6 +109,15 @@ __host__ __device__ constexpr int min_blocks() {
   CPF_PH_CASE(10, __VA_ARGS__) CPF_PH_CASE(12, __VA_ARGS__) CPF_PH_CASE(16, __VA_ARGS__)            \
   CPF_PH_CASE(17, __VA_ARGS__) CPF_PH_CASE(18, __VA_ARGS__) CPF_PH_CASE(20, __VA_ARGS__)            \
   CPF_PH_CASE(24, __VA_ARGS__)
+
+// Multi-target (MT) kernels are the instantiations whose sweep type declares MULTI_TARGET = true (InterpSweepMT,
+// heis_impl.cuh: HeisSweepAnyMT).  Sample b then reads its packed target, through L1 / L2, from the table at
+// p.target_packed (targets back to back, each in the single-target packed layout) at entry p.target_index[b]; nothing
+// is staged in shared memory.  Carrying the switch in the sweep type keeps the single-target kernels' names and code.
+template <typename S, typename = void>
+struct IsMultiTarget { static constexpr bool value = false; };
+template <typename S>
+struct IsMultiTarget<S, std::void_t<decltype(S::MULTI_TARGET)>> { static constexpr bool value = S::MULTI_TARGET; };
 
 // ------------------------------------------------------------------------------------------
 // Sweepers: how the forward and the adjoint sweep walk the gate schedule.
@@ -229,6 +240,11 @@ struct InterpSweep {
     }
   }
   }
+};
+
+template <typename R, int NQ, int RB, int CPT, bool SINGLE>
+struct InterpSweepMT : InterpSweep<R, NQ, RB, CPT, SINGLE> {
+  static constexpr bool MULTI_TARGET = true;
 };
 
 // Layered template: surface SU2 gate on every qubit (slot q), then K blocks; block k acts on the
@@ -399,6 +415,7 @@ engine_kernel(const KParams<R> p) {
   using T = VT<R, CPT>;
   using V = typename T::V;
   constexpr int N = C::N, TPS = C::TPS, SPB = C::SPB, LB = C::LB, NA = C::NA;
+  constexpr bool MT = IsMultiTarget<SW>::value;
 
   extern __shared__ __align__(16) unsigned char smem_raw[];
   __shared__ __align__(8) uint64_t s_bar;
@@ -408,7 +425,7 @@ engine_kernel(const KParams<R> p) {
   R* s_coef = reinterpret_cast<R*>(s_red + 8 * p.n_red);
 
   const int tid = threadIdx.x;
-  const bool need_target = p.mode == M_ADAM || p.mode == M_LOSSGRAD;
+  const bool need_target = !MT && (p.mode == M_ADAM || p.mode == M_LOSSGRAD);
 
   // ---- prologue: TMA-stage the target, copy the decoded schedule and the reduce tables ----
   if (need_target) {
@@ -442,7 +459,9 @@ engine_kernel(const KParams<R> p) {
   const int P = p.P;
   R* coef = s_coef + (size_t)sl * p.coef_stride;
   R* coef_cp = coef + 8 * p.n_su2;
-  const V* tv = reinterpret_cast<const V*>(s_target) + 2 * ((SINGLE ? 0 : cg * (N + 1)) + (la << RB));
+  const R* tgt = s_target;
+  if constexpr (MT) tgt = p.target_packed + (size_t)p.target_index[b] * (size_t)((SINGLE ? 1 : N / CPT) * (N + 1) * 2 * CPT);
+  const V* tv = reinterpret_cast<const V*>(tgt) + 2 * ((SINGLE ? 0 : cg * (N + 1)) + (la << RB));
 
   R* ang = p.angles + bs * P;   // M_LOSSGRAD/UNITARY/COTANGENT: read-only use
   R* mom = p.m ? p.m + b * P : nullptr;
@@ -677,6 +696,27 @@ __global__ void pack_target_kernel(const R* __restrict__ src, R* __restrict__ ds
                                    int single) {
   const int groups = single ? 1 : N / cpt;
   const int total = groups * (N + 1) * 2 * cpt;
+  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < total; i += gridDim.x * blockDim.x) {
+    int k = i % cpt, r = i / cpt;
+    int part = r % 2; r /= 2;
+    int j = r % (N + 1), cg = r / (N + 1);
+    R val = R(0);
+    if (j < N) {
+      if (single) val = src[j * 2 + part];
+      else val = src[(j * N + cg * cpt + k) * 2 + part];
+    }
+    dst[i] = val;
+  }
+}
+
+// All targets of a multi-target table in one launch (blockIdx.y = target): the layout of pack_target_kernel, target t
+// at dst + t * (packed words of one target).  src: n_targets row-major N x N (single: N) complex arrays.
+template <typename R>
+__global__ void pack_targets_kernel(const R* __restrict__ src, R* __restrict__ dst, int N, int cpt, int single) {
+  const int groups = single ? 1 : N / cpt;
+  const int total = groups * (N + 1) * 2 * cpt;
+  src += (size_t)blockIdx.y * (single ? N : N * N) * 2;
+  dst += (size_t)blockIdx.y * total;
   for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < total; i += gridDim.x * blockDim.x) {
     int k = i % cpt, r = i / cpt;
     int part = r % 2; r /= 2;

@@ -527,6 +527,13 @@ struct HeisSweepAny : HeisSweep<R, NQ, CPT, 1, 0x0ull, 0x1ull> {
   }
 };
 
+// The multi-target variant (engine_impl.cuh: IsMultiTarget): the same sweeps; the forward sweep starts from the sample's
+// own V^dag, read from the target table in global memory instead of the TMA-staged copy in shared memory.
+template <typename R, int NQ, int CPT>
+struct HeisSweepAnyMT : HeisSweepAny<R, NQ, CPT> {
+  static constexpr bool MULTI_TARGET = true;
+};
+
 // ------------------------------------------------------------------------------------------
 // update / coefficient phase helpers (per gate, executed by the gate's owner thread)
 // ------------------------------------------------------------------------------------------
@@ -1172,6 +1179,7 @@ heis_kernel(const KParams<R> p) {
   using V = typename T::V;
   constexpr int N = C::N, TPS = C::TPS, PB = C::PB, XR = C::XR;
   constexpr int SW = HEIS_SU2_WORDS, CW = HEIS_CP_WORDS;
+  constexpr bool MT = IsMultiTarget<SWP>::value;
 
   extern __shared__ __align__(16) unsigned char smem_raw[];
   __shared__ __align__(8) uint64_t s_bar;
@@ -1182,12 +1190,12 @@ heis_kernel(const KParams<R> p) {
 
   const int tid = threadIdx.x;
   // ---- prologue: TMA-stage V^dag (packed by pack_target_heis_kernel) ----
-  if (tid == 0) {
+  if (!MT && tid == 0) {
     mbar_init(&s_bar, 1);
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
   }
   __syncthreads();
-  if (tid == 0) {
+  if (!MT && tid == 0) {
     mbar_expect_tx(&s_bar, (uint32_t)p.target_bytes);
     tma_bulk_g2s(s_target, p.target_packed, (uint32_t)p.target_bytes, &s_bar);
   }
@@ -1213,7 +1221,7 @@ heis_kernel(const KParams<R> p) {
     s_cp[k] = hm;
   }
   __syncthreads();
-  mbar_wait(&s_bar, 0);
+  if constexpr (!MT) mbar_wait(&s_bar, 0);
 
   const int sl = tid / TPS;   // sample within the block
   const int m = tid % TPS;    // lane within the sample: column group (forward), x >> PB (backward)
@@ -1228,7 +1236,9 @@ heis_kernel(const KParams<R> p) {
   R* coef = s_coef + (size_t)(sl < p.spb ? sl : p.spb) * p.coef_stride;
   R* stage = coef + SW * p.n_su2;                          // staged rows of one layer of the backward sweep
   R* coef_cp = stage + HEIS_STAGE_WORDS * SWP::NSTAGE;
-  const V* tv = reinterpret_cast<const V*>(s_target) + 2 * (size_t)m * (N + 1);
+  const R* tgt = s_target;
+  if constexpr (MT) tgt = p.target_packed + (size_t)p.target_index[b] * (size_t)(2 * N * (N + 1));   // heis_target_words
+  const V* tv = reinterpret_cast<const V*>(tgt) + 2 * (size_t)m * (N + 1);
 
   const unsigned off = (unsigned)(b * P);   // host: B * P < 2^32
   R* aux = p.aux + (size_t)b * p.n_su2 * 4;
@@ -1473,6 +1483,26 @@ __global__ void pack_target_heis_kernel(const R* __restrict__ src, R* __restrict
   }
 }
 
+// All targets of a multi-target table in one launch (blockIdx.y = target): the layout of pack_target_heis_kernel,
+// target t at dst + t * heis_target_words.  src: n_targets row-major N x N complex matrices.
+template <typename R>
+__global__ void pack_targets_heis_kernel(const R* __restrict__ src, R* __restrict__ dst, int N, int cpt) {
+  const int total = (N / cpt) * (N + 1) * 2 * cpt;
+  src += (size_t)blockIdx.y * N * N * 2;
+  dst += (size_t)blockIdx.y * total;
+  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < total; i += gridDim.x * blockDim.x) {
+    int k = i % cpt, t = i / cpt;
+    int part = t % 2; t /= 2;
+    int r = t % (N + 1), l = t / (N + 1);
+    R val = R(0);
+    if (r < N) {
+      const R v = src[((size_t)(l * cpt + k) * N + r) * 2 + part];
+      val = part ? -v : v;
+    }
+    dst[i] = val;
+  }
+}
+
 // Launch geometry: spread the batch evenly over SMs and rounds so that the last wave is as full as the
 // first (every CTA runs all the Adam steps of its samples, so a ragged last wave costs a whole wave).
 //   ctas  resident CTAs per SM.  Each CTA is one synchronised instruction stream (its warps share the instruction
@@ -1642,5 +1672,17 @@ template <typename R> bool launch_heis(const KParams<R>& p, const Program& prog,
 // columns per thread of the heis kernels for (dtype, n): selects the target packing
 template <typename R> int heis_cpt(int n_qubits);
 template <typename R> int launch_pack_target_heis(const R* src, R* dst, int n_qubits, int cpt, cudaStream_t st);
+
+// Multi-target kernels (inst_multi_*.cu).  launch_heis_multi: HeisSweepAnyMT, returns false when none exists for the
+// program's qubit count; launch_engine_multi: InterpSweepMT over the decoded schedule of engine_rb<R>(n, single).
+// The pack functions fill a table of n_targets packed targets (heis / engine layout) in one launch.
+template <typename R> bool launch_heis_multi(const KParams<R>& p, const Program& prog, cudaStream_t st, std::string& err,
+                                             int& rc);
+template <typename R> int launch_engine_multi(const KParams<R>& p, int n_qubits, bool single, cudaStream_t st,
+                                              std::string& err);
+template <typename R> int launch_pack_targets_heis(const R* src, R* dst, int n_qubits, int cpt, int n_targets,
+                                                   cudaStream_t st);
+template <typename R> int launch_pack_targets(const R* src, R* dst, int n_qubits, int cpt, bool single, int n_targets,
+                                              cudaStream_t st);
 
 }  // namespace cpf

@@ -182,6 +182,59 @@ class Program:
         return state
 
 
+    # ---- many targets in one launch ------------------------------------------------------------
+    def workspace_bytes_multi(self, batch, n_targets, loss_kind=L.LOSS_HS, dtype=torch.float32):
+        """Device scratch one adam_run_multi over `batch` samples and `n_targets` targets needs
+        (cpf_workspace_bytes_multi)."""
+        n = C.c_int64()
+        L.check(L.load().cpf_workspace_bytes_multi(self._h, int(loss_kind), _DT[dtype], int(batch), int(n_targets),
+                                                   C.byref(n)))
+        return n.value
+
+    def _target_index(self, loss, target_index, batch):
+        """Host int32 copy of `target_index` after the checks that need no device (the library checks the range)."""
+        if not isinstance(loss, MultiLoss):
+            raise TypeError("the multi-target entry points take a MultiLoss(kind, targets)")
+        loss.check_program(self)
+        idx = np.ascontiguousarray(
+            target_index.detach().cpu().numpy() if isinstance(target_index, torch.Tensor) else target_index,
+            dtype=np.int32).reshape(-1)
+        if idx.shape[0] != batch:
+            raise ValueError(f"target_index has {idx.shape[0]} entries for a batch of {batch}")
+        return idx
+
+    def loss_grad_multi(self, angles, loss, target_index, penalty=None, want_grad=True):
+        """loss_grad with sample b scored against loss.targets[target_index[b]] (cpf_loss_grad_multi)."""
+        B = angles.shape[0]
+        idx = self._target_index(loss, target_index, B)
+        _need_cuda(angles)
+        dt = angles.dtype
+        tt = loss.table(dt, angles.device, idx)
+        lo = torch.empty(B, dtype=dt, device=angles.device)
+        rg = torch.empty(B, dtype=dt, device=angles.device)
+        gr = torch.empty(B, self.n_params, dtype=dt, device=angles.device) if want_grad else None
+        ps = penalty.spec() if penalty is not None else None
+        with _on(angles):
+            L.check(L.load().cpf_loss_grad_multi(self._h, C.byref(tt), C.byref(ps) if ps is not None else None,
+                                                 _DT[dt], B, _ptr(angles), _ptr(lo), _ptr(rg), _ptr(gr), _stream()))
+        return lo, rg, gr
+
+    def adam_run_multi(self, state, loss, target_index, penalty, lr, num_steps, b1=0.9, b2=0.999, eps=1e-8):
+        """adam_run with sample b optimised against loss.targets[target_index[b]] (cpf_adam_run_multi); the index
+        must be the same for every call that continues the same state."""
+        dt = state.angles.dtype
+        idx = self._target_index(loss, target_index, state.batch)
+        tt = loss.table(dt, state.angles.device, idx)
+        ps = penalty.spec() if penalty is not None else None
+        ad = L.CpfAdamSpec(float(lr), float(b1), float(b2), float(eps))
+        buf = state.buffers()
+        with _on(state.angles):
+            L.check(L.load().cpf_adam_run_multi(self._h, C.byref(tt), C.byref(ps) if ps is not None else None,
+                                                C.byref(ad), _DT[dt], state.batch, state.step, int(num_steps),
+                                                C.byref(buf), _stream()))
+        state.step += int(num_steps)
+        return state
+
     def adam_step(self, state, loss_values, grad, penalty, lr, b1=0.9, b2=0.999, eps=1e-8):
         """One iteration of the Adam loop for a loss evaluated outside the engine (cpf_adam_step): penalty, best
         tracking and the Adam update on `state`, given loss_values [B] and grad [B,P] = d loss / d theta."""
@@ -270,6 +323,55 @@ class Loss:
 
     def __repr__(self):
         return f"Loss({self.kind!r}, target{tuple(self.target.shape)})"
+
+
+class MultiLoss:
+    """Declarative loss over many targets (cpf_target_table): one kind ('hs' | 'state' | 'relphase') and `targets`
+    of shape [T, N, N] ('hs', 'relphase') or [T, N] ('state').  Sample b of a multi-target call is scored against
+    targets[target_index[b]]."""
+
+    def __init__(self, kind, targets):
+        if kind not in Loss.KINDS:
+            raise ValueError(f"unknown loss kind {kind!r}")
+        t = np.asarray(targets.detach().cpu().numpy() if isinstance(targets, torch.Tensor) else targets,
+                       dtype=np.complex128)
+        want = 2 if kind == "state" else 3
+        if t.ndim != want or t.shape[0] < 1 or (want == 3 and t.shape[1] != t.shape[2]):
+            raise ValueError(f"MultiLoss({kind!r}) takes targets of shape " + ("[T, N]" if want == 2 else "[T, N, N]") +
+                             f" with T >= 1, got {t.shape}")
+        self.kind = kind
+        self.targets = t
+        self._dev = {}
+
+    @property
+    def n_targets(self):
+        return self.targets.shape[0]
+
+    def check_program(self, program):
+        if self.targets.shape[1] != program.dim:
+            raise ValueError(f"targets of dimension {self.targets.shape[1]} for a {program.n_qubits}-qubit program "
+                             f"(dimension {program.dim})")
+
+    def table(self, dtype, device, index):
+        """cpf_target_table over the device copy of the targets (cached per dtype and device); `index` is the host
+        int32 array the table points to and must outlive the call."""
+        key = (dtype, str(device))
+        if key not in self._dev:
+            self._dev[key] = torch.as_tensor(self.targets, dtype=_CDT[dtype]).contiguous().to(device)
+        return L.CpfTargetTable(Loss.KINDS[self.kind], self.n_targets, self._dev[key].data_ptr(), index.ctypes.data)
+
+    def loss(self, i):
+        """The single-target Loss of target i."""
+        return Loss(self.kind, self.targets[i])
+
+    def __getstate__(self):
+        return {"kind": self.kind, "targets": self.targets}
+
+    def __setstate__(self, st):
+        self.kind, self.targets, self._dev = st["kind"], st["targets"], {}
+
+    def __repr__(self):
+        return f"MultiLoss({self.kind!r}, targets{tuple(self.targets.shape)})"
 
 
 class TorchLoss:

@@ -19,7 +19,7 @@ from . import parallel as PL
 from .ansatz import Ansatz
 from .circuit import convert_to_ZXZ, cp_template_cz_count_depth, cp_to_cz_circuit, gates_count, gates_depth
 from .cp_utils import (filter_cp_results, random_cp_angles, select_batch, verify_cp_result, verify_cp_results)
-from .engine import Loss, Penalty, TorchLoss
+from .engine import Loss, MultiLoss, Penalty, TorchLoss
 from .optimization import ProgramLoss, RawResults, mynimize_repeated, run_adam_batch
 from .penalty import PenaltyFunction, RegularizationOptions, make_regularization_function, tabulate_penalty
 from .matrix_utils import theoretical_lower_bound
@@ -595,3 +595,110 @@ class Synthesize:
                 say('\nTarget number of gates reached.')
                 break
         return results
+
+
+def synthesize_many(layer, targets, options, loss='hs', labels=None, cp_regularization_func=None,
+                    dtype=torch.float32, device=None, save_results=False):
+    """`Synthesize.static(options)` for many targets at once: returns one `Results` per target, in input order.
+
+    Target i gets exactly the work of `Synthesize(layer, unitary_loss_func=Loss(loss, targets[i])).static(options)`
+    (for loss='hs' the same as `target_unitary=targets[i]`): the same initial batch (samples 0..S-1 of
+    PRNGKey(options.random_seed), drawn once and used for every target), the same entry filter and
+    `accepted_num_cz_gates` cut, the same verification with the projected CP angles frozen.  What changes is that all
+    T * S samples run in ONE fused Adam launch (cpf_adam_run_multi), and all surviving candidates of all targets are
+    verified in one more.  Under torch.distributed the T * S items are sharded over the ranks by global index; every
+    rank returns the same list and only rank 0 saves.
+
+    targets: [T, N, N] ('hs', 'relphase') or [T, N] ('state'); labels: None or T labels (needed to save).  A user loss
+    function cannot serve several targets in one launch: `loss` is one of 'hs', 'state', 'relphase'."""
+    if not isinstance(loss, str):
+        raise TypeError("synthesize_many takes a loss kind ('hs', 'state' or 'relphase'); a user loss function runs "
+                        "one target at a time (Synthesize(layer, unitary_loss_func=...).static)")
+    num_qubits = num_qubits_from_layer(layer)
+    ml = MultiLoss(loss, targets)
+    if ml.targets.shape[1] != 2 ** num_qubits:
+        raise ValueError(f"targets of dimension {ml.targets.shape[1]} for a {num_qubits}-qubit layer")
+    T = ml.n_targets
+    if labels is None:
+        labels = [None] * T
+    labels = list(labels)
+    if len(labels) != T:
+        raise ValueError(f"{len(labels)} labels for {T} targets")
+    syns = [Synthesize(layer, unitary_loss_func=ml.loss(i), label=labels[i],
+                       cp_regularization_func=cp_regularization_func, dtype=dtype, device=device) for i in range(T)]
+    results = [s._initialize_results(save_results, '') for s in syns]
+    syn = syns[0]
+    rank, world = PL.rank_world()
+    say = print if rank == 0 else (lambda *a, **k: None)
+    say(f'\nStarting decomposition routine for {T} targets with the following options:')
+    say('\n', options)
+    anz = syn._ansatz(options)
+    P = anz.num_angles
+    S = options.num_samples
+    dev = syn._device()
+
+    # stage 1: item g = t * S + s (target t, sample s), this rank's contiguous block of the T * S items
+    say('\nComputing raw results...')
+    first, count = PL.shard_range(T * S)
+    if count > 0:
+        g = torch.arange(first, first + count, device=dev)
+        init = syn._generate_initial_angles(options.random_seed, anz, cp_dist=options.cp_distribution,
+                                            batch_size=S, dtype=dtype, device=dev)[g % S].contiguous()
+        raw = run_adam_batch(anz.program, ml, syn._penalty(options.r), init, options.learning_rate,
+                             options.num_gd_iterations, target_index=(g // S).cpu().numpy())
+        cz, lo, angles = select_batch(raw, anz.program, options.threshold_cp)
+        keep = torch.nonzero(lo <= options.entry_loss).flatten()
+        best_i = torch.argmin(raw.regloss, dim=1)
+        regloss = raw.regloss[torch.arange(count, device=dev), best_i]
+        gk = g[keep]
+        rec = torch.cat([(gk // S).to(torch.float64)[:, None], (gk % S).to(torch.float64)[:, None],
+                         cz[keep].to(torch.float64)[:, None], lo[keep].to(torch.float64)[:, None],
+                         regloss[keep].to(torch.float64)[:, None], angles[keep].to(torch.float64)], 1)
+    else:
+        rec = torch.zeros(0, 5 + P, dtype=torch.float64, device=dev)
+    rec = PL.gather_rows(rec)
+    # grouped by target; within a target sorted by cz, ties by sample index (the order of static())
+    order = torch.argsort(rec[:, 1], stable=True)
+    order = order[torch.argsort(rec[order, 2], stable=True)]
+    order = order[torch.argsort(rec[order, 0], stable=True)]
+    cand = rec[order]
+    cand = cand[cand[:, 2] <= options.accepted_num_cz_gates]
+    cand_t = cand[:, 0].to(torch.int64).cpu().numpy()
+    cand_cz = cand[:, 2].to(torch.int64).cpu().numpy()
+    for t in range(T):
+        syns[t].last_prospective_cz_counts = cand_cz[cand_t == t].tolist()
+
+    # stage 2: every candidate of every target, one multi-target verification run
+    if len(cand):
+        say(f'\nFound {len(cand)}. Verifying...')
+        mine = PL.round_robin(len(cand))
+        if mine:
+            angles = cand[mine][:, 5:].to(dtype).contiguous()
+            cz, proj, frozen = anz.program.count_cz(angles, options.threshold_cp, project=True)
+            raw = run_adam_batch(anz.program, ml, None, proj, options.learning_rate_at_verification,
+                                 options.num_gd_iterations_at_verification, freeze=frozen,
+                                 target_index=cand_t[mine])
+            bi = torch.argmin(raw.regloss, dim=1)
+            ar = torch.arange(len(mine), device=dev)
+            out = torch.cat([raw.regloss[ar, bi].to(torch.float64)[:, None], cz.to(torch.float64)[:, None],
+                             raw.params[ar, bi].to(torch.float64), frozen.to(torch.float64)], 1)
+        else:
+            out = torch.zeros(0, 2 + 2 * P, dtype=torch.float64, device=dev)
+        out = PL.gather_round_robin(out, len(cand)).cpu().numpy()
+        ok = out[:, 0] <= options.target_loss                    # cp_utils.py:245
+        np_dt = np.float32 if dtype == torch.float32 else np.float64
+        for t in range(T):
+            sel = ok & (cand_t == t)
+            ds = Decomposition._from_cp_batch(syns[t].unitary_loss_func, anz, out[sel, 2:2 + P].astype(np_dt),
+                                              out[sel, 2 + P:] > 0.5, label=labels[t], device=dev)
+            for d in ds:
+                d._static_options = options
+                d._decomposer = syns[t]
+            if ds:
+                results[t].decompositions = list(results[t].decompositions) + ds
+                if save_results and rank == 0:
+                    results[t].save()
+        say(f'\n{int(ok.sum())} successful over {T} targets.')
+    else:
+        say('\nNo results passed.')
+    return results

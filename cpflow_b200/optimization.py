@@ -17,7 +17,7 @@ import numpy as np
 import torch
 
 from . import _lib as L
-from .engine import Loss, Penalty, Program, TorchLoss
+from .engine import Loss, MultiLoss, Penalty, Program, TorchLoss
 
 HISTORY_BYTES_LIMIT = 64 << 30
 
@@ -80,9 +80,14 @@ class RawResults:
 
 
 def run_adam_batch(program, loss, penalty, initial_params, learning_rate, num_iterations,
-                   freeze=None, keep_history=False, chunk=None):
+                   freeze=None, keep_history=False, chunk=None, target_index=None):
     """Device-resident core: `initial_params` is a CUDA tensor [B,P] (not modified).  Returns
-    RawResults on the device.  Restates jit(vmap(mynimize_particular)) (optimization.py:344-362)."""
+    RawResults on the device.  Restates jit(vmap(mynimize_particular)) (optimization.py:344-362).
+    With `target_index` ([B] ints), `loss` is a MultiLoss and sample b runs against its target target_index[b], all in
+    one launch (cpf_adam_run_multi)."""
+    if target_index is not None and not isinstance(loss, MultiLoss):
+        raise TypeError("target_index needs a MultiLoss(kind, targets): a user loss function runs one target at a "
+                        "time on the host-driven loop")
     if not (isinstance(initial_params, torch.Tensor) and initial_params.is_cuda):
         raise L.CpflowError("run_adam_batch needs a CUDA tensor (no CPU fallback)")
     B, P = initial_params.shape
@@ -94,7 +99,9 @@ def run_adam_batch(program, loss, penalty, initial_params, learning_rate, num_it
                                 "use keep_history=False (the reference default for static())")
     with torch.cuda.device(initial_params.device):
         st = program.adam_state(initial_params.clone(), freeze=freeze, hist_len=T if keep_history else 0)
-        if isinstance(loss, TorchLoss):
+        if target_index is not None:
+            program.adam_run_multi(st, loss, target_index, penalty, learning_rate, T)
+        elif isinstance(loss, TorchLoss):
             # user loss outside the engine: the same loop, one iteration at a time (optimization.py:14-25, 61-75)
             for _ in range(T):
                 U = program.unitary(st.angles)

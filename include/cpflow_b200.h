@@ -204,6 +204,30 @@ int cpf_adam_step(const cpf_program* prog, const cpf_penalty_spec* penalty, cons
                   int32_t dtype, int64_t batch, int64_t step, const void* loss, const void* grad,
                   const cpf_adam_buffers* buf, void* stream);
 
+/* Multi-target runs: many independent targets of one loss kind, optimised on the same program in ONE launch.
+ * Sample b of the batch is scored against target target_index[b]; everything else (penalty, Adam, freeze mask,
+ * history, split runs with step0 > 0) works exactly as in cpf_loss_grad / cpf_adam_run, and a sample's results are
+ * those of a single-target call on its own target run on the same kernel family (the Heisenberg-picture kernel with
+ * run-time qubit pairs for HS on block-structured templates, otherwise the interpreter kernel).  Every entry of
+ * target_index is checked before any CUDA call: a bad index is CPF_ERR_INVALID with a message. */
+typedef struct cpf_target_table {
+  int32_t kind;                 /* cpf_loss_kind, as in cpf_loss_spec */
+  int32_t n_targets;
+  const void* targets;          /* device: n_targets x (N*N complex, row-major) for HS / RELPHASE, n_targets x N for STATE */
+  const int32_t* target_index;  /* HOST [batch]: target of each sample, validated in [0, n_targets) */
+} cpf_target_table;
+
+int cpf_loss_grad_multi(const cpf_program* prog, const cpf_target_table* table, const cpf_penalty_spec* penalty,
+                        int32_t dtype, int64_t batch, const void* angles, void* loss_out, void* reg_out,
+                        void* grad_out, void* stream);
+int cpf_adam_run_multi(const cpf_program* prog, const cpf_target_table* table, const cpf_penalty_spec* penalty,
+                       const cpf_adam_spec* adam, int32_t dtype, int64_t batch, int64_t step0, int64_t num_steps,
+                       const cpf_adam_buffers* buf, void* stream);
+/* Device scratch of one cpf_adam_run_multi / cpf_loss_grad_multi call: that of cpf_workspace_bytes without the staged
+ * target, plus the target table (n_targets packed targets) and the device copy of target_index (4 bytes a sample). */
+int cpf_workspace_bytes_multi(const cpf_program* prog, int32_t loss_kind, int32_t dtype, int64_t batch,
+                              int32_t n_targets, int64_t* bytes);
+
 /* cz[B] (int32) = count_cz(angles * cp_mask, threshold) (cpflow/cp_utils.py:45-67): per CP
  * parameter 0 if (a mod 2pi) is within `threshold` of 0 or 2pi, 1 if within of pi, else 2.
  * If `projected` (nullable [B,P]) and `frozen` (nullable uint8 [B,P]) are given they receive the
