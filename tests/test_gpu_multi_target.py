@@ -213,6 +213,40 @@ def test_synthesize_many_end_to_end():
     assert [_key(d) for d in alone.decompositions] == [_key(d) for d in res[1].decompositions]
 
 
+def _state_targets():
+    ghz = np.zeros(8, dtype=complex)
+    ghz[[0, 7]] = 1 / np.sqrt(2)
+    plus, zero = np.array([1, 1]) / np.sqrt(2), np.array([1, 0])
+    product = np.kron(np.kron(plus, zero), np.array([np.cos(0.3), np.exp(0.7j) * np.sin(0.3)]))
+    rng = np.random.default_rng(23)
+    haar = rng.normal(size=8) + 1j * rng.normal(size=8)
+    return np.stack([ghz, product, haar / np.linalg.norm(haar)]), ["ghz", "product", "haar"], 2
+
+
+@pytest.mark.parametrize("kind", ["state", "relphase"])
+def test_synthesize_many_end_to_end_state_and_relphase(kind):
+    """synthesize_many with the losses that run on InterpSweepMT: every decomposition re-scores below target_loss with
+    the single-target loss, labels and targets are carried through, a target alone gives the group's bits."""
+    if kind == "state":
+        tg, labels, easy = _state_targets()
+    else:
+        tg, labels, easy = np.stack([u_toff3, CCZ]), ["toffoli", "ccz"], 2
+    opts = cp.StaticOptions(num_cp_gates=12, accepted_num_cz_gates=14, num_samples=60)
+    res = cp.synthesize_many(chain_layer(3), tg, opts, loss=kind, labels=labels)
+    assert len(res) == len(tg)
+    for t, r in enumerate(res):
+        assert r.label == labels[t] and isinstance(r.loss_function, Loss) and r.loss_function.kind == kind
+        assert np.allclose(r.loss_function.target, tg[t])
+        for d in r.decompositions:
+            assert d.label == labels[t] and np.allclose(d.unitary_loss_func.target, tg[t])
+            # the float32 run's own loss passed the filter; the float64 re-score of its angles as in the HS test
+            assert d.loss <= opts.target_loss and Loss(kind, tg[t])(d.unitary) <= 1e-5
+            assert d.cz_count <= opts.accepted_num_cz_gates and d._static_options is opts
+    assert all(len(res[t].decompositions) >= 1 for t in range(easy))
+    alone = cp.synthesize_many(chain_layer(3), tg[1:2], opts, loss=kind, labels=labels[1:2])[0]
+    assert [_key(d) for d in alone.decompositions] == [_key(d) for d in res[1].decompositions]
+
+
 def test_synthesize_many_matches_static_statistics():
     """Toffoli-3, all-to-all, 10^4 samples: the share of samples verified at 6 CZ agrees with static() within
     binomial error (same initial batch, trajectories differ only by the kernel family's rounding)."""

@@ -1,6 +1,7 @@
 """Measured parity maxima of the CUDA engine against the CPU oracle (run on the GPU box):
 
     python tools/parity_report.py > profiles/parity_r2.txt
+    python tools/parity_report.py --steps > profiles/adam_steps_r1.txt
 
 Same measurement functions as tests/test_gpu_parity.py (tests/parity_lib.py); the tests assert the contract's
 tolerances (1e-5 complex64, 1e-12 complex128), this prints what was actually measured per configuration."""
@@ -45,5 +46,30 @@ def main():
     print("chain  complex64 T=10 " + " ".join(f"{k}={v:.2e}" if isinstance(v, float) else f"{k}={v}" for k, v in m.items()))
 
 
+def steps():
+    """Per-step maxima of tests/test_gpu_adam_steps.py: for every case and checkpoint k the largest error over the
+    samples and its ratio to the bound the test asserts (<= 1 passes; parity_lib.measure_adam_steps)."""
+    import subprocess
+    from cpflow_b200 import _lib
+    smi = subprocess.run(["nvidia-smi", "--query-gpu=name,driver_version,power.limit,clocks.max.sm", "--format=csv,noheader"],
+                         capture_output=True, text=True).stdout.strip()
+    print(f"# device: {torch.cuda.get_device_name(0)}; nvidia-smi: {smi}")
+    print(f"# torch {torch.__version__} (CUDA {torch.version.cuda}); library {os.path.relpath(_lib.LIB_PATH, ROOT)}, cpf_version "
+          f"{_lib.load().cpf_version()}")
+    print("# m, v: max over samples of the norm-wise error; theta: max entry error; loss: max |regloss / reg - oracle|;"
+          " *_r: ratio to the asserted bound")
+    import test_gpu_adam_steps as S
+    for name, dt in S.CASES:
+        got = P.measure_adam_steps(name, dt)
+        print(f"{name} {'c64' if dt == torch.float32 else 'c128'}: engine={got['engine']} "
+              f"words={got['words_per_sample']} chain_identical={got['chain_identical']} "
+              f"f32_breakpoint_entries={got['breakpoint_fixes']}")
+        for r in got["rows"]:
+            print(f"  k={r['k']:5d} m={r['m']:9.2e} m_r={r['m_ratio']:7.3f} v={r['v']:9.2e} v_r={r['v_ratio']:7.3f} "
+                  f"theta={r['theta']:9.2e} theta_r={r['theta_ratio']:7.3f} loss={r['loss']:9.2e} "
+                  f"loss_r={r['loss_ratio']:7.3f} improved={r['improved']:3d} best_ok={int(r['best_ok'])} "
+                  f"frozen_ok={int(r['frozen_unchanged'])}")
+
+
 if __name__ == "__main__":
-    main()
+    steps() if "--steps" in sys.argv[1:] else main()
