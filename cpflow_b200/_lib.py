@@ -16,7 +16,12 @@ MAX_QUBITS = 7
 # enums (mirror include/cpflow_b200.h)
 RX, RY, RZ, CP, CZ, CX = 0, 1, 2, 3, 4, 5
 F32, F64 = 0, 1
-LOSS_HS, LOSS_STATE, LOSS_RELPHASE = 0, 1, 2
+LOSS_HS, LOSS_STATE, LOSS_RELPHASE, LOSS_ISOMETRY = 0, 1, 2, 3
+
+
+def isometry_kind(ancilla_mask):
+    """CPF_ISOMETRY_KIND: the loss-kind argument of the query entry points for an isometry loss."""
+    return LOSS_ISOMETRY | (int(ancilla_mask) << 8)
 PEN_NONE, PEN_PIECEWISE, PEN_L1 = 0, 1, 2
 
 
@@ -26,7 +31,7 @@ class CpfOp(C.Structure):
 
 
 class CpfLossSpec(C.Structure):
-    _fields_ = [("kind", C.c_int32), ("target", C.c_void_p)]
+    _fields_ = [("kind", C.c_int32), ("target", C.c_void_p), ("ancilla_mask", C.c_int32)]
 
 
 class CpfPenaltySpec(C.Structure):

@@ -24,8 +24,8 @@ SOURCES = ["program.cpp", "inst_f32.cu", "inst_f64.cu", "inst_layer_f32.cu", "in
            "inst_heis_f32.cu", "inst_heis_f64.cu",
            "inst_heis_f32_p0.cu", "inst_heis_f32_p1.cu", "inst_heis_f32_p2.cu", "inst_heis_f32_p3.cu",
            "inst_heis_f64_p0.cu", "inst_heis_f64_p1.cu", "inst_heis_f64_p2.cu", "inst_heis_f64_p3.cu",
-           "inst_multi_f32.cu", "inst_multi_f64.cu", "capi.cu"]
-HEADERS = ["program.hpp", "engine.cuh", "engine_impl.cuh", "launch.cuh", "heis_impl.cuh",
+           "inst_multi_f32.cu", "inst_multi_f64.cu", "inst_iso_f32.cu", "inst_iso_f64.cu", "capi.cu"]
+HEADERS = ["program.hpp", "engine.cuh", "engine_impl.cuh", "launch.cuh", "heis_impl.cuh", "iso_impl.cuh",
            os.path.join(ROOT, "include", "cpflow_b200.h")]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
               "-Xcompiler", "-fPIC", "-I" + os.path.join(ROOT, "include"), "-I" + CSRC]

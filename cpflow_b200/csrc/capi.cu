@@ -9,6 +9,7 @@
 
 #include "cpflow_b200.h"
 #include "heis_impl.cuh"
+#include "iso_impl.cuh"
 #include "launch.cuh"
 #include "program.hpp"
 
@@ -315,16 +316,92 @@ int stage_heis_state(const cpf::Program* prog, cpf::KParams<R>& p, Scratch& sc) 
   return CPF_OK;
 }
 
-int check_loss(const cpf_loss_spec* loss) {
-  if (!loss || !loss->target) return fail(CPF_ERR_INVALID, "loss spec / target is NULL");
-  if (loss->kind < CPF_LOSS_HS || loss->kind > CPF_LOSS_RELPHASE)
-    return fail(CPF_ERR_INVALID, "unknown loss kind");
+// ---- isometry loss (CPF_LOSS_ISOMETRY) ----
+// Largest number of input columns k of the 6-7 qubit kernel: a sample is k lane groups of 2^(n-2) threads in one CTA.
+constexpr int ISO_MAX_K = 32;
+
+// Everything about an isometry request that can be refused is refused here, before any CUDA call.
+int check_iso(const cpf::Program* prog, int32_t mask) {
+  const int n = prog->n_qubits;
+  if (mask < 0 || (mask >> n) != 0)
+    return fail(CPF_ERR_INVALID, "ancilla_mask " + std::to_string(mask) + " names a qubit >= n = " + std::to_string(n));
+  if (n > 5 && mask == 0)
+    return fail(CPF_ERR_UNSUPPORTED, "full-unitary losses need n <= 5 qubits (6-7 qubits: state preparation and "
+                                     "cpf_unitary only)");
+  const int k = 1 << (n - __builtin_popcount((unsigned)mask));
+  if (n > 5 && k > ISO_MAX_K)
+    return fail(CPF_ERR_UNSUPPORTED, "isometry losses on 6-7 qubits take at most k = " + std::to_string(ISO_MAX_K) +
+                                     " input columns (k = 2^(n - popcount(ancilla_mask)) = " + std::to_string(k) + ")");
   return CPF_OK;
+}
+
+// k input columns; the ancilla qubits as amplitude-index bits (qubit q is bit n - 1 - q, big-endian)
+struct IsoSpec { int k, amask; };
+IsoSpec iso_spec(const cpf::Program* prog, int32_t mask) {
+  const int n = prog->n_qubits;
+  IsoSpec s{1 << (n - __builtin_popcount((unsigned)mask)), 0};
+  for (int q = 0; q < n; ++q)
+    if ((mask >> q) & 1) s.amask |= 1 << (n - 1 - q);
+  return s;
+}
+
+// The query entry points take a loss kind only: an isometry kind carries its ancilla mask in bits 8-15
+// (CPF_ISOMETRY_KIND).  Splits and checks such an argument.
+int split_kind(const cpf::Program* prog, int32_t arg, int32_t* kind, int32_t* mask) {
+  *kind = arg & 0xff;
+  *mask = (arg >> 8) & 0xff;
+  if (*kind < CPF_LOSS_HS || *kind > CPF_LOSS_ISOMETRY || (arg >> 16) != 0 || (*kind != CPF_LOSS_ISOMETRY && *mask))
+    return fail(CPF_ERR_INVALID, "unknown loss kind");
+  return *kind == CPF_LOSS_ISOMETRY ? check_iso(prog, *mask) : CPF_OK;
+}
+
+// n <= 5: the isometry loss is the HS loss on V = 2^a [W at the columns s_c, 0 elsewhere] (iso_impl.cuh:
+// pack_iso_hs_kernel), built in scratch; `hs` becomes the spec of that HS call.
+template <typename R>
+int stage_iso_as_hs(const cpf::Program* prog, const cpf_loss_spec* loss, Scratch& sc, cpf_loss_spec* hs) {
+  const int n = prog->n_qubits;
+  const IsoSpec is = iso_spec(prog, loss->ancilla_mask);
+  R* v = nullptr;
+  int rc = sc.get((void**)&v, ((size_t)2 << (2 * n)) * sizeof(R));
+  if (rc) return rc;
+  rc = cpf::launch_pack_iso<R>((const R*)loss->target, v, n, is.k, is.amask, true, sc.st);
+  if (rc) return fail(rc, "pack_iso launch failed");
+  *hs = cpf_loss_spec{};
+  hs->kind = CPF_LOSS_HS;
+  hs->target = v;
+  return CPF_OK;
+}
+
+// n >= 6: W packed column by column for the isometry kernel
+template <typename R>
+int stage_iso(const cpf::Program* prog, const cpf_loss_spec* loss, cpf::KParams<R>& p, Scratch& sc) {
+  const int n = prog->n_qubits;
+  const IsoSpec is = iso_spec(prog, loss->ancilla_mask);
+  R* packed = nullptr;
+  int rc = sc.get((void**)&packed, ((size_t)is.k << (n + 1)) * sizeof(R));
+  if (rc) return rc;
+  rc = cpf::launch_pack_iso<R>((const R*)loss->target, packed, n, is.k, is.amask, false, sc.st);
+  if (rc) return fail(rc, "pack_iso launch failed");
+  p.target_packed = packed;
+  p.target_bytes = 0;
+  p.loss_kind = CPF_LOSS_ISOMETRY;
+  p.iso_k = is.k;
+  p.iso_amask = is.amask;
+  return CPF_OK;
+}
+
+int check_loss(const cpf::Program* prog, const cpf_loss_spec* loss) {
+  if (!loss || !loss->target) return fail(CPF_ERR_INVALID, "loss spec / target is NULL");
+  if (loss->kind < CPF_LOSS_HS || loss->kind > CPF_LOSS_ISOMETRY)
+    return fail(CPF_ERR_INVALID, "unknown loss kind");
+  return loss->kind == CPF_LOSS_ISOMETRY ? check_iso(prog, loss->ancilla_mask) : CPF_OK;
 }
 
 // Everything a multi-target call needs to know is checked here, before any CUDA call.
 int check_table(const cpf::Program* prog, const cpf_target_table* tt, int64_t batch) {
   if (!tt) return fail(CPF_ERR_INVALID, "target table is NULL");
+  if (tt->kind == CPF_LOSS_ISOMETRY)
+    return fail(CPF_ERR_UNSUPPORTED, "multi-target tables do not take the isometry loss (one target per call)");
   if (tt->kind < CPF_LOSS_HS || tt->kind > CPF_LOSS_RELPHASE) return fail(CPF_ERR_INVALID, "unknown loss kind");
   if (tt->n_targets < 1) return fail(CPF_ERR_INVALID, "target table: n_targets must be >= 1");
   if (!tt->targets) return fail(CPF_ERR_INVALID, "target table: targets is NULL");
@@ -413,16 +490,24 @@ int run_loss_grad(const cpf::Program* prog, const cpf_loss_spec* loss, const cpf
                   int64_t batch, const void* angles, void* loss_out, void* reg_out, void* grad_out,
                   cudaStream_t st, const cpf_target_table* table = nullptr) {
   cpf::KParams<R> p;
-  const bool single = loss->kind == CPF_LOSS_STATE;
+  Scratch sc;
+  sc.st = st;
+  cpf_loss_spec hs;
+  const bool iso = loss->kind == CPF_LOSS_ISOMETRY && prog->n_qubits > 5;    // else n <= 5: an HS call on V
+  if (loss->kind == CPF_LOSS_ISOMETRY && !iso) {
+    int rc = stage_iso_as_hs<R>(prog, loss, sc, &hs);
+    if (rc) return rc;
+    loss = &hs;
+  }
+  const bool single = loss->kind == CPF_LOSS_STATE || iso;
   int rc = fill_common(prog, p, batch, single);
   if (rc) return rc;
   p.mode = cpf::M_LOSSGRAD;
   p.angles = (R*)angles; p.loss_out = (R*)loss_out; p.reg_out = (R*)reg_out; p.grad_out = (R*)grad_out;
-  Scratch sc;
-  sc.st = st;
   const bool heis = use_heis<R>(prog, loss) && (unsigned long long)batch * (unsigned long long)prog->n_params < (1ull << 32);
   rc = fill_penalty(prog, pen, p, sc);
   if (!rc && table) rc = stage_multi(prog, table, p, heis, sc);
+  else if (!rc && iso) rc = stage_iso(prog, loss, p, sc);
   else if (!rc) rc = heis ? stage_heis(prog, loss, p, sc) : stage_target(prog, loss, p, single, sc);
   if (!rc && grad_out) {
     cudaError_t e = cudaMemsetAsync(grad_out, 0, (size_t)batch * prog->n_params * sizeof(R), st);
@@ -430,7 +515,7 @@ int run_loss_grad(const cpf::Program* prog, const cpf_loss_spec* loss, const cpf
   }
   std::string err;
   if (!rc) {
-    rc = launch_staged<R>(p, prog, table, heis, single, st, err);
+    rc = iso ? cpf::launch_iso<R>(p, prog->n_qubits, st, err) : launch_staged<R>(p, prog, table, heis, single, st, err);
     if (rc) fail(rc, err);
   }
   return rc;
@@ -455,7 +540,8 @@ int run_adam(const cpf::Program* prog, const cpf_loss_spec* loss, const cpf_pena
              const cpf_adam_spec* adam, int64_t batch, int64_t step0, int64_t num_steps,
              const cpf_adam_buffers* buf, cudaStream_t st, const cpf_target_table* table = nullptr) {
   cpf::KParams<R> p;
-  const bool single = loss->kind == CPF_LOSS_STATE;
+  const bool iso = loss->kind == CPF_LOSS_ISOMETRY && prog->n_qubits > 5;    // else n <= 5: an HS call on V
+  const bool single = loss->kind == CPF_LOSS_STATE || iso;
   int rc = fill_common(prog, p, batch, single);
   if (rc) return rc;
   p.mode = cpf::M_ADAM;
@@ -473,13 +559,20 @@ int run_adam(const cpf::Program* prog, const cpf_loss_spec* loss, const cpf_pena
     sc.base = (char*)buf->workspace;
     sc.size = buf->workspace_bytes > 0 ? (size_t)buf->workspace_bytes : 0;
   }
+  cpf_loss_spec hs;
+  if (loss->kind == CPF_LOSS_ISOMETRY && !iso) {
+    rc = stage_iso_as_hs<R>(prog, loss, sc, &hs);
+    if (rc) return rc;
+    loss = &hs;
+  }
   const bool heis = use_heis<R>(prog, loss) && (unsigned long long)batch * (unsigned long long)prog->n_params < (1ull << 32);
   rc = fill_penalty(prog, pen, p, sc);
   if (!rc && table) rc = stage_multi(prog, table, p, heis, sc);
+  else if (!rc && iso) rc = stage_iso(prog, loss, p, sc);
   else if (!rc) rc = heis ? stage_heis(prog, loss, p, sc) : stage_target(prog, loss, p, single, sc);
   std::string err;
   if (!rc) {
-    rc = launch_staged<R>(p, prog, table, heis, single, st, err);
+    rc = iso ? cpf::launch_iso<R>(p, prog->n_qubits, st, err) : launch_staged<R>(p, prog, table, heis, single, st, err);
     if (rc) fail(rc, err);
   }
   return rc;
@@ -487,12 +580,18 @@ int run_adam(const cpf::Program* prog, const cpf_loss_spec* loss, const cpf_pena
 
 // bytes of scratch one cpf_adam_run / cpf_loss_grad needs (the blocks Scratch::get hands out, each 256-byte aligned)
 template <typename R>
-int64_t workspace_bytes_t(const cpf::Program* prog, int32_t loss_kind, int64_t batch) {
+int64_t workspace_bytes_t(const cpf::Program* prog, int32_t loss_kind, int32_t mask, int64_t batch) {
+  size_t total = Scratch::align(prog->cp.empty() ? 1 : prog->cp.size());          // penalty mask
+  if (loss_kind == CPF_LOSS_ISOMETRY) {
+    const int n = prog->n_qubits;
+    if (n > 5) return (int64_t)(total + Scratch::align(((size_t)iso_spec(prog, mask).k << (n + 1)) * sizeof(R)));
+    total += Scratch::align(((size_t)2 << (2 * n)) * sizeof(R));                   // V of the HS call
+    loss_kind = CPF_LOSS_HS;
+  }
   cpf_loss_spec ls{};
   ls.kind = loss_kind;
   const bool single = loss_kind == CPF_LOSS_STATE;
   const bool heis = use_heis<R>(prog, &ls) && (unsigned long long)batch * (unsigned long long)prog->n_params < (1ull << 32);
-  size_t total = Scratch::align(prog->cp.empty() ? 1 : prog->cp.size());          // penalty mask
   if (heis) {
     size_t tb, ap, pk;
     heis_scratch_sizes<R>(prog, batch, &tb, &ap, &pk);
@@ -798,6 +897,27 @@ static int launch_plan_t(const cpf::Program* prog, const cpf_loss_spec_kind_only
   return CPF_OK;
 }
 
+// the isometry kernel's geometry (iso_impl.cuh: iso_geometry); co-residency is not planned (ctas_per_sm = 0)
+template <typename R>
+static int iso_plan_t(const cpf::Program* prog, int32_t mask, int64_t batch, cpf_launch_info* out) {
+  const int n = prog->n_qubits, n_su2 = (int)prog->su2.size(), n_cp = (int)prog->cp.size();
+  const int k = iso_spec(prog, mask).k;
+  const cpf::DecodedSchedule ds = cpf::decode_schedule(*prog, cpf::engine_rb<R>(n, true));
+  const int n_red = ds.red.empty() ? 1 : (int)(ds.red.size() / 8);
+  const cpf::IsoGeometry g = cpf::iso_geometry(n, k, n_su2, n_cp, (int)prog->sched.size(), n_red, sizeof(R));
+  out->engine = 0;
+  out->block_threads = g.block;
+  out->samples_per_cta = g.spb;
+  out->threads_per_sample = g.spt;
+  out->max_block_threads = n == 6 ? 512 : 1024;          // __launch_bounds__ of iso_kernel
+  out->words_per_sample = cpf::iso_sample_words(cpf::coef_stride_words(n_su2, n_cp), k, cpf::iso_sum_stride(n_su2, n_cp));
+  out->time_slices = 1;
+  out->grid = (batch + g.spb - 1) / g.spb;
+  out->smem_bytes = (int64_t)g.smem;
+  out->launches_per_run = 1;
+  return CPF_OK;
+}
+
 extern "C" {
 
 int cpf_version(void) { return CPF_VERSION; }
@@ -874,11 +994,11 @@ int cpf_loss_grad(const cpf_program* prog, const cpf_loss_spec* loss, const cpf_
                   int32_t dtype, int64_t batch, const void* angles, void* loss_out, void* reg_out,
                   void* grad_out, void* stream) {
   if (!prog || batch < 0) return fail(CPF_ERR_INVALID, "NULL program / bad batch");
-  int rc = check_loss(loss);
+  const cpf::Program* p = reinterpret_cast<const cpf::Program*>(prog);
+  int rc = check_loss(p, loss);
   if (rc) return rc;
   if (batch == 0) return CPF_OK;
   if (!loss_out) return fail(CPF_ERR_INVALID, "loss_out is NULL");
-  const cpf::Program* p = reinterpret_cast<const cpf::Program*>(prog);
   if (!angles && p->n_params > 0) return fail(CPF_ERR_INVALID, "angles is NULL");
   CPF_DISPATCH(dtype, (run_loss_grad<R>(p, loss, penalty, batch, angles, loss_out, reg_out, grad_out,
                                         (cudaStream_t)stream)));
@@ -898,7 +1018,7 @@ int cpf_adam_run(const cpf_program* prog, const cpf_loss_spec* loss, const cpf_p
                  const cpf_adam_buffers* buf, void* stream) {
   if (!prog || !adam || !buf || batch < 0 || step0 < 0 || num_steps < 0)
     return fail(CPF_ERR_INVALID, "NULL argument / negative size");
-  int rc = check_loss(loss);
+  int rc = check_loss(reinterpret_cast<const cpf::Program*>(prog), loss);
   if (rc) return rc;
   if (batch == 0 || num_steps == 0) return CPF_OK;
   if (!buf->angles || !buf->m || !buf->v || !buf->best_params || !buf->best_regloss || !buf->best_reg ||
@@ -915,9 +1035,11 @@ int cpf_adam_run(const cpf_program* prog, const cpf_loss_spec* loss, const cpf_p
 
 int cpf_workspace_bytes(const cpf_program* prog, int32_t loss_kind, int32_t dtype, int64_t batch, int64_t* bytes) {
   if (!prog || !bytes || batch < 0) return fail(CPF_ERR_INVALID, "NULL argument / negative batch");
-  if (loss_kind < CPF_LOSS_HS || loss_kind > CPF_LOSS_RELPHASE) return fail(CPF_ERR_INVALID, "unknown loss kind");
   const cpf::Program* p = reinterpret_cast<const cpf::Program*>(prog);
-  *bytes = dtype == CPF_F64 ? workspace_bytes_t<double>(p, loss_kind, batch) : workspace_bytes_t<float>(p, loss_kind, batch);
+  int32_t kind, mask;
+  int rc = split_kind(p, loss_kind, &kind, &mask);
+  if (rc) return rc;
+  *bytes = dtype == CPF_F64 ? workspace_bytes_t<double>(p, kind, mask, batch) : workspace_bytes_t<float>(p, kind, mask, batch);
   return CPF_OK;
 }
 
@@ -931,7 +1053,7 @@ int cpf_loss_grad_multi(const cpf_program* prog, const cpf_target_table* table, 
   if (batch == 0) return CPF_OK;
   if (!loss_out) return fail(CPF_ERR_INVALID, "loss_out is NULL");
   if (!angles && p->n_params > 0) return fail(CPF_ERR_INVALID, "angles is NULL");
-  const cpf_loss_spec loss{table->kind, table->targets};
+  const cpf_loss_spec loss{table->kind, table->targets, 0};
   CPF_DISPATCH(dtype, (run_loss_grad<R>(p, &loss, penalty, batch, angles, loss_out, reg_out, grad_out,
                                         (cudaStream_t)stream, table)));
 }
@@ -951,7 +1073,7 @@ int cpf_adam_run_multi(const cpf_program* prog, const cpf_target_table* table, c
   if ((buf->hist_params || buf->hist_regloss) && buf->hist_len <= 0)
     return fail(CPF_ERR_INVALID, "history buffers given with hist_len <= 0");
   if (num_steps > 2000000000LL) return fail(CPF_ERR_INVALID, "num_steps too large");
-  const cpf_loss_spec loss{table->kind, table->targets};
+  const cpf_loss_spec loss{table->kind, table->targets, 0};
   CPF_DISPATCH(dtype, (run_adam<R>(p, &loss, penalty, adam, batch, step0, num_steps, buf, (cudaStream_t)stream,
                                    table)));
 }
@@ -959,6 +1081,8 @@ int cpf_adam_run_multi(const cpf_program* prog, const cpf_target_table* table, c
 int cpf_workspace_bytes_multi(const cpf_program* prog, int32_t loss_kind, int32_t dtype, int64_t batch,
                               int32_t n_targets, int64_t* bytes) {
   if (!prog || !bytes || batch < 0) return fail(CPF_ERR_INVALID, "NULL argument / negative batch");
+  if (loss_kind == CPF_LOSS_ISOMETRY)
+    return fail(CPF_ERR_UNSUPPORTED, "multi-target tables do not take the isometry loss (one target per call)");
   if (loss_kind < CPF_LOSS_HS || loss_kind > CPF_LOSS_RELPHASE) return fail(CPF_ERR_INVALID, "unknown loss kind");
   if (n_targets < 1) return fail(CPF_ERR_INVALID, "n_targets must be >= 1");
   if (dtype != CPF_F32 && dtype != CPF_F64) return fail(CPF_ERR_INVALID, "unknown dtype");
@@ -1052,8 +1176,11 @@ int cpf_initial_angles(const cpf_program* prog, int32_t dtype, uint64_t seed, in
 int cpf_eval_cost(const cpf_program* prog, int32_t loss_kind, int32_t dtype, double* flops, double* bytes) {
   if (!prog) return fail(CPF_ERR_INVALID, "NULL program");
   const cpf::Program* p = reinterpret_cast<const cpf::Program*>(prog);
+  int32_t kind, mask;
+  int rc = split_kind(p, loss_kind, &kind, &mask);
+  if (rc) return rc;
   const double N = (double)(1 << p->n_qubits);
-  const double C = loss_kind == CPF_LOSS_STATE ? 1.0 : N;
+  const double C = kind == CPF_LOSS_STATE ? 1.0 : kind == CPF_LOSS_ISOMETRY ? (double)iso_spec(p, mask).k : N;
   const double rs = dtype == CPF_F64 ? 8.0 : 4.0;
   if (flops) *flops = C * N * (16.0 * p->n_rot + 4.0 * p->n_phase + 8.0);
   if (bytes) *bytes = 6.0 * p->n_params * rs + 2.0 * rs;
@@ -1064,8 +1191,14 @@ int cpf_executed_cost(const cpf_program* prog, int32_t loss_kind, int32_t dtype,
   if (!prog || !flops) return fail(CPF_ERR_INVALID, "NULL argument");
   const cpf::Program* p = reinterpret_cast<const cpf::Program*>(prog);
   const double N = (double)(1 << p->n_qubits), n = p->n_qubits, K = (double)p->cp.size(), G = (double)p->su2.size();
+  int32_t kind, mask;
+  int rc = split_kind(p, loss_kind, &kind, &mask);
+  if (rc) return rc;
+  // isometry: n <= 5 runs as an HS call; n >= 6 on the isometry kernel, the state-adjoint count with C = k
+  const bool iso = kind == CPF_LOSS_ISOMETRY && p->n_qubits > 5;
+  if (kind == CPF_LOSS_ISOMETRY && !iso) kind = CPF_LOSS_HS;
   cpf_loss_spec ls{};
-  ls.kind = loss_kind;
+  ls.kind = kind;
   const bool heis = dtype == CPF_F64 ? use_heis<double>(p, &ls) : use_heis<float>(p, &ls);
   if (heis) {
     // heis_kernel (heis_impl.cuh), FMA = 2 flop, per sample and step:
@@ -1080,7 +1213,7 @@ int cpf_executed_cost(const cpf_program* prog, int32_t loss_kind, int32_t dtype,
   } else {
     // state-adjoint kernels: the credited count plus the uncompute of phi (6 flop per amplitude and rotation on
     // fused gates, 1.5 per phase gate), with fused gates instead of primitive rotations: C N (22 G + 5.5 K + 8)
-    const double C = loss_kind == CPF_LOSS_STATE ? 1.0 : N;
+    const double C = kind == CPF_LOSS_STATE ? 1.0 : iso ? (double)iso_spec(p, mask).k : N;
     *flops = C * N * (22.0 * G + 5.5 * K + 8.0) + 232.0 * G + 80.0 * K;
   }
   return CPF_OK;
@@ -1092,7 +1225,12 @@ int cpf_launch_plan(const cpf_program* prog, int32_t loss_kind, int32_t dtype, i
   if (batch < 0) return fail(CPF_ERR_INVALID, "negative batch");
   std::memset(out, 0, sizeof(*out));
   const cpf::Program* p = reinterpret_cast<const cpf::Program*>(prog);
-  const cpf_loss_spec_kind_only lk{loss_kind};
+  int32_t kind, mask;
+  int rc = split_kind(p, loss_kind, &kind, &mask);
+  if (rc) return rc;
+  if (kind == CPF_LOSS_ISOMETRY && p->n_qubits > 5)
+    return dtype == CPF_F64 ? iso_plan_t<double>(p, mask, batch, out) : iso_plan_t<float>(p, mask, batch, out);
+  const cpf_loss_spec_kind_only lk{kind == CPF_LOSS_ISOMETRY ? CPF_LOSS_HS : kind};   // n <= 5: an HS call
   return dtype == CPF_F64 ? launch_plan_t<double>(p, lk, batch, n_sm, regs_per_thread, out)
                           : launch_plan_t<float>(p, lk, batch, n_sm, regs_per_thread, out);
 }

@@ -79,6 +79,8 @@ struct KParams {
   // multi-target kernels (sweep types with MULTI_TARGET, engine_impl.cuh): device [B], sample b is scored against the
   // packed target target_index[b] of the table at target_packed (nothing is staged: target_bytes = 0)
   const int32_t* target_index;
+  // isometry kernels (iso_impl.cuh): k input columns per sample, and the ancilla qubits as amplitude-index bits
+  int iso_k, iso_amask;
 };
 
 // ------------------------------------------------------------------------------------------

@@ -286,28 +286,54 @@ class AdamState:
 
 
 class Loss:
-    """Declarative loss spec (cpf_loss_spec): 'hs' | 'state' | 'relphase' and a target array."""
-    KINDS = {"hs": L.LOSS_HS, "state": L.LOSS_STATE, "relphase": L.LOSS_RELPHASE}
+    """Declarative loss spec (cpf_loss_spec): 'hs' | 'state' | 'relphase' | 'isometry' and a target array.
 
-    def __init__(self, kind, target):
+    'isometry' takes `ancillas`, the qubits that start in |0>: with k = 2^(n - len(ancillas)) and s_0 < ... < s_{k-1}
+    the basis states whose ancilla qubits are 0, the target W is N x k (column c = the wanted image of |s_c>) and the
+    loss is 1 - |sum_c <W e_c| U |s_c>|^2 / k^2 (one global phase, like 'hs')."""
+    KINDS = {"hs": L.LOSS_HS, "state": L.LOSS_STATE, "relphase": L.LOSS_RELPHASE, "isometry": L.LOSS_ISOMETRY}
+
+    def __init__(self, kind, target, ancillas=None):
         if kind not in self.KINDS:
             raise ValueError(f"unknown loss kind {kind!r}")
+        if ancillas is not None and kind != "isometry":
+            raise ValueError(f"ancillas are an argument of the 'isometry' loss, not of {kind!r}")
         self.kind = kind
         self.target = np.asarray(target.detach().cpu().numpy() if isinstance(target, torch.Tensor) else target,
                                  dtype=np.complex128)
+        self.ancillas = ()
+        if kind == "isometry":
+            self.ancillas = _check_isometry(self.target, ancillas)
         self._dev = {}
+
+    @property
+    def ancilla_mask(self):
+        return sum(1 << q for q in self.ancillas)
+
+    @property
+    def columns(self):
+        """Basis indices s_0 < ... < s_{k-1} of the input columns ('isometry'): ancilla qubits (big-endian) are 0."""
+        n = int(self.target.shape[0]).bit_length() - 1
+        bits = sum(1 << (n - 1 - q) for q in self.ancillas)
+        return tuple(s for s in range(2 ** n) if s & bits == 0)
+
+    @property
+    def code(self):
+        """The loss-kind argument of the query entry points (workspace_bytes, launch_plan, eval_cost, executed_cost)."""
+        return L.isometry_kind(self.ancilla_mask) if self.kind == "isometry" else self.KINDS[self.kind]
 
     def spec(self, dtype, device):
         key = (dtype, str(device))
         if key not in self._dev:
             self._dev[key] = torch.as_tensor(self.target, dtype=_CDT[dtype]).contiguous().to(device)
-        return L.CpfLossSpec(self.KINDS[self.kind], self._dev[key].data_ptr())
+        return L.CpfLossSpec(self.KINDS[self.kind], self._dev[key].data_ptr(), self.ancilla_mask)
 
     def __getstate__(self):
-        return {"kind": self.kind, "target": self.target}
+        return {"kind": self.kind, "target": self.target, "ancillas": self.ancillas}
 
     def __setstate__(self, st):
         self.kind, self.target, self._dev = st["kind"], st["target"], {}
+        self.ancillas = tuple(st.get("ancillas", ()))
 
     def __call__(self, u):
         """Value of the loss at an explicit unitary `u` (host utility with the formulas of
@@ -319,10 +345,51 @@ class Loss:
             return float(1 - np.abs((u * self.target.conj()).sum()) ** 2 / n ** 2)
         if self.kind == "state":
             return float(1 - np.abs((self.target.conj() * u[:, 0]).sum()) ** 2)
+        if self.kind == "isometry":
+            k = self.target.shape[1]
+            return float(1 - np.abs((self.target.conj() * u[:, list(self.columns)]).sum()) ** 2 / k ** 2)
         return float(1 - (np.abs(self.target.conj() * u) ** 2).sum() / n)
 
     def __repr__(self):
+        if self.kind == "isometry":
+            return f"Loss('isometry', target{tuple(self.target.shape)}, ancillas={list(self.ancillas)})"
         return f"Loss({self.kind!r}, target{tuple(self.target.shape)})"
+
+
+def _check_isometry(W, ancillas):
+    """Shape checks of an 'isometry' target: W is N x k with N = 2^n and k = 2^(n - len(ancillas)); the ancillas are
+    distinct qubits in [0, n).  Returns the sorted ancilla tuple."""
+    if ancillas is None:
+        raise ValueError("the 'isometry' loss needs `ancillas` (the qubits that start in |0>; [] for none)")
+    anc = [int(q) for q in ancillas]
+    if W.ndim != 2 or W.shape[0] < 2 or W.shape[0] & (W.shape[0] - 1):
+        raise ValueError(f"an 'isometry' target is N x k with N = 2^n rows, got shape {W.shape}")
+    n = W.shape[0].bit_length() - 1
+    if len(set(anc)) != len(anc) or any(q < 0 or q >= n for q in anc):
+        raise ValueError(f"ancillas {list(ancillas)} must be distinct qubits in [0, {n})")
+    k = 2 ** (n - len(anc))
+    if W.shape[1] != k:
+        raise ValueError(f"an 'isometry' target with {len(anc)} ancillas on {n} qubits is {2 ** n} x {k}, "
+                         f"got shape {W.shape}")
+    return tuple(sorted(anc))
+
+
+def clean_ancilla_isometry(G, ancillas, n):
+    """Target W of Loss('isometry', W, ancillas) for a unitary G on the data qubits (the n - len(ancillas) qubits that
+    are not ancillas, in increasing order, big-endian) when the ancillas must return to |0>: column c of W is the
+    state with the data qubits in G|c> and every ancilla in |0>."""
+    G = np.asarray(G, dtype=np.complex128)
+    anc = sorted(set(int(q) for q in ancillas))
+    if any(q < 0 or q >= n for q in anc):
+        raise ValueError(f"ancillas {list(ancillas)} must be qubits in [0, {n})")
+    data = [q for q in range(n) if q not in anc]
+    k = 2 ** len(data)
+    if G.shape != (k, k):
+        raise ValueError(f"G acts on {len(data)} data qubits: expected shape {(k, k)}, got {G.shape}")
+    rows = [sum(((d >> (len(data) - 1 - i)) & 1) << (n - 1 - q) for i, q in enumerate(data)) for d in range(k)]
+    W = np.zeros((2 ** n, k), dtype=np.complex128)
+    W[rows, :] = G
+    return W
 
 
 class MultiLoss:

@@ -76,13 +76,25 @@ typedef enum cpf_dtype {
 typedef enum cpf_loss_kind {
   CPF_LOSS_HS = 0,       /* 1 - |sum_ij U_ij conj(V_ij)|^2 / N^2   matrix_utils.py:35-42 */
   CPF_LOSS_STATE = 1,    /* 1 - |<psi| U |0>|^2                    tutorial ipynb:1318    */
-  CPF_LOSS_RELPHASE = 2  /* 1 - sum_ij |conj(V_ij) U_ij|^2 / N     tutorial ipynb:1507    */
+  CPF_LOSS_RELPHASE = 2, /* 1 - sum_ij |conj(V_ij) U_ij|^2 / N     tutorial ipynb:1507    */
+  CPF_LOSS_ISOMETRY = 3  /* 1 - |sum_c <W e_c| U |s_c>|^2 / k^2     (ancilla qubits start in |0>) */
 } cpf_loss_kind;
 
+/* ISOMETRY: the qubits of `ancilla_mask` (bit q = qubit q) start in |0>, so only the images of the k = 2^(n - popcount)
+ * basis states s_0 < ... < s_{k-1} whose ancilla bits are 0 matter; column c of the N x k target W is the wanted
+ * image of |s_c>.  One global phase, like HS: ancilla_mask = 0 is the HS loss, all qubits (k = 1) the state loss.
+ * n <= 5 runs on the HS kernels (target 2^a [W at the columns s_c, 0 elsewhere], N = 2^a k: exact scaling); n = 6, 7
+ * on the isometry kernel with k <= 32 (k = 64 and ancilla_mask = 0 are CPF_ERR_UNSUPPORTED).  Not for multi-target
+ * tables.  A mask bit at a position >= n is CPF_ERR_INVALID. */
 typedef struct cpf_loss_spec {
   int32_t kind;       /* cpf_loss_kind */
-  const void* target; /* device: N*N complex row-major (HS, RELPHASE) or N complex (STATE) */
+  const void* target; /* device: N*N complex row-major (HS, RELPHASE), N complex (STATE), N*k row-major (ISOMETRY) */
+  int32_t ancilla_mask; /* ISOMETRY only (ignored for the other kinds) */
 } cpf_loss_spec;
+
+/* cpf_workspace_bytes, cpf_eval_cost, cpf_executed_cost and cpf_launch_plan take a loss kind only: for the isometry
+ * loss pass CPF_ISOMETRY_KIND(ancilla_mask), which carries the mask in bits 8-15. */
+#define CPF_ISOMETRY_KIND(ancilla_mask) ((int32_t)CPF_LOSS_ISOMETRY | ((int32_t)(ancilla_mask) << 8))
 
 typedef enum cpf_penalty_kind {
   CPF_PEN_NONE = 0,
@@ -250,7 +262,8 @@ int cpf_initial_angles(const cpf_program* prog, int32_t dtype, uint64_t seed,
                        void* out, void* stream);
 
 /* Algorithmic work of one loss+grad evaluation, SURVEY.md §8(d):
- * flops = C*N*(16*G1 + 4*K + 8), bytes = 6*P*sizeof(real) + 2*sizeof(real). */
+ * flops = C*N*(16*G1 + 4*K + 8), bytes = 6*P*sizeof(real) + 2*sizeof(real); C = N columns (HS, RELPHASE), 1 (STATE),
+ * k (ISOMETRY). */
 int cpf_eval_cost(const cpf_program* prog, int32_t loss_kind, int32_t dtype, double* flops,
                   double* bytes);
 
