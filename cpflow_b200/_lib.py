@@ -11,7 +11,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("CPF_LIB_PATH") or os.path.join(HERE, "lib", "libcpflow_b200.so")
 
 MAX_SEGMENTS = 16
-MAX_QUBITS = 7
+MAX_QUBITS = 8
 
 # enums (mirror include/cpflow_b200.h)
 RX, RY, RZ, CP, CZ, CX = 0, 1, 2, 3, 4, 5

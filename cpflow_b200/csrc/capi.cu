@@ -84,8 +84,7 @@ int device_program(const cpf::Program* prog, cpf::DeviceProgram* out) {
 // decoded schedule for a kernel configuration with `rb` register bits, cached per device
 int device_decoded(const cpf::Program* prog, int rb, cpf::DeviceDecoded* out) {
   if (rb < 0 || rb >= 8)
-    return fail(CPF_ERR_UNSUPPORTED, "full-unitary losses need n <= 5 qubits (6-7 qubits: state preparation and "
-                                     "cpf_unitary only)");
+    return fail(CPF_ERR_UNSUPPORTED, cpf::FULL_UNITARY_LIMIT);
   int dev = 0;
   CPF_CUDA(cudaGetDevice(&dev));
   std::lock_guard<std::mutex> lock(prog->mu);
@@ -316,8 +315,15 @@ int stage_heis_state(const cpf::Program* prog, cpf::KParams<R>& p, Scratch& sc) 
   return CPF_OK;
 }
 
+// HS and relative-phase losses run on the full-unitary kernels, which stop at 5 qubits: refused before any CUDA call.
+int check_full_unitary(const cpf::Program* prog, int32_t kind) {
+  if ((kind == CPF_LOSS_HS || kind == CPF_LOSS_RELPHASE) && prog->n_qubits > 5)
+    return fail(CPF_ERR_UNSUPPORTED, cpf::FULL_UNITARY_LIMIT);
+  return CPF_OK;
+}
+
 // ---- isometry loss (CPF_LOSS_ISOMETRY) ----
-// Largest number of input columns k of the 6-7 qubit kernel: a sample is k lane groups of 2^(n-2) threads in one CTA.
+// Largest number of input columns k of the 6-8 qubit kernel: a sample is k lane groups of 2^(n-RB) threads in one CTA.
 constexpr int ISO_MAX_K = 32;
 
 // Everything about an isometry request that can be refused is refused here, before any CUDA call.
@@ -326,11 +332,10 @@ int check_iso(const cpf::Program* prog, int32_t mask) {
   if (mask < 0 || (mask >> n) != 0)
     return fail(CPF_ERR_INVALID, "ancilla_mask " + std::to_string(mask) + " names a qubit >= n = " + std::to_string(n));
   if (n > 5 && mask == 0)
-    return fail(CPF_ERR_UNSUPPORTED, "full-unitary losses need n <= 5 qubits (6-7 qubits: state preparation and "
-                                     "cpf_unitary only)");
+    return fail(CPF_ERR_UNSUPPORTED, cpf::FULL_UNITARY_LIMIT);
   const int k = 1 << (n - __builtin_popcount((unsigned)mask));
   if (n > 5 && k > ISO_MAX_K)
-    return fail(CPF_ERR_UNSUPPORTED, "isometry losses on 6-7 qubits take at most k = " + std::to_string(ISO_MAX_K) +
+    return fail(CPF_ERR_UNSUPPORTED, "isometry losses on 6-8 qubits take at most k = " + std::to_string(ISO_MAX_K) +
                                      " input columns (k = 2^(n - popcount(ancilla_mask)) = " + std::to_string(k) + ")");
   return CPF_OK;
 }
@@ -394,7 +399,7 @@ int check_loss(const cpf::Program* prog, const cpf_loss_spec* loss) {
   if (!loss || !loss->target) return fail(CPF_ERR_INVALID, "loss spec / target is NULL");
   if (loss->kind < CPF_LOSS_HS || loss->kind > CPF_LOSS_ISOMETRY)
     return fail(CPF_ERR_INVALID, "unknown loss kind");
-  return loss->kind == CPF_LOSS_ISOMETRY ? check_iso(prog, loss->ancilla_mask) : CPF_OK;
+  return loss->kind == CPF_LOSS_ISOMETRY ? check_iso(prog, loss->ancilla_mask) : check_full_unitary(prog, loss->kind);
 }
 
 // Everything a multi-target call needs to know is checked here, before any CUDA call.
@@ -406,9 +411,7 @@ int check_table(const cpf::Program* prog, const cpf_target_table* tt, int64_t ba
   if (tt->n_targets < 1) return fail(CPF_ERR_INVALID, "target table: n_targets must be >= 1");
   if (!tt->targets) return fail(CPF_ERR_INVALID, "target table: targets is NULL");
   if (batch > 0 && !tt->target_index) return fail(CPF_ERR_INVALID, "target table: target_index is NULL");
-  if (tt->kind != CPF_LOSS_STATE && prog->n_qubits > 5)
-    return fail(CPF_ERR_UNSUPPORTED, "full-unitary losses need n <= 5 qubits (6-7 qubits: state preparation and "
-                                     "cpf_unitary only)");
+  if (int rc = check_full_unitary(prog, tt->kind)) return rc;
   for (int64_t b = 0; b < batch; ++b) {
     const int32_t t = tt->target_index[b];
     if (t < 0 || t >= tt->n_targets)
@@ -472,7 +475,7 @@ int launch_staged(const cpf::KParams<R>& p, const cpf::Program* prog, const cpf_
 template <typename R>
 int run_unitary(const cpf::Program* prog, int64_t batch, const void* angles, void* u_out, cudaStream_t st) {
   cpf::KParams<R> p;
-  // 6-7 qubits: a column per virtual sample on the single-column kernels (engine_impl.cuh: colmode)
+  // 6-8 qubits: a column per virtual sample on the single-column kernels (engine_impl.cuh: colmode)
   const bool colmode = prog->n_qubits > 5;
   int rc = fill_common(prog, p, colmode ? batch << prog->n_qubits : batch, colmode);
   if (rc) return rc;
@@ -902,9 +905,10 @@ template <typename R>
 static int iso_plan_t(const cpf::Program* prog, int32_t mask, int64_t batch, cpf_launch_info* out) {
   const int n = prog->n_qubits, n_su2 = (int)prog->su2.size(), n_cp = (int)prog->cp.size();
   const int k = iso_spec(prog, mask).k;
-  const cpf::DecodedSchedule ds = cpf::decode_schedule(*prog, cpf::engine_rb<R>(n, true));
+  const int rb = cpf::engine_rb<R>(n, true);
+  const cpf::DecodedSchedule ds = cpf::decode_schedule(*prog, rb);
   const int n_red = ds.red.empty() ? 1 : (int)(ds.red.size() / 8);
-  const cpf::IsoGeometry g = cpf::iso_geometry(n, k, n_su2, n_cp, (int)prog->sched.size(), n_red, sizeof(R));
+  const cpf::IsoGeometry g = cpf::iso_geometry(n, rb, k, n_su2, n_cp, (int)prog->sched.size(), n_red, sizeof(R));
   out->engine = 0;
   out->block_threads = g.block;
   out->samples_per_cta = g.spb;
@@ -1038,6 +1042,7 @@ int cpf_workspace_bytes(const cpf_program* prog, int32_t loss_kind, int32_t dtyp
   const cpf::Program* p = reinterpret_cast<const cpf::Program*>(prog);
   int32_t kind, mask;
   int rc = split_kind(p, loss_kind, &kind, &mask);
+  if (!rc) rc = check_full_unitary(p, kind);
   if (rc) return rc;
   *bytes = dtype == CPF_F64 ? workspace_bytes_t<double>(p, kind, mask, batch) : workspace_bytes_t<float>(p, kind, mask, batch);
   return CPF_OK;
@@ -1087,6 +1092,7 @@ int cpf_workspace_bytes_multi(const cpf_program* prog, int32_t loss_kind, int32_
   if (n_targets < 1) return fail(CPF_ERR_INVALID, "n_targets must be >= 1");
   if (dtype != CPF_F32 && dtype != CPF_F64) return fail(CPF_ERR_INVALID, "unknown dtype");
   const cpf::Program* p = reinterpret_cast<const cpf::Program*>(prog);
+  if (int rc = check_full_unitary(p, loss_kind)) return rc;
   *bytes = dtype == CPF_F64 ? workspace_bytes_multi_t<double>(p, loss_kind, batch, n_targets)
                             : workspace_bytes_multi_t<float>(p, loss_kind, batch, n_targets);
   return CPF_OK;

@@ -14,6 +14,7 @@ int launch_engine<double>(const KParams<double>& p, int n, bool single, cudaStre
       case 5: return launch_one<double, 5, 1, 1, true>(p, st, err);
       case 6: return launch_one<double, 6, 2, 1, true>(p, st, err);
       case 7: return launch_one<double, 7, 2, 1, true>(p, st, err);
+      case 8: return launch_one<double, 8, 3, 1, true>(p, st, err);
     }
   } else {
     switch (n) {
@@ -23,15 +24,17 @@ int launch_engine<double>(const KParams<double>& p, int n, bool single, cudaStre
       case 5: return launch_one<double, 5, 5, 1, false>(p, st, err);
     }
   }
-  err = single ? "unsupported number of qubits"
-               : "full-unitary losses need n <= 5 qubits (6-7 qubits: state preparation and cpf_unitary only)";
+  err = single ? "unsupported number of qubits" : FULL_UNITARY_LIMIT;
   return CPF_ERR_UNSUPPORTED;
 }
 
 template <>
 int engine_rb<double>(int n, bool single) {
   if (single) {
-    switch (n) { case 2: return 2; case 3: return 2; case 4: return 1; case 5: return 1; case 6: return 2; case 7: return 2; }
+    switch (n) {
+      case 2: return 2; case 3: return 2; case 4: return 1; case 5: return 1; case 6: return 2; case 7: return 2;
+      case 8: return 3;
+    }
   } else {
     switch (n) { case 2: return 2; case 3: return 2; case 4: return 3; case 5: return 5; }
   }

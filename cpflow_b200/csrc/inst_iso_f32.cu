@@ -1,5 +1,5 @@
-// Isometry kernels on 6-7 qubits, float32 / complex64 (iso_impl.cuh).  The decoded schedule is the one of the single-column
-// kernels with 2 register bits (engine_rb of 6-7 qubits).
+// Isometry kernels on 6-8 qubits, float32 / complex64 (iso_impl.cuh).  The decoded schedule is the one of the single-column
+// kernels (engine_rb: 2 register bits on 6-7 qubits, 3 on 8).
 #include "iso_impl.cuh"
 
 namespace cpf {
@@ -9,8 +9,9 @@ int launch_iso<float>(const KParams<float>& p, int n, cudaStream_t st, std::stri
   switch (n) {
     case 6: return launch_iso_sized<float, 6>(p, st, err);
     case 7: return launch_iso_sized<float, 7>(p, st, err);
+    case 8: return launch_iso_sized<float, 8>(p, st, err);
   }
-  err = "the isometry kernel runs 6-7 qubits (n <= 5: the HS kernels)";
+  err = "the isometry kernel runs 6-8 qubits (n <= 5: the HS kernels)";
   return CPF_ERR_UNSUPPORTED;
 }
 

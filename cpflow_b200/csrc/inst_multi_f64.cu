@@ -30,6 +30,7 @@ int launch_engine_multi<double>(const KParams<double>& p, int n, bool single, cu
       case 5: return launch_one<double, 5, 1, 1, true, InterpSweepMT<double, 5, 1, 1, true>>(p, st, err);
       case 6: return launch_one<double, 6, 2, 1, true, InterpSweepMT<double, 6, 2, 1, true>>(p, st, err);
       case 7: return launch_one<double, 7, 2, 1, true, InterpSweepMT<double, 7, 2, 1, true>>(p, st, err);
+      case 8: return launch_one<double, 8, 3, 1, true, InterpSweepMT<double, 8, 3, 1, true>>(p, st, err);
     }
   } else {
     switch (n) {
@@ -39,8 +40,7 @@ int launch_engine_multi<double>(const KParams<double>& p, int n, bool single, cu
       case 5: return launch_one<double, 5, 5, 1, false, InterpSweepMT<double, 5, 5, 1, false>>(p, st, err);
     }
   }
-  err = single ? "unsupported number of qubits"
-               : "full-unitary losses need n <= 5 qubits (6-7 qubits: state preparation and cpf_unitary only)";
+  err = single ? "unsupported number of qubits" : FULL_UNITARY_LIMIT;
   return CPF_ERR_UNSUPPORTED;
 }
 

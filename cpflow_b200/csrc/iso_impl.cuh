@@ -1,8 +1,9 @@
-// Isometry loss on 6-7 qubits (DESIGN.md section 2.4): L = 1 - |sum_c <W e_c| U |s_c>|^2 / k^2, where the s_c are the
+// Isometry loss on 6-8 qubits (DESIGN.md section 2.4): L = 1 - |sum_c <W e_c| U |s_c>|^2 / k^2, where the s_c are the
 // k basis states whose ancilla bits are 0 and W is the N x k matrix of their wanted images.
 //
-// A variant of engine_kernel's single-column interpreter (RB = 2 register bits, 2^(n-2) lanes per column): one sample
-// is k lane groups, one per input column s_c, so a sample spans up to 1024 threads and several warps.  The sample's
+// A variant of engine_kernel's single-column interpreter (RB register bits, 2^(n-RB) lanes per column, the split of
+// the single-column kernels: RB = 2 on 6-7 qubits, 16 / 32 lanes; RB = 3 on 8 qubits, 32 lanes): one sample is k lane
+// groups, one per input column s_c, so a sample spans up to 1024 threads and several warps.  The sample's
 // threads build ONE shared coefficient store per step; each group runs the forward sweep from e_{s_c}; the groups'
 // partial overlaps are summed in a fixed order through shared memory, and every group seeds its adjoint with the same
 // t (the HS seed with NN = k^2 and its own column of W).  The backward sweep must not overwrite coefficients another
@@ -17,12 +18,16 @@
 
 namespace cpf {
 
+// Register bits of the isometry kernel on NQ qubits: those of the single-column kernels (engine_rb(NQ, true)), whose
+// decoded schedule it runs; a lane group (one column) stays within one warp.
+template <int NQ> constexpr int iso_rb() { return NQ == 8 ? 3 : 2; }
+
 template <typename R, int NQ>
-struct InterpSweepIso : InterpSweep<R, NQ, 2, 1, true> {
-  using Base = InterpSweep<R, NQ, 2, 1, true>;
+struct InterpSweepIso : InterpSweep<R, NQ, iso_rb<NQ>(), 1, true> {
+  using Base = InterpSweep<R, NQ, iso_rb<NQ>(), 1, true>;
   using CO = typename Base::CO;
   using V = typename Base::V;
-  static constexpr int NA = Base::NA, LB = Base::LB, TPS = Base::TPS, RB = 2;
+  static constexpr int NA = Base::NA, LB = Base::LB, TPS = Base::TPS, RB = iso_rb<NQ>();
   static constexpr bool ISOMETRY = true;
   // InterpSweep::backward with the reduced sums stored at `sums` (this group's slots, reduce table re-pointed) instead
   // of over the coefficients, which the other groups of the sample may still be reading.
@@ -248,10 +253,11 @@ __host__ __device__ inline int iso_sample_words(int coef_stride, int k, int sum_
 
 template <typename R, int NQ, typename SW>
 __global__ void __launch_bounds__(NQ == 6 ? 512 : 1024, 1) iso_kernel(const KParams<R> p) {
-  using C = Cfg<R, NQ, 2, 1, true>;
+  constexpr int RB = SW::RB;
+  using C = Cfg<R, NQ, RB, 1, true>;
   using T = VT<R, 1>;
   using V = typename T::V;
-  constexpr int N = C::N, GT = C::TPS, NA = C::NA, RB = 2;
+  constexpr int N = C::N, GT = C::TPS, NA = C::NA;
   static_assert(SW::ISOMETRY, "iso_kernel runs the isometry sweep type");
 
   extern __shared__ __align__(16) unsigned char smem_raw[];
@@ -371,7 +377,7 @@ __global__ void __launch_bounds__(NQ == 6 ? 512 : 1024, 1) iso_kernel(const KPar
   }
 }
 
-// Target packing for the 6-7 qubit kernel: W (N x k, row-major complex) -> column-major [k][N] complex, so a group
+// Target packing for the 6-8 qubit kernel: W (N x k, row-major complex) -> column-major [k][N] complex, so a group
 // reads its column's amplitudes contiguously.
 template <typename R>
 __global__ void pack_iso_kernel(const R* __restrict__ src, R* __restrict__ dst, int N, int k) {
@@ -405,9 +411,9 @@ struct IsoGeometry {
   int spt, spb, block;
   size_t smem;
 };
-inline IsoGeometry iso_geometry(int n, int k, int n_su2, int n_cp, int n_sched, int n_red, size_t real_bytes) {
+inline IsoGeometry iso_geometry(int n, int rb, int k, int n_su2, int n_cp, int n_sched, int n_red, size_t real_bytes) {
   IsoGeometry g;
-  g.spt = k << (n - 2);
+  g.spt = k << (n - rb);
   g.spb = g.spt >= 128 ? 1 : 128 / g.spt;
   g.block = g.spb * g.spt;
   const int words = iso_sample_words(coef_stride_words(n_su2, n_cp), k, iso_sum_stride(n_su2, n_cp));
@@ -420,7 +426,11 @@ int launch_iso_sized(KParams<R> p, cudaStream_t st, std::string& err) {
   using SW = InterpSweepIso<R, NQ>;
   p.coef_stride = coef_stride_words(p.n_su2, p.n_cp);
   p.sync_sweeps = 0;
-  const IsoGeometry g = iso_geometry(NQ, p.iso_k, p.n_su2, p.n_cp, p.n_sched, p.n_red, sizeof(R));
+  if (engine_rb<R>(NQ, true) != SW::RB) {        // the decoded schedule in p is the one of engine_rb's split
+    err = "isometry kernel: register bits differ from the decoded schedule's";
+    return CPF_ERR_UNSUPPORTED;
+  }
+  const IsoGeometry g = iso_geometry(NQ, SW::RB, p.iso_k, p.n_su2, p.n_cp, p.n_sched, p.n_red, sizeof(R));
   if (g.smem > 227 * 1024) {
     err = "program too large for the shared-memory store of the isometry kernel (" + std::to_string(g.smem) + " bytes)";
     return CPF_ERR_UNSUPPORTED;

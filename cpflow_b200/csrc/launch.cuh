@@ -6,6 +6,10 @@
 
 namespace cpf {
 
+// refusal of HS and relative-phase losses above 5 qubits (the full-unitary kernels stop at n = 5)
+constexpr char FULL_UNITARY_LIMIT[] =
+    "full-unitary losses need n <= 5 qubits (6-8 qubits: state preparation, isometries and cpf_unitary only)";
+
 inline int coef_stride_words(int n_su2, int n_cp) {
   int w = (coef_words(n_su2, n_cp) + 3) & ~3;
   if (w == 0) w = 4;

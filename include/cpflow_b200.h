@@ -37,7 +37,7 @@ extern "C" {
 #endif
 
 #define CPF_VERSION 200 /* 0.2.0 */
-#define CPF_MAX_QUBITS 7
+#define CPF_MAX_QUBITS 8
 #define CPF_MAX_SEGMENTS 16
 
 typedef enum cpf_status {
@@ -83,8 +83,8 @@ typedef enum cpf_loss_kind {
 /* ISOMETRY: the qubits of `ancilla_mask` (bit q = qubit q) start in |0>, so only the images of the k = 2^(n - popcount)
  * basis states s_0 < ... < s_{k-1} whose ancilla bits are 0 matter; column c of the N x k target W is the wanted
  * image of |s_c>.  One global phase, like HS: ancilla_mask = 0 is the HS loss, all qubits (k = 1) the state loss.
- * n <= 5 runs on the HS kernels (target 2^a [W at the columns s_c, 0 elsewhere], N = 2^a k: exact scaling); n = 6, 7
- * on the isometry kernel with k <= 32 (k = 64 and ancilla_mask = 0 are CPF_ERR_UNSUPPORTED).  Not for multi-target
+ * n <= 5 runs on the HS kernels (target 2^a [W at the columns s_c, 0 elsewhere], N = 2^a k: exact scaling); n = 6-8
+ * on the isometry kernel with k <= 32 (k > 32 and ancilla_mask = 0 are CPF_ERR_UNSUPPORTED).  Not for multi-target
  * tables.  A mask bit at a position >= n is CPF_ERR_INVALID. */
 typedef struct cpf_loss_spec {
   int32_t kind;       /* cpf_loss_kind */
