@@ -13,7 +13,7 @@ import torch
 
 from . import _lib as L
 from .engine import Loss, TorchLoss, _DT, _ptr, _stream
-from .optimization import RawResults, run_adam_batch
+from .optimization import RawResults, run_adam_batch, torch_loss_chunk
 
 
 def random_cp_angles(anz, num_samples=1, cp_dist='uniform', seed=0, first=0, count=None,
@@ -160,7 +160,8 @@ def verify_cp_results(results, anz, unitary_loss_func, options, keep_history=Fal
     angles = torch.stack([p.to(device, dtype) for p in picks]).contiguous()
     cz, proj, frozen = prog.count_cz(angles, options.threshold_cp, project=True)
     raw = run_adam_batch(prog, unitary_loss_func, None, proj, options.learning_rate_at_verification,
-                         options.num_gd_iterations_at_verification, freeze=frozen, keep_history=False)
+                         options.num_gd_iterations_at_verification, freeze=frozen, keep_history=False,
+                         chunk=torch_loss_chunk(prog, dtype))
     best_i = torch.argmin(raw.regloss, dim=1)
     idx = torch.arange(len(raw), device=angles.device)
     best_loss = raw.regloss[idx, best_i].cpu().numpy()

@@ -524,9 +524,45 @@ int run_loss_grad(const cpf::Program* prog, const cpf_loss_spec* loss, const cpf
   return rc;
 }
 
+// 6-8 qubits: the cotangent mode of the isometry kernel (iso_impl.cuh: InterpSweepIsoCot), one launch item per
+// (sample, chunk of k_c columns), each item's gradient in a scratch row; the rows of a sample are then added in chunk
+// order.  k_c depends on the program and the precision only, so a sample's gradient does not depend on the batch.
+template <typename R>
+int run_cotangent_iso(const cpf::Program* prog, int64_t batch, const void* angles, const void* cot, void* grad_out,
+                      cudaStream_t st) {
+  const int n = prog->n_qubits;
+  cpf::KParams<R> p;
+  int rc = fill_common(prog, p, batch, true);
+  if (rc) return rc;
+  const int kc = cpf::iso_cot_columns(n, cpf::engine_rb<R>(n, true), p.n_su2, p.n_cp, p.n_sched, p.n_red, sizeof(R));
+  if (kc == 0)
+    return fail(CPF_ERR_UNSUPPORTED, "program too large for cpf_adjoint_from_cotangent on " + std::to_string(n) +
+                                     " qubits: the shared-memory store of one column does not fit 227 KB");
+  const int n_chunks = (1 << n) / kc;
+  p.mode = cpf::M_COTANGENT;
+  p.B = batch * n_chunks;
+  p.iso_k = kc;
+  p.angles = (R*)angles; p.cot = (const R*)cot;
+  Scratch sc;
+  sc.st = st;
+  R* partial = nullptr;
+  const size_t pbytes = (size_t)p.B * prog->n_params * sizeof(R);
+  rc = sc.get((void**)&partial, pbytes);
+  if (rc) return rc;
+  // parameters that feed no gate get no row entry from the kernel
+  CPF_CUDA(cudaMemsetAsync(partial, 0, pbytes, st));
+  p.grad_out = partial;
+  std::string err;
+  rc = cpf::launch_iso_cot<R>(p, n, st, err);
+  if (rc) return fail(rc, err);
+  rc = cpf::launch_cot_reduce<R>(partial, (R*)grad_out, batch, prog->n_params, n_chunks, st);
+  return rc ? fail(rc, "cot_reduce launch failed") : CPF_OK;
+}
+
 template <typename R>
 int run_cotangent(const cpf::Program* prog, int64_t batch, const void* angles, const void* cot,
                   void* grad_out, cudaStream_t st) {
+  if (prog->n_qubits > 5) return run_cotangent_iso<R>(prog, batch, angles, cot, grad_out, st);
   cpf::KParams<R> p;
   int rc = fill_common(prog, p, batch);
   if (rc) return rc;

@@ -29,6 +29,7 @@ struct InterpSweepIso : InterpSweep<R, NQ, iso_rb<NQ>(), 1, true> {
   using V = typename Base::V;
   static constexpr int NA = Base::NA, LB = Base::LB, TPS = Base::TPS, RB = iso_rb<NQ>();
   static constexpr bool ISOMETRY = true;
+  static constexpr bool COTANGENT = false;
   // InterpSweep::backward with the reduced sums stored at `sums` (this group's slots, reduce table re-pointed) instead
   // of over the coefficients, which the other groups of the sample may still be reading.
   static __device__ __forceinline__ void backward_into(const KParams<R>& p, const R* coef, R* sums, const uint2* s_dec,
@@ -101,6 +102,16 @@ struct InterpSweepIso : InterpSweep<R, NQ, iso_rb<NQ>(), 1, true> {
     }
   }
   }
+};
+
+// The cotangent mode of iso_kernel (cpf_adjoint_from_cotangent on 6-8 qubits, DESIGN.md section 2.4): a launch item
+// is (sample b / n_chunks, column chunk b % n_chunks) with n_chunks = N / k; group c runs input column
+// (b % n_chunks) * k + c and seeds its adjoint with that column of the caller's cotangent instead of the loss seed.
+// The item's gradient (its groups' sums added in group order) goes to row b of a scratch array that
+// launch_cot_reduce sums over the chunks in increasing order.
+template <typename R, int NQ>
+struct InterpSweepIsoCot : InterpSweepIso<R, NQ> {
+  static constexpr bool COTANGENT = true;
 };
 
 // words per group of the per-group gradient sums (odd: the groups of a sample store the same slot in distinct banks)
@@ -287,10 +298,12 @@ __global__ void __launch_bounds__(NQ == 6 ? 512 : 1024, 1) iso_kernel(const KPar
   R* coef = s_smp + (size_t)sl * iso_sample_words(p.coef_stride, k, sum_stride);
   R* sums = coef + p.coef_stride;
   R* part = sums + (size_t)k * sum_stride;         // [k][3]: Re t_c, Im t_c, penalty share of group c
-  const R* tv = p.target_packed + 2 * ((size_t)grp * N + (la << RB));
-  const int col0 = iso_column(grp, p.iso_amask, NQ);
+  const R* tv = SW::COTANGENT ? nullptr : p.target_packed + 2 * ((size_t)grp * N + (la << RB));
+  // cotangent mode: item b is column chunk b % (N / k) of sample b / (N / k)
+  const long long bs = SW::COTANGENT ? b / (N / k) : b;
+  const int col0 = SW::COTANGENT ? (int)(b % (N / k)) * k + grp : iso_column(grp, p.iso_amask, NQ);
 
-  R* ang = p.angles + b * P;
+  R* ang = p.angles + bs * P;
   R* mom = p.m ? p.m + b * P : nullptr;
   R* vel = p.v ? p.v + b * P : nullptr;
   const uint8_t* frz = p.freeze ? p.freeze + b * P : nullptr;
@@ -310,6 +323,19 @@ __global__ void __launch_bounds__(NQ == 6 ? 512 : 1024, 1) iso_kernel(const KPar
 #pragma unroll
     for (int r = 0; r < NA; ++r) { pr[r] = T::onehot((la << RB) | r, col0); pi[r] = T::bc(R(0)); }
     SW::forward(p, coef, s_dec, la, pr, pi);
+
+    if constexpr (SW::COTANGENT) {
+      // the adjoint seed is column col0 of cot[bs] (row-major [N][N] complex), read directly
+      V lr[NA], li[NA];
+#pragma unroll
+      for (int j = 0; j < NA; ++j) {
+        const R* src = p.cot + ((bs * N + ((la << RB) | j)) * N + col0) * 2;
+        lr[j] = src[0]; li[j] = src[1];
+      }
+      SW::backward_into(p, coef, sums + (size_t)grp * sum_stride, s_dec, s_red, la, la, pr, pi, lr, li);
+      __syncthreads();
+      continue;
+    }
 
     // ---------------- overlap: group partials, then the same fixed-order sum in every thread ----------------
     {
@@ -406,6 +432,19 @@ __global__ void pack_iso_hs_kernel(const R* __restrict__ src, R* __restrict__ ds
   }
 }
 
+// grad[b, i] = sum over h of partial[b * n_chunks + h, i], in increasing h (the cotangent mode's chunk sum)
+template <typename R>
+__global__ void cot_reduce_kernel(const R* __restrict__ partial, R* __restrict__ grad, long long B, int P,
+                                  int n_chunks) {
+  for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < B * P;
+       i += (long long)gridDim.x * blockDim.x) {
+    const R* s = partial + (i / P) * n_chunks * P + i % P;
+    R x = s[0];
+    for (int h = 1; h < n_chunks; ++h) x += s[(size_t)h * P];
+    grad[i] = x;
+  }
+}
+
 // host side: geometry of one launch (also reported by cpf_launch_plan)
 struct IsoGeometry {
   int spt, spb, block;
@@ -421,9 +460,16 @@ inline IsoGeometry iso_geometry(int n, int rb, int k, int n_su2, int n_cp, int n
   return g;
 }
 
-template <typename R, int NQ>
+// Columns per launch item of the cotangent mode: 32 (the k = 32 isometry launch shape), halved until the item's
+// shared memory fits; a function of the program and the precision only.  0: not even one column fits.
+inline int iso_cot_columns(int n, int rb, int n_su2, int n_cp, int n_sched, int n_red, size_t real_bytes) {
+  for (int k = 32; k >= 1; k >>= 1)
+    if (iso_geometry(n, rb, k, n_su2, n_cp, n_sched, n_red, real_bytes).smem <= 227 * 1024) return k;
+  return 0;
+}
+
+template <typename R, int NQ, typename SW = InterpSweepIso<R, NQ>>
 int launch_iso_sized(KParams<R> p, cudaStream_t st, std::string& err) {
-  using SW = InterpSweepIso<R, NQ>;
   p.coef_stride = coef_stride_words(p.n_su2, p.n_cp);
   p.sync_sweeps = 0;
   if (engine_rb<R>(NQ, true) != SW::RB) {        // the decoded schedule in p is the one of engine_rb's split
@@ -449,6 +495,10 @@ int launch_iso_sized(KParams<R> p, cudaStream_t st, std::string& err) {
 
 // inst_iso_f32.cu / inst_iso_f64.cu
 template <typename R> int launch_iso(const KParams<R>& p, int n_qubits, cudaStream_t st, std::string& err);
+// cotangent mode: p.B launch items of p.iso_k columns (p.B = batch * N / p.iso_k), gradients to p.grad_out [p.B][P]
+template <typename R> int launch_iso_cot(const KParams<R>& p, int n_qubits, cudaStream_t st, std::string& err);
+template <typename R> int launch_cot_reduce(const R* partial, R* grad, long long batch, int P, int n_chunks,
+                                            cudaStream_t st);
 template <typename R> int launch_pack_iso(const R* src, R* dst, int n_qubits, int k, int amask, bool as_hs,
                                           cudaStream_t st);
 

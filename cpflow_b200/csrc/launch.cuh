@@ -6,9 +6,10 @@
 
 namespace cpf {
 
-// refusal of HS and relative-phase losses above 5 qubits (the full-unitary kernels stop at n = 5)
+// refusal of the fused HS and relative-phase losses above 5 qubits (the full-unitary kernels stop at n = 5)
 constexpr char FULL_UNITARY_LIMIT[] =
-    "full-unitary losses need n <= 5 qubits (6-8 qubits: state preparation, isometries and cpf_unitary only)";
+    "full-unitary losses need n <= 5 qubits (6-8 qubits: state preparation, isometries, cpf_unitary and "
+    "cpf_adjoint_from_cotangent, so a full-unitary loss runs there as a callable on the host-driven loop)";
 
 inline int coef_stride_words(int n_su2, int n_cp) {
   int w = (coef_words(n_su2, n_cp) + 3) & ~3;

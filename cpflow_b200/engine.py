@@ -446,7 +446,11 @@ class TorchLoss:
     a function of ONE unitary (complex tensor [N,N]) returning a real scalar tensor.  It cannot run inside the
     fused kernel, so the optimisation alternates cpf_unitary -> this function and its autograd cotangent ->
     cpf_adjoint_from_cotangent -> cpf_adam_step (optimization.run_adam_batch); the Adam arithmetic, penalty, best
-    tracking and freeze masks are the engine's own."""
+    tracking and freeze masks are the engine's own.  Every stage runs on 2-8 qubits, so on 6-8 qubits this is the
+    route for full-unitary and custom objectives (the fused HS and relative-phase kinds stop at 5 qubits); U and its
+    cotangent take N^2 complex numbers per sample each (512 KiB at n = 8 in complex64), and Synthesize splits such runs
+    into sample chunks (optimization.torch_loss_chunk).  The result objects also call `fn` on host unitaries
+    (`Decomposition.loss`, `refine`), so it should work for a unitary on any device and of either precision."""
 
     def __init__(self, fn):
         if not callable(fn):

@@ -21,7 +21,7 @@ import torch
 
 from . import _lib as L
 from .circuit import Circuit, Gate, convert_to_ZXZ, cp_to_cz_circuit, gates_count, gates_depth  # noqa: F401
-from .engine import Program
+from .engine import Program, TorchLoss
 from .matrix_utils import cost_HST
 
 _ROT = {'rx': L.RX, 'ry': L.RY, 'rz': L.RZ}
@@ -65,6 +65,9 @@ def circuit_angle_program(qc):
 
 def _batched_loss(prog, loss, cand, device):
     a = torch.as_tensor(cand, dtype=torch.float64, device=device).contiguous()
+    if isinstance(loss, TorchLoss):     # a user loss: evaluated by torch on the candidates' unitaries
+        with torch.no_grad():
+            return loss.batch(prog.unitary(a)).cpu().numpy()
     lo, _, _ = prog.loss_grad(a, loss, None, want_grad=False)
     return lo.cpu().numpy()
 

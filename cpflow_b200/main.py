@@ -20,7 +20,7 @@ from .ansatz import Ansatz
 from .circuit import convert_to_ZXZ, cp_template_cz_count_depth, cp_to_cz_circuit, gates_count, gates_depth
 from .cp_utils import (filter_cp_results, random_cp_angles, select_batch, verify_cp_result, verify_cp_results)
 from .engine import Loss, MultiLoss, Penalty, TorchLoss
-from .optimization import ProgramLoss, RawResults, mynimize_repeated, run_adam_batch
+from .optimization import ProgramLoss, RawResults, mynimize_repeated, run_adam_batch, torch_loss_chunk
 from .penalty import PenaltyFunction, RegularizationOptions, make_regularization_function, tabulate_penalty
 from .matrix_utils import theoretical_lower_bound
 from .topology import fill_layers, num_qubits_from_layer
@@ -399,7 +399,8 @@ class Synthesize:
             ProgramLoss(anz.program, self.unitary_loss_func), anz.num_angles, method=options.method,
             learning_rate=options.learning_rate, num_iterations=options.num_gd_iterations,
             initial_params_batch=initial_angles_array, regularization_func=self._penalty(options.r),
-            keep_history=keep_history, dtype=self.dtype, device=dev, return_device=return_device)
+            keep_history=keep_history, dtype=self.dtype, device=dev, return_device=return_device,
+            chunk=torch_loss_chunk(anz.program, self.dtype))
         return raw
 
     def _evaluate_raw(self, raw_results, options, disable_tqdm=False):
@@ -481,7 +482,8 @@ class Synthesize:
                 cz, proj, frozen = anz.program.count_cz(angles, options.threshold_cp, project=True)
                 raw = run_adam_batch(anz.program, self.unitary_loss_func, None, proj,
                                      options.learning_rate_at_verification,
-                                     options.num_gd_iterations_at_verification, freeze=frozen)
+                                     options.num_gd_iterations_at_verification, freeze=frozen,
+                                     chunk=torch_loss_chunk(anz.program, self.dtype))
                 bi = torch.argmin(raw.regloss, dim=1)
                 ar = torch.arange(len(mine), device=dev)
                 out = torch.cat([raw.regloss[ar, bi].to(torch.float64)[:, None], cz.to(torch.float64)[:, None],

@@ -20,6 +20,27 @@ from . import _lib as L
 from .engine import Loss, MultiLoss, Penalty, Program, TorchLoss
 
 HISTORY_BYTES_LIMIT = 64 << 30
+# Bound on the unitaries one host-loop iteration of a TorchLoss run holds at once (U, and as much again for its
+# cotangent): Synthesize splits 6-8 qubit runs into sample chunks under it.
+TORCH_LOSS_U_BYTES = 2 << 30
+
+
+def torch_loss_chunk(program, dtype):
+    """Samples per chunk of a TorchLoss run on `program` that keep U [chunk,N,N] within TORCH_LOSS_U_BYTES: None
+    (one run) on n <= 5, where U is at most 8 KiB per sample in complex64."""
+    if program.n_qubits <= 5:
+        return None
+    per_sample = program.dim * program.dim * 2 * torch.tensor([], dtype=dtype).element_size()
+    return max(1, TORCH_LOSS_U_BYTES // per_sample)
+
+
+def chunk_ranges(batch, chunk):
+    """[start, stop) sample ranges of a run split into chunks of at most `chunk` samples (one range without)."""
+    if chunk is None or chunk >= batch:
+        return [(0, batch)]
+    if chunk < 1:
+        raise ValueError(f"chunk must be >= 1 (got {chunk})")
+    return [(i, min(i + chunk, batch)) for i in range(0, batch, chunk)]
 
 
 @dataclass
@@ -84,7 +105,10 @@ def run_adam_batch(program, loss, penalty, initial_params, learning_rate, num_it
     """Device-resident core: `initial_params` is a CUDA tensor [B,P] (not modified).  Returns
     RawResults on the device.  Restates jit(vmap(mynimize_particular)) (optimization.py:344-362).
     With `target_index` ([B] ints), `loss` is a MultiLoss and sample b runs against its target target_index[b], all in
-    one launch (cpf_adam_run_multi)."""
+    one launch (cpf_adam_run_multi).
+    With a TorchLoss, `chunk` (samples) splits the run into independent runs of at most that many samples, whose
+    results are those of the whole run: the host loop then holds U and its cotangent for one chunk only
+    (`torch_loss_chunk`).  The fused kernels ignore it."""
     if target_index is not None and not isinstance(loss, MultiLoss):
         raise TypeError("target_index needs a MultiLoss(kind, targets): a user loss function runs one target at a "
                         "time on the host-driven loop")
@@ -97,6 +121,12 @@ def run_adam_batch(program, loss, penalty, initial_params, learning_rate, num_it
         if need > HISTORY_BYTES_LIMIT:
             raise L.CpflowError(f"keep_history=True needs {need / 2**30:.1f} GiB for B={B}, T={T}, P={P}; "
                                 "use keep_history=False (the reference default for static())")
+    if isinstance(loss, TorchLoss) and len(chunk_ranges(B, chunk)) > 1:
+        parts = [run_adam_batch(program, loss, penalty, initial_params[i:j], learning_rate, num_iterations,
+                                freeze=None if freeze is None else freeze[i:j], keep_history=keep_history)
+                 for i, j in chunk_ranges(B, chunk)]
+        return RawResults(torch.cat([r.params for r in parts]), torch.cat([r.regloss for r in parts]),
+                          torch.cat([r.reg for r in parts]))
     with torch.cuda.device(initial_params.device):
         st = program.adam_state(initial_params.clone(), freeze=freeze, hist_len=T if keep_history else 0)
         if target_index is not None:
@@ -144,12 +174,13 @@ def mynimize_repeated(loss_func, num_params=None, method='adam', learning_rate=0
                       u_func=None, initial_params_batch=None, num_repeats=1, regularization_func=None,
                       keep_history=True, compute_losses=True, num_iterations=5000, dtype=torch.float32,
                       device='cuda', freeze_mask=None, return_device=False, zero_regularization=False,
-                      **kwargs):
+                      chunk=None, **kwargs):
     """Reference optimization.py:269-382 on the CUDA engine.
 
     loss_func: ProgramLoss; regularization_func: Penalty or None; initial_params_batch: (P,) or
     (B, P) array on the host (numpy / torch) or the device.  Returns one dict for a 1-D input, else
-    a list-like of B dicts with host numpy arrays (device tensors if return_device=True)."""
+    a list-like of B dicts with host numpy arrays (device tensors if return_device=True).  `chunk`: see
+    run_adam_batch."""
     if not isinstance(loss_func, ProgramLoss):
         raise TypeError("loss_func must be a ProgramLoss(program, Loss(...)): the CUDA engine takes a "
                         "declarative spec instead of a Python closure")
@@ -185,7 +216,7 @@ def mynimize_repeated(loss_func, num_params=None, method='adam', learning_rate=0
     if freeze_mask is not None:
         freeze_mask = _as_device_batch(freeze_mask, torch.uint8, device).reshape(-1, P)
     raw = run_adam_batch(program, loss_func.loss, regularization_func, init, learning_rate, num_iterations,
-                         freeze=freeze_mask, keep_history=keep_history)
+                         freeze=freeze_mask, keep_history=keep_history, chunk=chunk)
     if not return_device:
         raw = raw.numpy()
     if not compute_losses or (regularization_func is None and not zero_regularization):

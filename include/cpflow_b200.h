@@ -185,7 +185,12 @@ int cpf_loss_grad(const cpf_program* prog, const cpf_loss_spec* loss,
 
 /* Generic vector-Jacobian product for a user loss evaluated outside the engine on the
  * materialised unitary (cpflow/main.py:528-529 `unitary_loss_func`): given
- * cotangent[B,N,N] = dL/dconj(U) it returns grad[B,P] = 2 Re <cotangent, dU/dtheta>. */
+ * cotangent[B,N,N] = dL/dconj(U) it returns grad[B,P] = 2 Re <cotangent, dU/dtheta>, on 2-8 qubits.
+ * n <= 5 runs on the full-unitary kernels; n = 6-8 on the cotangent mode of the isometry kernel (one launch item
+ * per sample and chunk of up to 32 columns, the chunks' gradients added in a fixed order), which needs scratch of
+ * batch x (N / columns per item) x P reals from the device's stream-ordered pool.  A sample's gradient does not
+ * depend on its batch position or on the batch size.  A program whose shared-memory store does not fit even at one
+ * column per item is refused with CPF_ERR_UNSUPPORTED. */
 int cpf_adjoint_from_cotangent(const cpf_program* prog, int32_t dtype, int64_t batch,
                                const void* angles, const void* cotangent, void* grad_out,
                                void* stream);
