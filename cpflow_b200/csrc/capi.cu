@@ -126,19 +126,27 @@ int fill_common(const cpf::Program* prog, cpf::KParams<R>& p, int64_t batch, boo
 
 // layered templates run on their specialised kernel when one was compiled for the layer
 // (CPF_NO_LAYERED=1 forces the interpreter kernel: used by the tests to cover both)
-template <typename R>
-int launch_any(const cpf::KParams<R>& p, const cpf::Program* prog, bool single, cudaStream_t st,
-               std::string& err) {
+bool layered_kernels(const cpf::Program* prog) {
   const char* e = getenv("CPF_NO_LAYERED");
-  const bool no_layered = e && e[0] == '1';
+  return prog->layered && !(e && e[0] == '1');
+}
+
+// the state-adjoint kernels: the one compiled for the layer when `layered` and one exists, else the interpreter
+template <typename R>
+int launch_any(const cpf::KParams<R>& p, const cpf::Program* prog, bool single, bool layered, cudaStream_t st,
+               std::string& err) {
   int rc = CPF_OK;
-  if (prog->layered && !no_layered && cpf::launch_layered<R>(p, *prog, single, st, err, rc)) return rc;
+  if (layered && cpf::launch_layered<R>(p, *prog, single, st, err, rc)) return rc;
   return cpf::launch_engine<R>(p, prog->n_qubits, single, st, err);
 }
 
+// The penalty in the kernels' form.  Refuses a bad spec and a cp_mask that selects a parameter of no CP gate; the mask
+// itself goes to the device with upload_cp_mask.
 template <typename R>
-int fill_penalty(const cpf::Program* prog, const cpf_penalty_spec* pen, cpf::KParams<R>& p, Scratch& sc) {
-  cudaStream_t st = sc.st;
+int penalty_params(const cpf::Program* prog, const cpf_penalty_spec* pen, cpf::PenaltyT<R>* out) {
+  cpf::PenaltyT<R>& q = *out;
+  std::memset(&q, 0, sizeof(q));
+  q.kind = CPF_PEN_NONE;
   if (!pen || pen->kind == CPF_PEN_NONE) return CPF_OK;
   if (pen->kind != CPF_PEN_PIECEWISE && pen->kind != CPF_PEN_L1)
     return fail(CPF_ERR_INVALID, "unknown penalty kind");
@@ -146,58 +154,36 @@ int fill_penalty(const cpf::Program* prog, const cpf_penalty_spec* pen, cpf::KPa
     return fail(CPF_ERR_INVALID, "penalty n_segments out of range");
   if (pen->kind == CPF_PEN_PIECEWISE && !(pen->period > 0))
     return fail(CPF_ERR_INVALID, "penalty period must be positive");
-  p.pen.kind = pen->kind; p.pen.nseg = pen->n_segments;
-  p.pen.r = (R)pen->r; p.pen.period = (R)pen->period;
-  for (int s = 0; s < CPF_MAX_SEGMENTS; ++s) {
-    const bool on = pen->kind == CPF_PEN_PIECEWISE && s < pen->n_segments;
-    p.pen.lo[s] = on ? (R)pen->lo[s] : (R)INFINITY; p.pen.hi[s] = on ? (R)pen->hi[s] : (R)INFINITY;
-    p.pen.slope[s] = on ? (R)pen->slope[s] : R(0); p.pen.icpt[s] = on ? (R)pen->intercept[s] : R(0);
-  }
-  // ascending, disjoint segments (in the kernel's precision) can be searched instead of scanned
-  p.pen.sorted = pen->kind == CPF_PEN_PIECEWISE;
-  for (int s = 0; s < pen->n_segments && s < CPF_MAX_SEGMENTS && p.pen.sorted; ++s) {
-    if (!(p.pen.lo[s] <= p.pen.hi[s])) p.pen.sorted = 0;
-    if (s + 1 < pen->n_segments && !(p.pen.hi[s] <= p.pen.lo[s + 1])) p.pen.sorted = 0;
-  }
-  if (pen->cp_mask) {
-    // only parameters of CP gates may be penalised
+  // only parameters of CP gates may be penalised
+  if (pen->cp_mask)
     for (int i = 0; i < prog->n_params; ++i)
       if (pen->cp_mask[i] && !prog->is_cp_param[i])
         return fail(CPF_ERR_UNSUPPORTED, "cp_mask selects a parameter that does not feed a CP gate");
-    std::string flags(prog->cp.size(), '\0');
-    for (size_t k = 0; k < prog->cp.size(); ++k)
-      flags[k] = prog->cp[k].pidx >= 0 && pen->cp_mask[prog->cp[k].pidx] ? 1 : 0;
-    if (!flags.empty()) {
-      uint8_t* dev = nullptr;
-      int rc = sc.get((void**)&dev, flags.size());
-      if (rc) return rc;
-      // pageable source: the runtime stages the bytes before returning, so `flags` may die
-      CPF_CUDA(cudaMemcpyAsync(dev, flags.data(), flags.size(), cudaMemcpyHostToDevice, st));
-      p.cp_pen = dev;
-    }
+  q.kind = pen->kind; q.nseg = pen->n_segments;
+  q.r = (R)pen->r; q.period = (R)pen->period;
+  for (int s = 0; s < CPF_MAX_SEGMENTS; ++s) {
+    const bool on = pen->kind == CPF_PEN_PIECEWISE && s < pen->n_segments;
+    q.lo[s] = on ? (R)pen->lo[s] : (R)INFINITY; q.hi[s] = on ? (R)pen->hi[s] : (R)INFINITY;
+    q.slope[s] = on ? (R)pen->slope[s] : R(0); q.icpt[s] = on ? (R)pen->intercept[s] : R(0);
+  }
+  // ascending, disjoint segments (in the kernel's precision) can be searched instead of scanned
+  q.sorted = pen->kind == CPF_PEN_PIECEWISE;
+  for (int s = 0; s < pen->n_segments && s < CPF_MAX_SEGMENTS && q.sorted; ++s) {
+    if (!(q.lo[s] <= q.hi[s])) q.sorted = 0;
+    if (s + 1 < pen->n_segments && !(q.hi[s] <= q.lo[s + 1])) q.sorted = 0;
   }
   return CPF_OK;
 }
 
-template <typename R>
-int stage_target(const cpf::Program* prog, const cpf_loss_spec* loss, cpf::KParams<R>& p, bool single, Scratch& sc) {
-  cudaStream_t st = sc.st;
-  const int cpt = single ? 1 : cpf::cpt_for<R>(prog->n_qubits);
-  const int words = cpf::target_words<R>(prog->n_qubits, cpt, single);
-  const size_t bytes = ((size_t)words * sizeof(R) + 15) & ~(size_t)15;
-  R* packed = nullptr;
-  int rc = sc.get((void**)&packed, bytes);
-  if (rc) return rc;
-  if (bytes != (size_t)words * sizeof(R)) CPF_CUDA(cudaMemsetAsync(packed, 0, bytes, st));
-  rc = cpf::launch_pack_target<R>((const R*)loss->target, packed, prog->n_qubits, cpt, single, st);
-  if (rc) return fail(rc, "pack_target launch failed");
-  p.target_packed = packed;
-  p.target_bytes = (int)bytes;
-  p.loss_kind = loss->kind;
+// the cp_mask as one flag per CP gate, copied into its scratch block
+int upload_cp_mask(const cpf::Program* prog, const uint8_t* cp_mask, void* dev, cudaStream_t st) {
+  std::string flags(prog->cp.size(), '\0');
+  for (size_t k = 0; k < prog->cp.size(); ++k)
+    flags[k] = prog->cp[k].pidx >= 0 && cp_mask[prog->cp[k].pidx] ? 1 : 0;
+  // pageable source: the runtime stages the bytes before returning, so `flags` may die
+  CPF_CUDA(cudaMemcpyAsync(dev, flags.data(), flags.size(), cudaMemcpyHostToDevice, st));
   return CPF_OK;
 }
-
-struct cpf_loss_spec_kind_only { int32_t kind; };
 
 // Per-call scratch (packed optimiser state, staged targets) comes from the device's default stream-ordered pool.
 // Its release threshold defaults to 0: freed blocks go back to the driver at the next synchronisation and the
@@ -217,72 +203,13 @@ static void keep_pool_memory() {
   done[dev] = true;
 }
 
-// ---- Heisenberg-picture kernels (heis_impl.cuh): HS loss on layered templates ----
-// CPF_ENGINE=adjoint forces the state-adjoint kernels (tests cover both engines).
+// The target-independent part of the heis set-up: per-gate scratch (`aux_pad` bytes at the start of `blk`) followed by
+// the packed optimiser state, gate-pattern flags.
 template <typename R>
-bool use_heis(const cpf::Program* prog, const cpf_loss_spec* loss) {
-  if (loss->kind != CPF_LOSS_HS || !prog->layered) return false;
-  // the kernel's shared-memory metadata holds parameter and slot indices in 16 bits (heis_impl.cuh: HSu2, HCp)
-  if (prog->n_params > 32767 || prog->su2.size() > 32767) return false;
-  const char* e = getenv("CPF_ENGINE");
-  if (e && std::strcmp(e, "adjoint") == 0) return false;
-  const char* nl = getenv("CPF_NO_LAYERED");
-  if (nl && nl[0] == '1') return false;
-  cpf::KParams<R> dummy;
-  std::string err;
-  int rc = 0;
-  return cpf::launch_heis<R>(dummy, *prog, nullptr, err, rc, true);
-}
-
-// bytes of the two heis scratch blocks: staged target; per-gate scratch followed by the packed optimiser state
-template <typename R>
-void heis_scratch_sizes(const cpf::Program* prog, int64_t batch, size_t* target_bytes, size_t* aux_pad, size_t* pk_bytes) {
+void stage_heis_state(const cpf::Program* prog, cpf::KParams<R>& p, void* blk, size_t aux_pad) {
   const int cpt = cpf::heis_cpt<R>(prog->n_qubits);
-  const int words = cpf::heis_target_words<R>(prog->n_qubits, cpt);
-  *target_bytes = ((size_t)words * sizeof(R) + 15) & ~(size_t)15;
-  const size_t aux_bytes = (size_t)batch * (prog->su2.empty() ? 1 : prog->su2.size()) * 4 * sizeof(R);
-  *aux_pad = (aux_bytes + 255) & ~(size_t)255;      // the packed state starts on a 256-byte boundary (blocks of 16 positions)
-  // lane-interleaved packed optimiser state (heis_impl.cuh: heis_pk_stride words per sample)
-  const int tps = (1 << prog->n_qubits) / cpt;
-  *pk_bytes = (size_t)batch * (size_t)cpf::heis_pk_stride(prog->n_qubits, tps, (int)prog->su2.size(), (int)prog->cp.size()) *
-              sizeof(R);
-}
-
-template <typename R>
-int stage_heis_state(const cpf::Program* prog, cpf::KParams<R>& p, Scratch& sc);
-
-template <typename R>
-int stage_heis(const cpf::Program* prog, const cpf_loss_spec* loss, cpf::KParams<R>& p, Scratch& sc) {
-  cudaStream_t st = sc.st;
-  if (!sc.base) keep_pool_memory();
-  const int cpt = cpf::heis_cpt<R>(prog->n_qubits);
-  const int words = cpf::heis_target_words<R>(prog->n_qubits, cpt);
-  size_t bytes, aux_pad, pk_bytes;
-  heis_scratch_sizes<R>(prog, p.B, &bytes, &aux_pad, &pk_bytes);
-  R* packed = nullptr;
-  int rc = sc.get((void**)&packed, bytes);
-  if (rc) return rc;
-  if (bytes != (size_t)words * sizeof(R)) CPF_CUDA(cudaMemsetAsync(packed, 0, bytes, st));
-  rc = cpf::launch_pack_target_heis<R>((const R*)loss->target, packed, prog->n_qubits, cpt, st);
-  if (rc) return fail(rc, "pack_target_heis launch failed");
-  p.target_packed = packed;
-  p.target_bytes = (int)bytes;
-  p.loss_kind = loss->kind;
-  return stage_heis_state(prog, p, sc);
-}
-
-// the target-independent part of the heis set-up: per-gate scratch and packed optimiser state, gate-pattern flags
-template <typename R>
-int stage_heis_state(const cpf::Program* prog, cpf::KParams<R>& p, Scratch& sc) {
-  const int cpt = cpf::heis_cpt<R>(prog->n_qubits);
-  size_t bytes, aux_pad, pk_bytes;
-  heis_scratch_sizes<R>(prog, p.B, &bytes, &aux_pad, &pk_bytes);
-  R* aux = nullptr;
-  // one block: per-gate scratch, then the packed optimiser state (32-byte aligned)
-  int rc = sc.get((void**)&aux, aux_pad + pk_bytes);
-  if (rc) return rc;
-  p.pk = reinterpret_cast<char*>(aux) + aux_pad;
-  p.aux = aux;
+  p.pk = reinterpret_cast<char*>(blk) + aux_pad;
+  p.aux = reinterpret_cast<R*>(blk);
   // rotation-axis pattern shared by the surface gates (slots < n) and by the block gates (the rest)
   auto pattern = [&](size_t lo, size_t hi) {
     int pat = -1;
@@ -312,33 +239,11 @@ int stage_heis_state(const cpf::Program* prog, cpf::KParams<R>& p, Scratch& sc) 
   }
   p.unreferenced_params = referenced != prog->n_params;      // (a parameter feeds at most one gate: program.cpp)
   p.pk_stride = cpf::heis_pk_stride(prog->n_qubits, (1 << prog->n_qubits) / cpt, (int)prog->su2.size(), (int)prog->cp.size());
-  return CPF_OK;
-}
-
-// HS and relative-phase losses run on the full-unitary kernels, which stop at 5 qubits: refused before any CUDA call.
-int check_full_unitary(const cpf::Program* prog, int32_t kind) {
-  if ((kind == CPF_LOSS_HS || kind == CPF_LOSS_RELPHASE) && prog->n_qubits > 5)
-    return fail(CPF_ERR_UNSUPPORTED, cpf::FULL_UNITARY_LIMIT);
-  return CPF_OK;
 }
 
 // ---- isometry loss (CPF_LOSS_ISOMETRY) ----
 // Largest number of input columns k of the 6-8 qubit kernel: a sample is k lane groups of 2^(n-RB) threads in one CTA.
 constexpr int ISO_MAX_K = 32;
-
-// Everything about an isometry request that can be refused is refused here, before any CUDA call.
-int check_iso(const cpf::Program* prog, int32_t mask) {
-  const int n = prog->n_qubits;
-  if (mask < 0 || (mask >> n) != 0)
-    return fail(CPF_ERR_INVALID, "ancilla_mask " + std::to_string(mask) + " names a qubit >= n = " + std::to_string(n));
-  if (n > 5 && mask == 0)
-    return fail(CPF_ERR_UNSUPPORTED, cpf::FULL_UNITARY_LIMIT);
-  const int k = 1 << (n - __builtin_popcount((unsigned)mask));
-  if (n > 5 && k > ISO_MAX_K)
-    return fail(CPF_ERR_UNSUPPORTED, "isometry losses on 6-8 qubits take at most k = " + std::to_string(ISO_MAX_K) +
-                                     " input columns (k = 2^(n - popcount(ancilla_mask)) = " + std::to_string(k) + ")");
-  return CPF_OK;
-}
 
 // k input columns; the ancilla qubits as amplitude-index bits (qubit q is bit n - 1 - q, big-endian)
 struct IsoSpec { int k, amask; };
@@ -350,126 +255,212 @@ IsoSpec iso_spec(const cpf::Program* prog, int32_t mask) {
   return s;
 }
 
-// The query entry points take a loss kind only: an isometry kind carries its ancilla mask in bits 8-15
-// (CPF_ISOMETRY_KIND).  Splits and checks such an argument.
-int split_kind(const cpf::Program* prog, int32_t arg, int32_t* kind, int32_t* mask) {
-  *kind = arg & 0xff;
-  *mask = (arg >> 8) & 0xff;
-  if (*kind < CPF_LOSS_HS || *kind > CPF_LOSS_ISOMETRY || (arg >> 16) != 0 || (*kind != CPF_LOSS_ISOMETRY && *mask))
-    return fail(CPF_ERR_INVALID, "unknown loss kind");
-  return *kind == CPF_LOSS_ISOMETRY ? check_iso(prog, *mask) : CPF_OK;
-}
+// ---- the plan of a loss call ----
+// Which kernel runs a loss call and which scratch blocks it needs, decided on the host.  The staged calls and the query
+// entry points all read it, so the size cpf_workspace_bytes reports is the sum of the blocks run_staged carves.
+enum Route { ROUTE_ADJOINT, ROUTE_HEIS, ROUTE_ISO };
+// scratch blocks, in carve order
+enum Block { BLK_MASK, BLK_V, BLK_INDEX, BLK_TARGET, BLK_HEIS, N_BLK };
 
-// n <= 5: the isometry loss is the HS loss on V = 2^a [W at the columns s_c, 0 elsewhere] (iso_impl.cuh:
-// pack_iso_hs_kernel), built in scratch; `hs` becomes the spec of that HS call.
 template <typename R>
-int stage_iso_as_hs(const cpf::Program* prog, const cpf_loss_spec* loss, Scratch& sc, cpf_loss_spec* hs) {
-  const int n = prog->n_qubits;
-  const IsoSpec is = iso_spec(prog, loss->ancilla_mask);
-  R* v = nullptr;
-  int rc = sc.get((void**)&v, ((size_t)2 << (2 * n)) * sizeof(R));
-  if (rc) return rc;
-  rc = cpf::launch_pack_iso<R>((const R*)loss->target, v, n, is.k, is.amask, true, sc.st);
-  if (rc) return fail(rc, "pack_iso launch failed");
-  *hs = cpf_loss_spec{};
-  hs->kind = CPF_LOSS_HS;
-  hs->target = v;
-  return CPF_OK;
-}
+struct CallPlan {
+  Route route;          // the state-adjoint kernels, the Heisenberg-picture kernel (HS on layered templates) or the
+                        // isometry kernel (n >= 6); each in a single- or a multi-target form
+  bool multi;           // sample b is scored against target target_index[b] of a table
+  bool layered;         // ROUTE_ADJOINT: try the kernel compiled for the layer before the interpreter
+  bool single;          // single-column kernels (state loss, isometry kernel)
+  bool iso_as_hs;       // n <= 5 isometry: the HS call on V = 2^a [W at the columns s_c, 0 elsewhere] (iso_impl.cuh:
+                        // pack_iso_hs_kernel), built in BLK_V
+  int32_t kind;         // the loss the kernel sees
+  IsoSpec iso;          // isometry kinds
+  int n_stage;          // ROUTE_HEIS: SWP::NSTAGE of the kernel chosen
+  int cpt, words;       // not ROUTE_ISO: columns per thread and words of one packed target
+  size_t heis_aux;      // ROUTE_HEIS: per-gate scratch at the start of BLK_HEIS (the packed state follows, 256-byte aligned)
+  cpf::PenaltyT<R> pen;
+  bool pen_mask;        // a cp_mask is uploaded: BLK_MASK is carved
+  size_t bytes[N_BLK];  // 0: no such block
+  // the caller-owned workspace: every block, each 256-byte aligned (BLK_MASK whether or not a cp_mask is given)
+  int64_t workspace() const {
+    size_t total = 0;
+    for (size_t b : bytes) total += Scratch::align(b);
+    return (int64_t)total;
+  }
+};
 
-// n >= 6: W packed column by column for the isometry kernel
+// Every refusal of a loss call is made here, before any CUDA call.  table != NULL: a multi-target call (`kind` is the
+// table's; its target_index, if given, is checked over `batch`).  pen may be NULL.
 template <typename R>
-int stage_iso(const cpf::Program* prog, const cpf_loss_spec* loss, cpf::KParams<R>& p, Scratch& sc) {
+int plan_call(const cpf::Program* prog, int32_t kind, int32_t mask, int64_t batch, const cpf_target_table* table,
+              const cpf_penalty_spec* pen, CallPlan<R>* pl) {
   const int n = prog->n_qubits;
-  const IsoSpec is = iso_spec(prog, loss->ancilla_mask);
-  R* packed = nullptr;
-  int rc = sc.get((void**)&packed, ((size_t)is.k << (n + 1)) * sizeof(R));
-  if (rc) return rc;
-  rc = cpf::launch_pack_iso<R>((const R*)loss->target, packed, n, is.k, is.amask, false, sc.st);
-  if (rc) return fail(rc, "pack_iso launch failed");
-  p.target_packed = packed;
-  p.target_bytes = 0;
-  p.loss_kind = CPF_LOSS_ISOMETRY;
-  p.iso_k = is.k;
-  p.iso_amask = is.amask;
-  return CPF_OK;
-}
-
-int check_loss(const cpf::Program* prog, const cpf_loss_spec* loss) {
-  if (!loss || !loss->target) return fail(CPF_ERR_INVALID, "loss spec / target is NULL");
-  if (loss->kind < CPF_LOSS_HS || loss->kind > CPF_LOSS_ISOMETRY)
-    return fail(CPF_ERR_INVALID, "unknown loss kind");
-  return loss->kind == CPF_LOSS_ISOMETRY ? check_iso(prog, loss->ancilla_mask) : check_full_unitary(prog, loss->kind);
-}
-
-// Everything a multi-target call needs to know is checked here, before any CUDA call.
-int check_table(const cpf::Program* prog, const cpf_target_table* tt, int64_t batch) {
-  if (!tt) return fail(CPF_ERR_INVALID, "target table is NULL");
-  if (tt->kind == CPF_LOSS_ISOMETRY)
+  *pl = CallPlan<R>();
+  if (kind < CPF_LOSS_HS || kind > CPF_LOSS_ISOMETRY) return fail(CPF_ERR_INVALID, "unknown loss kind");
+  if (table && kind == CPF_LOSS_ISOMETRY)
     return fail(CPF_ERR_UNSUPPORTED, "multi-target tables do not take the isometry loss (one target per call)");
-  if (tt->kind < CPF_LOSS_HS || tt->kind > CPF_LOSS_RELPHASE) return fail(CPF_ERR_INVALID, "unknown loss kind");
-  if (tt->n_targets < 1) return fail(CPF_ERR_INVALID, "target table: n_targets must be >= 1");
+  if (table && table->n_targets < 1) return fail(CPF_ERR_INVALID, "target table: n_targets must be >= 1");
+  // HS, relative phase and an isometry without ancillas run on the full-unitary kernels, which stop at 5 qubits
+  if (kind == CPF_LOSS_ISOMETRY) {
+    if (mask < 0 || (mask >> n) != 0)
+      return fail(CPF_ERR_INVALID, "ancilla_mask " + std::to_string(mask) + " names a qubit >= n = " + std::to_string(n));
+    if (n > 5 && mask == 0) return fail(CPF_ERR_UNSUPPORTED, cpf::FULL_UNITARY_LIMIT);
+    pl->iso = iso_spec(prog, mask);
+    if (n > 5 && pl->iso.k > ISO_MAX_K)
+      return fail(CPF_ERR_UNSUPPORTED, "isometry losses on 6-8 qubits take at most k = " + std::to_string(ISO_MAX_K) +
+                                       " input columns (k = 2^(n - popcount(ancilla_mask)) = " +
+                                       std::to_string(pl->iso.k) + ")");
+  } else if (kind != CPF_LOSS_STATE && n > 5) {
+    return fail(CPF_ERR_UNSUPPORTED, cpf::FULL_UNITARY_LIMIT);
+  }
+  for (int64_t b = 0; table && table->target_index && b < batch; ++b) {
+    const int32_t t = table->target_index[b];
+    if (t < 0 || t >= table->n_targets)
+      return fail(CPF_ERR_INVALID, "target_index[" + std::to_string(b) + "] = " + std::to_string(t) +
+                                       " is outside [0, n_targets = " + std::to_string(table->n_targets) + ")");
+  }
+  if (int rc = penalty_params<R>(prog, pen, &pl->pen)) return rc;
+
+  pl->multi = table != nullptr;
+  pl->iso_as_hs = kind == CPF_LOSS_ISOMETRY && n <= 5;
+  pl->kind = pl->iso_as_hs ? CPF_LOSS_HS : kind;
+  pl->single = pl->kind == CPF_LOSS_STATE || pl->kind == CPF_LOSS_ISOMETRY;
+  pl->layered = layered_kernels(prog);
+  // The Heisenberg-picture kernel keeps parameter and slot indices in 16 bits of shared memory (heis_impl.cuh: HSu2,
+  // HCp) and B * P below 2^32.  CPF_ENGINE=adjoint forces the state-adjoint kernels (tests cover both engines).
+  const char* eng = getenv("CPF_ENGINE");
+  bool heis = pl->kind == CPF_LOSS_HS && pl->layered && prog->n_params <= 32767 && prog->su2.size() <= 32767 &&
+              !(eng && std::strcmp(eng, "adjoint") == 0) &&
+              (unsigned long long)batch * (unsigned long long)prog->n_params < (1ull << 32);
+  if (heis) {
+    cpf::KParams<R> dummy;
+    std::string err;
+    int rc = 0;
+    heis = cpf::launch_heis<R>(dummy, *prog, nullptr, err, rc, true, &pl->n_stage);
+  }
+  pl->route = pl->kind == CPF_LOSS_ISOMETRY ? ROUTE_ISO : heis ? ROUTE_HEIS : ROUTE_ADJOINT;
+
+  pl->bytes[BLK_MASK] = prog->cp.empty() ? 1 : prog->cp.size();
+  pl->pen_mask = pl->pen.kind != CPF_PEN_NONE && pen->cp_mask && !prog->cp.empty();
+  if (pl->iso_as_hs) pl->bytes[BLK_V] = ((size_t)2 << (2 * n)) * sizeof(R);
+  if (pl->route == ROUTE_ISO) {
+    pl->bytes[BLK_TARGET] = ((size_t)pl->iso.k << (n + 1)) * sizeof(R);      // W packed column by column
+    return CPF_OK;
+  }
+  pl->cpt = heis ? cpf::heis_cpt<R>(n) : pl->single ? 1 : cpf::cpt_for<R>(n);
+  pl->words = heis ? cpf::heis_target_words<R>(n, pl->cpt) : cpf::target_words<R>(n, pl->cpt, pl->single);
+  if (table) {
+    // the kernels read index and targets (back to back) from global memory: no shared-memory copy, no padding
+    pl->bytes[BLK_INDEX] = (size_t)batch * sizeof(int32_t);
+    pl->bytes[BLK_TARGET] = (size_t)table->n_targets * (size_t)pl->words * sizeof(R);
+  } else {
+    pl->bytes[BLK_TARGET] = ((size_t)pl->words * sizeof(R) + 15) & ~(size_t)15;
+  }
+  if (heis) {
+    const size_t aux = (size_t)batch * (prog->su2.empty() ? 1 : prog->su2.size()) * 4 * sizeof(R);
+    pl->heis_aux = (aux + 255) & ~(size_t)255;      // the packed state starts on a 256-byte boundary (blocks of 16 positions)
+    // lane-interleaved packed optimiser state (heis_impl.cuh: heis_pk_stride words per sample)
+    const int tps = (1 << n) / pl->cpt;
+    pl->bytes[BLK_HEIS] = pl->heis_aux + (size_t)batch *
+                          (size_t)cpf::heis_pk_stride(n, tps, (int)prog->su2.size(), (int)prog->cp.size()) * sizeof(R);
+  }
+  return CPF_OK;
+}
+
+// the buffers every Adam entry point needs
+int check_adam_buffers(const cpf_adam_buffers* buf) {
+  if (!buf->angles || !buf->m || !buf->v || !buf->best_params || !buf->best_regloss || !buf->best_reg ||
+      !buf->init_regloss || !buf->init_reg)
+    return fail(CPF_ERR_INVALID, "a required cpf_adam_buffers pointer is NULL");
+  if ((buf->hist_params || buf->hist_regloss) && buf->hist_len <= 0)
+    return fail(CPF_ERR_INVALID, "history buffers given with hist_len <= 0");
+  return CPF_OK;
+}
+
+// the table's own pointers; everything else about it is checked by plan_call
+int check_table_pointers(const cpf_target_table* tt, int64_t batch) {
+  if (!tt) return fail(CPF_ERR_INVALID, "target table is NULL");
   if (!tt->targets) return fail(CPF_ERR_INVALID, "target table: targets is NULL");
   if (batch > 0 && !tt->target_index) return fail(CPF_ERR_INVALID, "target table: target_index is NULL");
-  if (int rc = check_full_unitary(prog, tt->kind)) return rc;
-  for (int64_t b = 0; b < batch; ++b) {
-    const int32_t t = tt->target_index[b];
-    if (t < 0 || t >= tt->n_targets)
-      return fail(CPF_ERR_INVALID, "target_index[" + std::to_string(b) + "] = " + std::to_string(t) +
-                                       " is outside [0, n_targets = " + std::to_string(tt->n_targets) + ")");
-  }
   return CPF_OK;
 }
 
-// bytes of the multi-target table of the kernel a call runs on (targets back to back in the kernel's packed layout)
-template <typename R>
-size_t multi_table_bytes(const cpf::Program* prog, int32_t kind, bool heis, int32_t n_targets) {
-  const bool single = kind == CPF_LOSS_STATE;
-  const int n = prog->n_qubits;
-  const int words = heis ? cpf::heis_target_words<R>(n, cpf::heis_cpt<R>(n))
-                         : cpf::target_words<R>(n, single ? 1 : cpf::cpt_for<R>(n), single);
-  return (size_t)n_targets * (size_t)words * sizeof(R);
-}
-
-// Multi-target staging: the index array (host, checked by check_table) goes to the device, all targets are packed in
-// one launch; the kernels read both from global memory (p.target_bytes = 0: no shared-memory copy).
-template <typename R>
-int stage_multi(const cpf::Program* prog, const cpf_target_table* tt, cpf::KParams<R>& p, bool heis, Scratch& sc) {
-  cudaStream_t st = sc.st;
-  if (heis && !sc.base) keep_pool_memory();
-  const bool single = tt->kind == CPF_LOSS_STATE;
-  const int n = prog->n_qubits;
-  int32_t* idx = nullptr;
-  R* table = nullptr;
-  int rc = sc.get((void**)&idx, (size_t)p.B * sizeof(int32_t));
-  if (!rc) rc = sc.get((void**)&table, multi_table_bytes<R>(prog, tt->kind, heis, tt->n_targets));
-  if (rc) return rc;
-  // pageable source: the runtime stages the bytes before returning
-  CPF_CUDA(cudaMemcpyAsync(idx, tt->target_index, (size_t)p.B * sizeof(int32_t), cudaMemcpyHostToDevice, st));
-  rc = heis ? cpf::launch_pack_targets_heis<R>((const R*)tt->targets, table, n, cpf::heis_cpt<R>(n), tt->n_targets, st)
-            : cpf::launch_pack_targets<R>((const R*)tt->targets, table, n, single ? 1 : cpf::cpt_for<R>(n), single,
-                                          tt->n_targets, st);
-  if (rc) return fail(rc, "pack_targets launch failed");
-  p.target_packed = table;
-  p.target_bytes = 0;
-  p.target_index = idx;
-  p.loss_kind = tt->kind;
-  return heis ? stage_heis_state(prog, p, sc) : CPF_OK;
-}
-
-// Launch of a staged call: the single-target kernels, or (table != NULL) their multi-target variants.
-template <typename R>
-int launch_staged(const cpf::KParams<R>& p, const cpf::Program* prog, const cpf_target_table* table, bool heis,
-                  bool single, cudaStream_t st, std::string& err) {
-  int rc = CPF_OK;
-  if (table) {
-    if (heis) cpf::launch_heis_multi<R>(p, *prog, st, err, rc);
-    else rc = cpf::launch_engine_multi<R>(p, prog->n_qubits, single, st, err);
-  } else {
-    if (heis) cpf::launch_heis<R>(p, *prog, st, err, rc, false);
-    else rc = launch_any<R>(p, prog, single, st, err);
+// A planned loss call: check the caller's workspace, carve every scratch block, then upload the program, stage the
+// penalty mask and the target and launch.  Nothing touches the device before the blocks are carved.  `target` is the
+// loss spec's or the table's; `set_mode` fills the mode fields of KParams; grad_out, if given, is zeroed first.
+template <typename R, typename SetMode>
+int run_staged(const cpf::Program* prog, const CallPlan<R>& pl, const void* target, const cpf_target_table* table,
+               const cpf_penalty_spec* pen, int64_t batch, void* workspace, int64_t workspace_bytes, void* grad_out,
+               cudaStream_t st, SetMode set_mode) {
+  Scratch sc;
+  sc.st = st;
+  if (workspace) {
+    if (((uintptr_t)workspace & 255) != 0) return fail(CPF_ERR_INVALID, "workspace must be 256-byte aligned");
+    if (workspace_bytes < pl.workspace())
+      return fail(CPF_ERR_INVALID, "workspace too small: cpf_workspace_bytes gives the size this call needs");
+    sc.base = (char*)workspace;
+    sc.size = (size_t)workspace_bytes;
+  } else if (pl.route == ROUTE_HEIS) {
+    keep_pool_memory();
   }
-  return rc;
+  void* blk[N_BLK] = {};
+  for (int b = 0; b < N_BLK; ++b)
+    if (pl.bytes[b] && (b != BLK_MASK || pl.pen_mask))
+      if (int rc = sc.get(&blk[b], pl.bytes[b])) return rc;
+
+  const int n = prog->n_qubits;
+  cpf::KParams<R> p;
+  int rc = fill_common(prog, p, batch, pl.single);
+  if (rc) return rc;
+  set_mode(p);
+  p.pen = pl.pen;
+  if (blk[BLK_MASK]) {
+    if ((rc = upload_cp_mask(prog, pen->cp_mask, blk[BLK_MASK], st))) return rc;
+    p.cp_pen = (const uint8_t*)blk[BLK_MASK];
+  }
+  if (pl.iso_as_hs) {
+    rc = cpf::launch_pack_iso<R>((const R*)target, (R*)blk[BLK_V], n, pl.iso.k, pl.iso.amask, true, st);
+    if (rc) return fail(rc, "pack_iso launch failed");
+    target = blk[BLK_V];
+  }
+  R* packed = (R*)blk[BLK_TARGET];
+  p.target_packed = packed;
+  p.loss_kind = pl.kind;
+  if (pl.multi) {
+    // pageable source: the runtime stages the bytes before returning
+    CPF_CUDA(cudaMemcpyAsync(blk[BLK_INDEX], table->target_index, (size_t)batch * sizeof(int32_t),
+                             cudaMemcpyHostToDevice, st));
+    rc = pl.route == ROUTE_HEIS
+             ? cpf::launch_pack_targets_heis<R>((const R*)target, packed, n, pl.cpt, table->n_targets, st)
+             : cpf::launch_pack_targets<R>((const R*)target, packed, n, pl.cpt, pl.single, table->n_targets, st);
+    if (rc) return fail(rc, "pack_targets launch failed");
+    p.target_index = (const int32_t*)blk[BLK_INDEX];
+  } else if (pl.route == ROUTE_ISO) {
+    rc = cpf::launch_pack_iso<R>((const R*)target, packed, n, pl.iso.k, pl.iso.amask, false, st);
+    if (rc) return fail(rc, "pack_iso launch failed");
+    p.iso_k = pl.iso.k;
+    p.iso_amask = pl.iso.amask;
+  } else {
+    const size_t bytes = pl.bytes[BLK_TARGET];
+    if (bytes != (size_t)pl.words * sizeof(R)) CPF_CUDA(cudaMemsetAsync(packed, 0, bytes, st));
+    rc = pl.route == ROUTE_HEIS ? cpf::launch_pack_target_heis<R>((const R*)target, packed, n, pl.cpt, st)
+                                : cpf::launch_pack_target<R>((const R*)target, packed, n, pl.cpt, pl.single, st);
+    if (rc) return fail(rc, "pack_target launch failed");
+    p.target_bytes = (int)bytes;
+  }
+  if (pl.route == ROUTE_HEIS) stage_heis_state(prog, p, blk[BLK_HEIS], pl.heis_aux);
+  if (grad_out) CPF_CUDA(cudaMemsetAsync(grad_out, 0, (size_t)batch * prog->n_params * sizeof(R), st));
+
+  std::string err;
+  if (pl.route == ROUTE_ISO) {
+    rc = cpf::launch_iso<R>(p, n, st, err);
+  } else if (pl.route == ROUTE_HEIS) {
+    if (!(pl.multi ? cpf::launch_heis_multi<R>(p, *prog, st, err, rc) : cpf::launch_heis<R>(p, *prog, st, err, rc, false))) {
+      rc = CPF_ERR_UNSUPPORTED;
+      err = "no Heisenberg-picture kernel for this program";
+    }
+  } else {
+    rc = pl.multi ? cpf::launch_engine_multi<R>(p, n, pl.single, st, err) : launch_any<R>(p, prog, pl.single, pl.layered, st, err);
+  }
+  return rc ? fail(rc, err) : CPF_OK;
 }
 
 template <typename R>
@@ -483,45 +474,24 @@ int run_unitary(const cpf::Program* prog, int64_t batch, const void* angles, voi
   p.colmode = colmode ? 1 : 0;
   p.angles = (R*)angles; p.u_out = (R*)u_out;
   std::string err;
-  rc = launch_any<R>(p, prog, colmode, st, err);
+  rc = launch_any<R>(p, prog, colmode, layered_kernels(prog), st, err);
   return rc ? fail(rc, err) : CPF_OK;
 }
 
-// table != NULL: multi-target call (loss->kind = table->kind, loss->target unused)
+// table != NULL: multi-target call (kind = table->kind, target = table->targets)
 template <typename R>
-int run_loss_grad(const cpf::Program* prog, const cpf_loss_spec* loss, const cpf_penalty_spec* pen,
+int run_loss_grad(const cpf::Program* prog, int32_t kind, int32_t mask, const void* target, const cpf_penalty_spec* pen,
                   int64_t batch, const void* angles, void* loss_out, void* reg_out, void* grad_out,
                   cudaStream_t st, const cpf_target_table* table = nullptr) {
-  cpf::KParams<R> p;
-  Scratch sc;
-  sc.st = st;
-  cpf_loss_spec hs;
-  const bool iso = loss->kind == CPF_LOSS_ISOMETRY && prog->n_qubits > 5;    // else n <= 5: an HS call on V
-  if (loss->kind == CPF_LOSS_ISOMETRY && !iso) {
-    int rc = stage_iso_as_hs<R>(prog, loss, sc, &hs);
-    if (rc) return rc;
-    loss = &hs;
-  }
-  const bool single = loss->kind == CPF_LOSS_STATE || iso;
-  int rc = fill_common(prog, p, batch, single);
-  if (rc) return rc;
-  p.mode = cpf::M_LOSSGRAD;
-  p.angles = (R*)angles; p.loss_out = (R*)loss_out; p.reg_out = (R*)reg_out; p.grad_out = (R*)grad_out;
-  const bool heis = use_heis<R>(prog, loss) && (unsigned long long)batch * (unsigned long long)prog->n_params < (1ull << 32);
-  rc = fill_penalty(prog, pen, p, sc);
-  if (!rc && table) rc = stage_multi(prog, table, p, heis, sc);
-  else if (!rc && iso) rc = stage_iso(prog, loss, p, sc);
-  else if (!rc) rc = heis ? stage_heis(prog, loss, p, sc) : stage_target(prog, loss, p, single, sc);
-  if (!rc && grad_out) {
-    cudaError_t e = cudaMemsetAsync(grad_out, 0, (size_t)batch * prog->n_params * sizeof(R), st);
-    if (e != cudaSuccess) rc = cuda_fail("cudaMemsetAsync(grad)", e);
-  }
-  std::string err;
-  if (!rc) {
-    rc = iso ? cpf::launch_iso<R>(p, prog->n_qubits, st, err) : launch_staged<R>(p, prog, table, heis, single, st, err);
-    if (rc) fail(rc, err);
-  }
-  return rc;
+  CallPlan<R> pl;
+  if (int rc = plan_call<R>(prog, kind, mask, batch, table, pen, &pl)) return rc;
+  if (batch == 0) return CPF_OK;
+  if (!loss_out) return fail(CPF_ERR_INVALID, "loss_out is NULL");
+  if (!angles && prog->n_params > 0) return fail(CPF_ERR_INVALID, "angles is NULL");
+  return run_staged<R>(prog, pl, target, table, pen, batch, nullptr, 0, grad_out, st, [&](cpf::KParams<R>& p) {
+    p.mode = cpf::M_LOSSGRAD;
+    p.angles = (R*)angles; p.loss_out = (R*)loss_out; p.reg_out = (R*)reg_out; p.grad_out = (R*)grad_out;
+  });
 }
 
 // 6-8 qubits: the cotangent mode of the isometry kernel (iso_impl.cuh: InterpSweepIsoCot), one launch item per
@@ -570,92 +540,38 @@ int run_cotangent(const cpf::Program* prog, int64_t batch, const void* angles, c
   p.angles = (R*)angles; p.cot = (const R*)cot; p.grad_out = (R*)grad_out;
   CPF_CUDA(cudaMemsetAsync(grad_out, 0, (size_t)batch * prog->n_params * sizeof(R), st));
   std::string err;
-  rc = launch_any<R>(p, prog, false, st, err);
+  rc = launch_any<R>(p, prog, false, layered_kernels(prog), st, err);
   return rc ? fail(rc, err) : CPF_OK;
 }
 
 template <typename R>
-int run_adam(const cpf::Program* prog, const cpf_loss_spec* loss, const cpf_penalty_spec* pen,
+int run_adam(const cpf::Program* prog, int32_t kind, int32_t mask, const void* target, const cpf_penalty_spec* pen,
              const cpf_adam_spec* adam, int64_t batch, int64_t step0, int64_t num_steps,
              const cpf_adam_buffers* buf, cudaStream_t st, const cpf_target_table* table = nullptr) {
-  cpf::KParams<R> p;
-  const bool iso = loss->kind == CPF_LOSS_ISOMETRY && prog->n_qubits > 5;    // else n <= 5: an HS call on V
-  const bool single = loss->kind == CPF_LOSS_STATE || iso;
-  int rc = fill_common(prog, p, batch, single);
-  if (rc) return rc;
-  p.mode = cpf::M_ADAM;
-  p.lr = (R)adam->lr; p.b1 = (R)adam->b1; p.b2 = (R)adam->b2; p.eps = (R)adam->eps;
-  p.omb1 = (R)(1.0 - adam->b1); p.omb2 = (R)(1.0 - adam->b2);
-  p.step0 = step0; p.nsteps = (int)num_steps;
-  p.angles = (R*)buf->angles; p.m = (R*)buf->m; p.v = (R*)buf->v; p.freeze = buf->freeze;
-  p.best_params = (R*)buf->best_params; p.best_regloss = (R*)buf->best_regloss;
-  p.best_reg = (R*)buf->best_reg; p.init_regloss = (R*)buf->init_regloss; p.init_reg = (R*)buf->init_reg;
-  p.hist_params = (R*)buf->hist_params; p.hist_regloss = (R*)buf->hist_regloss; p.hist_len = buf->hist_len;
-  Scratch sc;
-  sc.st = st;
-  if (buf->workspace) {
-    if (((uintptr_t)buf->workspace & 255) != 0) return fail(CPF_ERR_INVALID, "workspace must be 256-byte aligned");
-    sc.base = (char*)buf->workspace;
-    sc.size = buf->workspace_bytes > 0 ? (size_t)buf->workspace_bytes : 0;
-  }
-  cpf_loss_spec hs;
-  if (loss->kind == CPF_LOSS_ISOMETRY && !iso) {
-    rc = stage_iso_as_hs<R>(prog, loss, sc, &hs);
-    if (rc) return rc;
-    loss = &hs;
-  }
-  const bool heis = use_heis<R>(prog, loss) && (unsigned long long)batch * (unsigned long long)prog->n_params < (1ull << 32);
-  rc = fill_penalty(prog, pen, p, sc);
-  if (!rc && table) rc = stage_multi(prog, table, p, heis, sc);
-  else if (!rc && iso) rc = stage_iso(prog, loss, p, sc);
-  else if (!rc) rc = heis ? stage_heis(prog, loss, p, sc) : stage_target(prog, loss, p, single, sc);
-  std::string err;
-  if (!rc) {
-    rc = iso ? cpf::launch_iso<R>(p, prog->n_qubits, st, err) : launch_staged<R>(p, prog, table, heis, single, st, err);
-    if (rc) fail(rc, err);
-  }
-  return rc;
+  CallPlan<R> pl;
+  if (int rc = plan_call<R>(prog, kind, mask, batch, table, pen, &pl)) return rc;
+  if (batch == 0 || num_steps == 0) return CPF_OK;
+  if (int rc = check_adam_buffers(buf)) return rc;
+  if (num_steps > 2000000000LL) return fail(CPF_ERR_INVALID, "num_steps too large");
+  return run_staged<R>(prog, pl, target, table, pen, batch, buf->workspace, buf->workspace_bytes, nullptr, st,
+                       [&](cpf::KParams<R>& p) {
+    p.mode = cpf::M_ADAM;
+    p.lr = (R)adam->lr; p.b1 = (R)adam->b1; p.b2 = (R)adam->b2; p.eps = (R)adam->eps;
+    p.omb1 = (R)(1.0 - adam->b1); p.omb2 = (R)(1.0 - adam->b2);
+    p.step0 = step0; p.nsteps = (int)num_steps;
+    p.angles = (R*)buf->angles; p.m = (R*)buf->m; p.v = (R*)buf->v; p.freeze = buf->freeze;
+    p.best_params = (R*)buf->best_params; p.best_regloss = (R*)buf->best_regloss;
+    p.best_reg = (R*)buf->best_reg; p.init_regloss = (R*)buf->init_regloss; p.init_reg = (R*)buf->init_reg;
+    p.hist_params = (R*)buf->hist_params; p.hist_regloss = (R*)buf->hist_regloss; p.hist_len = buf->hist_len;
+  });
 }
 
-// bytes of scratch one cpf_adam_run / cpf_loss_grad needs (the blocks Scratch::get hands out, each 256-byte aligned)
+// The plan behind a query entry point's loss-kind argument: an isometry kind carries its ancilla mask in bits 8-15
+// (CPF_ISOMETRY_KIND); any other use of bits 8-31 makes an unknown kind.
 template <typename R>
-int64_t workspace_bytes_t(const cpf::Program* prog, int32_t loss_kind, int32_t mask, int64_t batch) {
-  size_t total = Scratch::align(prog->cp.empty() ? 1 : prog->cp.size());          // penalty mask
-  if (loss_kind == CPF_LOSS_ISOMETRY) {
-    const int n = prog->n_qubits;
-    if (n > 5) return (int64_t)(total + Scratch::align(((size_t)iso_spec(prog, mask).k << (n + 1)) * sizeof(R)));
-    total += Scratch::align(((size_t)2 << (2 * n)) * sizeof(R));                   // V of the HS call
-    loss_kind = CPF_LOSS_HS;
-  }
-  cpf_loss_spec ls{};
-  ls.kind = loss_kind;
-  const bool single = loss_kind == CPF_LOSS_STATE;
-  const bool heis = use_heis<R>(prog, &ls) && (unsigned long long)batch * (unsigned long long)prog->n_params < (1ull << 32);
-  if (heis) {
-    size_t tb, ap, pk;
-    heis_scratch_sizes<R>(prog, batch, &tb, &ap, &pk);
-    total += Scratch::align(tb) + Scratch::align(ap + pk);
-  } else {
-    const int cpt = single ? 1 : cpf::cpt_for<R>(prog->n_qubits);
-    total += Scratch::align((((size_t)cpf::target_words<R>(prog->n_qubits, cpt, single) * sizeof(R)) + 15) & ~(size_t)15);
-  }
-  return (int64_t)total;
-}
-
-template <typename R>
-int64_t workspace_bytes_multi_t(const cpf::Program* prog, int32_t loss_kind, int64_t batch, int32_t n_targets) {
-  cpf_loss_spec ls{};
-  ls.kind = loss_kind;
-  const bool heis = use_heis<R>(prog, &ls) && (unsigned long long)batch * (unsigned long long)prog->n_params < (1ull << 32);
-  size_t total = Scratch::align(prog->cp.empty() ? 1 : prog->cp.size());          // penalty mask
-  total += Scratch::align((size_t)batch * sizeof(int32_t));                         // target_index
-  total += Scratch::align(multi_table_bytes<R>(prog, loss_kind, heis, n_targets));  // target table
-  if (heis) {
-    size_t tb, ap, pk;
-    heis_scratch_sizes<R>(prog, batch, &tb, &ap, &pk);
-    total += Scratch::align(ap + pk);
-  }
-  return (int64_t)total;
+int plan_query(const cpf::Program* prog, int32_t arg, int64_t batch, CallPlan<R>* pl) {
+  const int32_t kind = (arg & ~0xff00) == CPF_LOSS_ISOMETRY || (arg >> 8) == 0 ? arg & 0xff : -1;
+  return plan_call<R>(prog, kind, (arg >> 8) & 0xff, batch, nullptr, nullptr, pl);
 }
 
 // ---- count_cz / projection (cp_utils.py:45-77, 111-141) ----
@@ -870,18 +786,12 @@ __global__ void initial_angles_kernel(const cpf::CpMeta* cp, int n_cp, int P, ui
 template <typename R>
 static int run_adam_step(const cpf::Program* prog, const cpf_penalty_spec* pen, const cpf_adam_spec* adam, int64_t batch,
                          int64_t step, const void* loss, const void* grad, const cpf_adam_buffers* buf, cudaStream_t st) {
-  cpf::KParams<R> p;
-  std::memset(&p, 0, sizeof(p));
-  // fill_penalty validates the spec and converts the table; the per-parameter mask is rebuilt here ([P], not [n_cp])
-  int rc;
-  {
-    Scratch sc;
-    sc.st = st;
-    rc = fill_penalty(prog, pen, p, sc);
-  }
+  // the penalty mask is per parameter here ([P], not [n_cp])
+  cpf::PenaltyT<R> pt;
+  int rc = penalty_params<R>(prog, pen, &pt);
   if (rc) return rc;
   uint8_t* mask_dev = nullptr;
-  if (p.pen.kind != CPF_PEN_NONE && prog->n_params > 0) {
+  if (pt.kind != CPF_PEN_NONE && prog->n_params > 0) {
     std::string mask((size_t)prog->n_params, '\0');
     for (int i = 0; i < prog->n_params; ++i)
       mask[i] = prog->is_cp_param[i] && (!pen->cp_mask || pen->cp_mask[i]) ? 1 : 0;
@@ -891,7 +801,7 @@ static int run_adam_step(const cpf::Program* prog, const cpf_penalty_spec* pen, 
   dim3 block(32, 8);
   const unsigned grid = (unsigned)((batch + 7) / 8);
   adam_step_kernel<R><<<grid, block, 0, st>>>(
-      p.pen, mask_dev, prog->n_params, batch, step, (R)adam->lr, (R)adam->b1, (R)adam->b2, (R)adam->eps,
+      pt, mask_dev, prog->n_params, batch, step, (R)adam->lr, (R)adam->b1, (R)adam->b2, (R)adam->eps,
       (R)(1.0 - adam->b1), (R)(1.0 - adam->b2), (const R*)loss, (const R*)grad, (R*)buf->angles, (R*)buf->m, (R*)buf->v,
       buf->freeze, (R*)buf->best_params, (R*)buf->best_regloss, (R*)buf->best_reg, (R*)buf->init_regloss,
       (R*)buf->init_reg, (R*)buf->hist_params, (R*)buf->hist_regloss, buf->hist_len);
@@ -902,59 +812,92 @@ static int run_adam_step(const cpf::Program* prog, const cpf_penalty_spec* pen, 
 }
 
 template <typename R>
-static int launch_plan_t(const cpf::Program* prog, const cpf_loss_spec_kind_only& lk, int64_t batch, int n_sm, int regs,
+static int workspace_t(const cpf::Program* prog, int32_t loss_kind, int64_t batch, const cpf_target_table* table,
+                       int64_t* bytes) {
+  CallPlan<R> pl;
+  const int rc = table ? plan_call<R>(prog, loss_kind, 0, batch, table, nullptr, &pl)
+                       : plan_query<R>(prog, loss_kind, batch, &pl);
+  if (!rc) *bytes = pl.workspace();
+  return rc;
+}
+
+template <typename R>
+static int launch_plan_t(const cpf::Program* prog, int32_t loss_kind, int64_t batch, int n_sm, int regs,
                          cpf_launch_info* out, int adam_steps = 2000) {
-  cpf_loss_spec ls{};
-  ls.kind = lk.kind;
-  const bool heis = use_heis<R>(prog, &ls) && (unsigned long long)batch * (unsigned long long)prog->n_params < (1ull << 32);
-  out->engine = heis ? 1 : 0;
-  if (!heis) return CPF_OK;
-  const int n = prog->n_qubits, N = 1 << n, cpt = cpf::heis_cpt<R>(n), tps = N / cpt;
-  const int maxt = 2 * N * cpt * (int)(sizeof(R) / 4) <= 64 ? 512 : 256;          // HCfg::MAXT
-  const int n_su2 = (int)prog->su2.size(), n_cp = (int)prog->cp.size();
-  int n_stage = n;                                                                // SWP::NSTAGE of the kernel chosen
-  {
-    cpf::KParams<R> dummy;
-    std::string e2;
-    int rc2 = 0;
-    cpf::launch_heis<R>(dummy, *prog, nullptr, e2, rc2, true, &n_stage);
+  CallPlan<R> pl;
+  if (int rc = plan_query<R>(prog, loss_kind, batch, &pl)) return rc;
+  const int n = prog->n_qubits, N = 1 << n, n_su2 = (int)prog->su2.size(), n_cp = (int)prog->cp.size();
+  if (pl.route == ROUTE_ISO) {
+    // the isometry kernel's geometry (iso_impl.cuh: iso_geometry); co-residency is not planned (ctas_per_sm = 0)
+    const int k = pl.iso.k, rb = cpf::engine_rb<R>(n, true);
+    const cpf::DecodedSchedule ds = cpf::decode_schedule(*prog, rb);
+    const int n_red = ds.red.empty() ? 1 : (int)(ds.red.size() / 8);
+    const cpf::IsoGeometry g = cpf::iso_geometry(n, rb, k, n_su2, n_cp, (int)prog->sched.size(), n_red, sizeof(R));
+    out->block_threads = g.block;
+    out->samples_per_cta = g.spb;
+    out->threads_per_sample = g.spt;
+    out->max_block_threads = n == 6 ? 512 : 1024;          // __launch_bounds__ of iso_kernel
+    out->words_per_sample = cpf::iso_sample_words(cpf::coef_stride_words(n_su2, n_cp), k, cpf::iso_sum_stride(n_su2, n_cp));
+    out->time_slices = 1;
+    out->grid = (batch + g.spb - 1) / g.spb;
+    out->smem_bytes = (int64_t)g.smem;
+    out->launches_per_run = 1;
+    return CPF_OK;
   }
-  const int stride = cpf::heis_coef_stride(n_su2, n_cp, n_stage);
-  const size_t target = (((size_t)cpf::heis_target_words<R>(n, cpt) * sizeof(R)) + 15) & ~(size_t)15;
-  const cpf::HeisGeometry g = cpf::heis_geometry(batch, target + cpf::heis_meta_bytes(n_su2, n_cp),
-                                                 (size_t)stride * sizeof(R), tps, maxt, regs > 0 ? regs : 128,
-                                                 n_sm > 0 ? n_sm : 148);
+  out->engine = pl.route == ROUTE_HEIS ? 1 : 0;
+  if (pl.route != ROUTE_HEIS) return CPF_OK;
+  const int tps = N / pl.cpt;
+  const int maxt = 2 * N * pl.cpt * (int)(sizeof(R) / 4) <= 64 ? 512 : 256;       // HCfg::MAXT
+  const int stride = cpf::heis_coef_stride(n_su2, n_cp, pl.n_stage);
+  const size_t fixed = pl.bytes[BLK_TARGET] + cpf::heis_meta_bytes(n_su2, n_cp);
+  const cpf::HeisGeometry g = cpf::heis_geometry(batch, fixed, (size_t)stride * sizeof(R), tps, maxt,
+                                                 regs > 0 ? regs : 128, n_sm > 0 ? n_sm : 148);
   out->ctas_per_sm = g.ctas; out->block_threads = g.block; out->samples_per_cta = g.spb; out->grid = g.grid;
   out->smem_bytes = (int64_t)g.smem; out->threads_per_sample = tps; out->max_block_threads = maxt;
   out->words_per_sample = stride;
   // time slices an Adam run of `adam_steps` iterations over this batch would be cut into (1 = one launch)
-  const cpf::HeisSlicing sl = cpf::heis_slicing(batch, adam_steps > 0 ? adam_steps : 2000,
-                                                target + cpf::heis_meta_bytes(n_su2, n_cp), (size_t)stride * sizeof(R), tps,
-                                                maxt, regs > 0 ? regs : 128, n_sm > 0 ? n_sm : 148, true);
+  const cpf::HeisSlicing sl = cpf::heis_slicing(batch, adam_steps > 0 ? adam_steps : 2000, fixed,
+                                                (size_t)stride * sizeof(R), tps, maxt, regs > 0 ? regs : 128,
+                                                n_sm > 0 ? n_sm : 148, true);
   out->time_slices = sl.k;
   out->launches_per_run = sl.k > 1 ? (batch * sl.k + sl.slots - 1) / sl.slots : 1;
   return CPF_OK;
 }
 
-// the isometry kernel's geometry (iso_impl.cuh: iso_geometry); co-residency is not planned (ctas_per_sm = 0)
 template <typename R>
-static int iso_plan_t(const cpf::Program* prog, int32_t mask, int64_t batch, cpf_launch_info* out) {
-  const int n = prog->n_qubits, n_su2 = (int)prog->su2.size(), n_cp = (int)prog->cp.size();
-  const int k = iso_spec(prog, mask).k;
-  const int rb = cpf::engine_rb<R>(n, true);
-  const cpf::DecodedSchedule ds = cpf::decode_schedule(*prog, rb);
-  const int n_red = ds.red.empty() ? 1 : (int)(ds.red.size() / 8);
-  const cpf::IsoGeometry g = cpf::iso_geometry(n, rb, k, n_su2, n_cp, (int)prog->sched.size(), n_red, sizeof(R));
-  out->engine = 0;
-  out->block_threads = g.block;
-  out->samples_per_cta = g.spb;
-  out->threads_per_sample = g.spt;
-  out->max_block_threads = n == 6 ? 512 : 1024;          // __launch_bounds__ of iso_kernel
-  out->words_per_sample = cpf::iso_sample_words(cpf::coef_stride_words(n_su2, n_cp), k, cpf::iso_sum_stride(n_su2, n_cp));
-  out->time_slices = 1;
-  out->grid = (batch + g.spb - 1) / g.spb;
-  out->smem_bytes = (int64_t)g.smem;
-  out->launches_per_run = 1;
+static int eval_cost_t(const cpf::Program* p, int32_t loss_kind, double* flops, double* bytes) {
+  CallPlan<R> pl;
+  if (int rc = plan_query<R>(p, loss_kind, 1, &pl)) return rc;
+  const double N = (double)(1 << p->n_qubits);
+  const double C = pl.kind == CPF_LOSS_STATE ? 1.0 : pl.iso.k ? (double)pl.iso.k : N;     // isometry: C = k
+  const double rs = (double)sizeof(R);
+  if (flops) *flops = C * N * (16.0 * p->n_rot + 4.0 * p->n_phase + 8.0);
+  if (bytes) *bytes = 6.0 * p->n_params * rs + 2.0 * rs;
+  return CPF_OK;
+}
+
+template <typename R>
+static int executed_cost_t(const cpf::Program* p, int32_t loss_kind, double* flops) {
+  CallPlan<R> pl;
+  if (int rc = plan_query<R>(p, loss_kind, 1, &pl)) return rc;
+  const double N = (double)(1 << p->n_qubits), n = p->n_qubits, K = (double)p->cp.size(), G = (double)p->su2.size();
+  if (pl.route == ROUTE_HEIS) {
+    // heis_kernel (heis_impl.cuh), FMA = 2 flop, per sample and step:
+    //   forward   block: 3 diagonal phases on N/4 rows (6 flop per complex amplitude) + 2 Ry in lifting form (3 shears on
+    //             re and im): N^2 (4.5 + 12); surface gate: phase on N/2 rows + Ry: 9 N^2; pending phases at the end: 3 N^2
+    //   backward  fused gate: Rx exchange + merged Rz on the N^2 real coefficients: 4.5 N^2; ZZ pair rotations
+    //             (lifting): 3 N^2 per block; outgoing Rz of the last gate per qubit: 3 N^2
+    //   pivot     Walsh-Hadamard transform (re, im) + seed of h: N^2 (2 n + 6)
+    //   update    per fused gate: chain rule, 3 x Adam, 3 x sin/cos, SU(2) products, ZYZ data, staging: ~232;
+    //             per entangler: Adam, sin/cos, penalty, merged diagonal: ~80
+    *flops = N * N * (28.5 * K + 19.5 * n + 2.0 * n + 6.0) + 232.0 * G + 80.0 * K;
+  } else {
+    // state-adjoint kernels: the credited count plus the uncompute of phi (6 flop per amplitude and rotation on
+    // fused gates, 1.5 per phase gate), with fused gates instead of primitive rotations: C N (22 G + 5.5 K + 8);
+    // an isometry runs as an HS call on n <= 5 and on the isometry kernel with C = k on n >= 6
+    const double C = pl.kind == CPF_LOSS_STATE ? 1.0 : pl.route == ROUTE_ISO ? (double)pl.iso.k : N;
+    *flops = C * N * (22.0 * G + 5.5 * K + 8.0) + 232.0 * G + 80.0 * K;
+  }
   return CPF_OK;
 }
 
@@ -1034,14 +977,10 @@ int cpf_loss_grad(const cpf_program* prog, const cpf_loss_spec* loss, const cpf_
                   int32_t dtype, int64_t batch, const void* angles, void* loss_out, void* reg_out,
                   void* grad_out, void* stream) {
   if (!prog || batch < 0) return fail(CPF_ERR_INVALID, "NULL program / bad batch");
+  if (!loss || !loss->target) return fail(CPF_ERR_INVALID, "loss spec / target is NULL");
   const cpf::Program* p = reinterpret_cast<const cpf::Program*>(prog);
-  int rc = check_loss(p, loss);
-  if (rc) return rc;
-  if (batch == 0) return CPF_OK;
-  if (!loss_out) return fail(CPF_ERR_INVALID, "loss_out is NULL");
-  if (!angles && p->n_params > 0) return fail(CPF_ERR_INVALID, "angles is NULL");
-  CPF_DISPATCH(dtype, (run_loss_grad<R>(p, loss, penalty, batch, angles, loss_out, reg_out, grad_out,
-                                        (cudaStream_t)stream)));
+  CPF_DISPATCH(dtype, (run_loss_grad<R>(p, loss->kind, loss->ancilla_mask, loss->target, penalty, batch, angles,
+                                        loss_out, reg_out, grad_out, (cudaStream_t)stream)));
 }
 
 int cpf_adjoint_from_cotangent(const cpf_program* prog, int32_t dtype, int64_t batch, const void* angles,
@@ -1058,45 +997,26 @@ int cpf_adam_run(const cpf_program* prog, const cpf_loss_spec* loss, const cpf_p
                  const cpf_adam_buffers* buf, void* stream) {
   if (!prog || !adam || !buf || batch < 0 || step0 < 0 || num_steps < 0)
     return fail(CPF_ERR_INVALID, "NULL argument / negative size");
-  int rc = check_loss(reinterpret_cast<const cpf::Program*>(prog), loss);
-  if (rc) return rc;
-  if (batch == 0 || num_steps == 0) return CPF_OK;
-  if (!buf->angles || !buf->m || !buf->v || !buf->best_params || !buf->best_regloss || !buf->best_reg ||
-      !buf->init_regloss || !buf->init_reg)
-    return fail(CPF_ERR_INVALID, "a required cpf_adam_buffers pointer is NULL");
-  if ((buf->hist_params || buf->hist_regloss) && buf->hist_len <= 0)
-    return fail(CPF_ERR_INVALID, "history buffers given with hist_len <= 0");
-  if (num_steps > 2000000000LL) return fail(CPF_ERR_INVALID, "num_steps too large");
-  if (batch == 0 || num_steps == 0) return CPF_OK;
+  if (!loss || !loss->target) return fail(CPF_ERR_INVALID, "loss spec / target is NULL");
   const cpf::Program* p = reinterpret_cast<const cpf::Program*>(prog);
-  CPF_DISPATCH(dtype, (run_adam<R>(p, loss, penalty, adam, batch, step0, num_steps, buf,
-                                   (cudaStream_t)stream)));
+  CPF_DISPATCH(dtype, (run_adam<R>(p, loss->kind, loss->ancilla_mask, loss->target, penalty, adam, batch, step0,
+                                   num_steps, buf, (cudaStream_t)stream)));
 }
 
 int cpf_workspace_bytes(const cpf_program* prog, int32_t loss_kind, int32_t dtype, int64_t batch, int64_t* bytes) {
   if (!prog || !bytes || batch < 0) return fail(CPF_ERR_INVALID, "NULL argument / negative batch");
   const cpf::Program* p = reinterpret_cast<const cpf::Program*>(prog);
-  int32_t kind, mask;
-  int rc = split_kind(p, loss_kind, &kind, &mask);
-  if (!rc) rc = check_full_unitary(p, kind);
-  if (rc) return rc;
-  *bytes = dtype == CPF_F64 ? workspace_bytes_t<double>(p, kind, mask, batch) : workspace_bytes_t<float>(p, kind, mask, batch);
-  return CPF_OK;
+  CPF_DISPATCH(dtype, (workspace_t<R>(p, loss_kind, batch, nullptr, bytes)));
 }
 
 int cpf_loss_grad_multi(const cpf_program* prog, const cpf_target_table* table, const cpf_penalty_spec* penalty,
                         int32_t dtype, int64_t batch, const void* angles, void* loss_out, void* reg_out,
                         void* grad_out, void* stream) {
   if (!prog || batch < 0) return fail(CPF_ERR_INVALID, "NULL program / bad batch");
+  if (int rc = check_table_pointers(table, batch)) return rc;
   const cpf::Program* p = reinterpret_cast<const cpf::Program*>(prog);
-  int rc = check_table(p, table, batch);
-  if (rc) return rc;
-  if (batch == 0) return CPF_OK;
-  if (!loss_out) return fail(CPF_ERR_INVALID, "loss_out is NULL");
-  if (!angles && p->n_params > 0) return fail(CPF_ERR_INVALID, "angles is NULL");
-  const cpf_loss_spec loss{table->kind, table->targets, 0};
-  CPF_DISPATCH(dtype, (run_loss_grad<R>(p, &loss, penalty, batch, angles, loss_out, reg_out, grad_out,
-                                        (cudaStream_t)stream, table)));
+  CPF_DISPATCH(dtype, (run_loss_grad<R>(p, table->kind, 0, table->targets, penalty, batch, angles, loss_out, reg_out,
+                                        grad_out, (cudaStream_t)stream, table)));
 }
 
 int cpf_adam_run_multi(const cpf_program* prog, const cpf_target_table* table, const cpf_penalty_spec* penalty,
@@ -1104,34 +1024,18 @@ int cpf_adam_run_multi(const cpf_program* prog, const cpf_target_table* table, c
                        const cpf_adam_buffers* buf, void* stream) {
   if (!prog || !adam || !buf || batch < 0 || step0 < 0 || num_steps < 0)
     return fail(CPF_ERR_INVALID, "NULL argument / negative size");
+  if (int rc = check_table_pointers(table, batch)) return rc;
   const cpf::Program* p = reinterpret_cast<const cpf::Program*>(prog);
-  int rc = check_table(p, table, batch);
-  if (rc) return rc;
-  if (batch == 0 || num_steps == 0) return CPF_OK;
-  if (!buf->angles || !buf->m || !buf->v || !buf->best_params || !buf->best_regloss || !buf->best_reg ||
-      !buf->init_regloss || !buf->init_reg)
-    return fail(CPF_ERR_INVALID, "a required cpf_adam_buffers pointer is NULL");
-  if ((buf->hist_params || buf->hist_regloss) && buf->hist_len <= 0)
-    return fail(CPF_ERR_INVALID, "history buffers given with hist_len <= 0");
-  if (num_steps > 2000000000LL) return fail(CPF_ERR_INVALID, "num_steps too large");
-  const cpf_loss_spec loss{table->kind, table->targets, 0};
-  CPF_DISPATCH(dtype, (run_adam<R>(p, &loss, penalty, adam, batch, step0, num_steps, buf, (cudaStream_t)stream,
-                                   table)));
+  CPF_DISPATCH(dtype, (run_adam<R>(p, table->kind, 0, table->targets, penalty, adam, batch, step0, num_steps, buf,
+                                   (cudaStream_t)stream, table)));
 }
 
 int cpf_workspace_bytes_multi(const cpf_program* prog, int32_t loss_kind, int32_t dtype, int64_t batch,
                               int32_t n_targets, int64_t* bytes) {
   if (!prog || !bytes || batch < 0) return fail(CPF_ERR_INVALID, "NULL argument / negative batch");
-  if (loss_kind == CPF_LOSS_ISOMETRY)
-    return fail(CPF_ERR_UNSUPPORTED, "multi-target tables do not take the isometry loss (one target per call)");
-  if (loss_kind < CPF_LOSS_HS || loss_kind > CPF_LOSS_RELPHASE) return fail(CPF_ERR_INVALID, "unknown loss kind");
-  if (n_targets < 1) return fail(CPF_ERR_INVALID, "n_targets must be >= 1");
-  if (dtype != CPF_F32 && dtype != CPF_F64) return fail(CPF_ERR_INVALID, "unknown dtype");
   const cpf::Program* p = reinterpret_cast<const cpf::Program*>(prog);
-  if (int rc = check_full_unitary(p, loss_kind)) return rc;
-  *bytes = dtype == CPF_F64 ? workspace_bytes_multi_t<double>(p, loss_kind, batch, n_targets)
-                            : workspace_bytes_multi_t<float>(p, loss_kind, batch, n_targets);
-  return CPF_OK;
+  const cpf_target_table tt{loss_kind, n_targets, nullptr, nullptr};
+  CPF_DISPATCH(dtype, (workspace_t<R>(p, loss_kind, batch, &tt, bytes)));
 }
 
 int cpf_adam_step(const cpf_program* prog, const cpf_penalty_spec* penalty, const cpf_adam_spec* adam, int32_t dtype,
@@ -1140,11 +1044,7 @@ int cpf_adam_step(const cpf_program* prog, const cpf_penalty_spec* penalty, cons
   if (!prog || !adam || !buf || batch < 0 || step < 0) return fail(CPF_ERR_INVALID, "NULL argument / negative size");
   if (batch == 0) return CPF_OK;
   if (!loss || !grad) return fail(CPF_ERR_INVALID, "loss / grad is NULL");
-  if (!buf->angles || !buf->m || !buf->v || !buf->best_params || !buf->best_regloss || !buf->best_reg ||
-      !buf->init_regloss || !buf->init_reg)
-    return fail(CPF_ERR_INVALID, "a required cpf_adam_buffers pointer is NULL");
-  if ((buf->hist_params || buf->hist_regloss) && buf->hist_len <= 0)
-    return fail(CPF_ERR_INVALID, "history buffers given with hist_len <= 0");
+  if (int rc = check_adam_buffers(buf)) return rc;
   const cpf::Program* p = reinterpret_cast<const cpf::Program*>(prog);
   CPF_DISPATCH(dtype, (run_adam_step<R>(p, penalty, adam, batch, step, loss, grad, buf, (cudaStream_t)stream)));
 }
@@ -1218,47 +1118,13 @@ int cpf_initial_angles(const cpf_program* prog, int32_t dtype, uint64_t seed, in
 int cpf_eval_cost(const cpf_program* prog, int32_t loss_kind, int32_t dtype, double* flops, double* bytes) {
   if (!prog) return fail(CPF_ERR_INVALID, "NULL program");
   const cpf::Program* p = reinterpret_cast<const cpf::Program*>(prog);
-  int32_t kind, mask;
-  int rc = split_kind(p, loss_kind, &kind, &mask);
-  if (rc) return rc;
-  const double N = (double)(1 << p->n_qubits);
-  const double C = kind == CPF_LOSS_STATE ? 1.0 : kind == CPF_LOSS_ISOMETRY ? (double)iso_spec(p, mask).k : N;
-  const double rs = dtype == CPF_F64 ? 8.0 : 4.0;
-  if (flops) *flops = C * N * (16.0 * p->n_rot + 4.0 * p->n_phase + 8.0);
-  if (bytes) *bytes = 6.0 * p->n_params * rs + 2.0 * rs;
-  return CPF_OK;
+  CPF_DISPATCH(dtype, (eval_cost_t<R>(p, loss_kind, flops, bytes)));
 }
 
 int cpf_executed_cost(const cpf_program* prog, int32_t loss_kind, int32_t dtype, double* flops) {
   if (!prog || !flops) return fail(CPF_ERR_INVALID, "NULL argument");
   const cpf::Program* p = reinterpret_cast<const cpf::Program*>(prog);
-  const double N = (double)(1 << p->n_qubits), n = p->n_qubits, K = (double)p->cp.size(), G = (double)p->su2.size();
-  int32_t kind, mask;
-  int rc = split_kind(p, loss_kind, &kind, &mask);
-  if (rc) return rc;
-  // isometry: n <= 5 runs as an HS call; n >= 6 on the isometry kernel, the state-adjoint count with C = k
-  const bool iso = kind == CPF_LOSS_ISOMETRY && p->n_qubits > 5;
-  if (kind == CPF_LOSS_ISOMETRY && !iso) kind = CPF_LOSS_HS;
-  cpf_loss_spec ls{};
-  ls.kind = kind;
-  const bool heis = dtype == CPF_F64 ? use_heis<double>(p, &ls) : use_heis<float>(p, &ls);
-  if (heis) {
-    // heis_kernel (heis_impl.cuh), FMA = 2 flop, per sample and step:
-    //   forward   block: 3 diagonal phases on N/4 rows (6 flop per complex amplitude) + 2 Ry in lifting form (3 shears on
-    //             re and im): N^2 (4.5 + 12); surface gate: phase on N/2 rows + Ry: 9 N^2; pending phases at the end: 3 N^2
-    //   backward  fused gate: Rx exchange + merged Rz on the N^2 real coefficients: 4.5 N^2; ZZ pair rotations
-    //             (lifting): 3 N^2 per block; outgoing Rz of the last gate per qubit: 3 N^2
-    //   pivot     Walsh-Hadamard transform (re, im) + seed of h: N^2 (2 n + 6)
-    //   update    per fused gate: chain rule, 3 x Adam, 3 x sin/cos, SU(2) products, ZYZ data, staging: ~232;
-    //             per entangler: Adam, sin/cos, penalty, merged diagonal: ~80
-    *flops = N * N * (28.5 * K + 19.5 * n + 2.0 * n + 6.0) + 232.0 * G + 80.0 * K;
-  } else {
-    // state-adjoint kernels: the credited count plus the uncompute of phi (6 flop per amplitude and rotation on
-    // fused gates, 1.5 per phase gate), with fused gates instead of primitive rotations: C N (22 G + 5.5 K + 8)
-    const double C = kind == CPF_LOSS_STATE ? 1.0 : iso ? (double)iso_spec(p, mask).k : N;
-    *flops = C * N * (22.0 * G + 5.5 * K + 8.0) + 232.0 * G + 80.0 * K;
-  }
-  return CPF_OK;
+  CPF_DISPATCH(dtype, (executed_cost_t<R>(p, loss_kind, flops)));
 }
 
 int cpf_launch_plan(const cpf_program* prog, int32_t loss_kind, int32_t dtype, int64_t batch, int32_t n_sm,
@@ -1267,14 +1133,7 @@ int cpf_launch_plan(const cpf_program* prog, int32_t loss_kind, int32_t dtype, i
   if (batch < 0) return fail(CPF_ERR_INVALID, "negative batch");
   std::memset(out, 0, sizeof(*out));
   const cpf::Program* p = reinterpret_cast<const cpf::Program*>(prog);
-  int32_t kind, mask;
-  int rc = split_kind(p, loss_kind, &kind, &mask);
-  if (rc) return rc;
-  if (kind == CPF_LOSS_ISOMETRY && p->n_qubits > 5)
-    return dtype == CPF_F64 ? iso_plan_t<double>(p, mask, batch, out) : iso_plan_t<float>(p, mask, batch, out);
-  const cpf_loss_spec_kind_only lk{kind == CPF_LOSS_ISOMETRY ? CPF_LOSS_HS : kind};   // n <= 5: an HS call
-  return dtype == CPF_F64 ? launch_plan_t<double>(p, lk, batch, n_sm, regs_per_thread, out)
-                          : launch_plan_t<float>(p, lk, batch, n_sm, regs_per_thread, out);
+  CPF_DISPATCH(dtype, (launch_plan_t<R>(p, loss_kind, batch, n_sm, regs_per_thread, out)));
 }
 
 }  // extern "C"

@@ -25,7 +25,12 @@
  *     stream) and perform no hidden synchronisation;
  *   - qubit order is big-endian as in the reference: qubit 0 is the MOST significant bit of the
  *     row index of the unitary (cpflow/circuit_assembly.py:31-45);
- *   - a cpf_program is immutable after creation and may be shared by threads and streams.
+ *   - a cpf_program is immutable after creation and may be shared by threads and streams;
+ *   - a loss call (cpf_loss_grad, cpf_adam_run and their _multi forms) is refused before any CUDA call: loss kind
+ *     and mask, qubit limits, target table and target_index, penalty spec and cp_mask, dtype, Adam buffers and the
+ *     caller-owned workspace (alignment and size) are all checked first.  The query entry points
+ *     (cpf_workspace_bytes(_multi), cpf_launch_plan, cpf_eval_cost, cpf_executed_cost) refuse the same loss kinds
+ *     and dtypes with the same codes.
  */
 #ifndef CPFLOW_B200_H
 #define CPFLOW_B200_H
@@ -208,7 +213,9 @@ int cpf_adam_run(const cpf_program* prog, const cpf_loss_spec* loss,
 /* Device scratch one cpf_adam_run (or cpf_loss_grad) call on `batch` samples needs: the packed optimiser state
  * (16 bytes per parameter position and sample on the Heisenberg-picture kernel; positions are the parameters padded
  * to the lanes' pair slots, see heis_impl.cuh: heis_pk_stride), the staged target and the penalty mask.
- * Callers that manage device memory themselves allocate this once and pass it in cpf_adam_buffers.workspace. */
+ * Callers that manage device memory themselves allocate this once and pass it in cpf_adam_buffers.workspace; a call
+ * given a smaller or misaligned workspace is refused with CPF_ERR_INVALID (before any CUDA call, as every refusal of a
+ * loss call). */
 int cpf_workspace_bytes(const cpf_program* prog, int32_t loss_kind, int32_t dtype, int64_t batch, int64_t* bytes);
 
 /* One iteration of the same loop for a loss that is evaluated OUTSIDE the engine (an arbitrary user

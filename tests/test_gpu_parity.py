@@ -625,28 +625,53 @@ def test_time_sliced_runs_are_bit_identical():
 
 
 def test_caller_owned_workspace():
-    """cpf_workspace_bytes + cpf_adam_buffers.workspace (SURVEY.md 8b: 'per-call scratch from a caller-visible
-    workspace query'): the same bits as with the library's own pool scratch; a short or misaligned buffer is refused."""
-    anz = Ansatz(4, "cp", fill_layers(chain_layer(4), 12))
+    """cpf_workspace_bytes(_multi) + cpf_adam_buffers.workspace (SURVEY.md 8b: 'per-call scratch from a caller-visible
+    workspace query'), on every kernel route: a workspace of exactly the size the query gives yields the same bits as
+    the library's own pool scratch, one byte less or a misaligned buffer is refused."""
+    from cpflow_b200.engine import MultiLoss
     V = unitary_group.rvs(16, random_state=1)
+    V64 = unitary_group.rvs(64, random_state=2)
     B = 300
-    a = anz.program.initial_angles(4, B)
-    for kind, tgt in (("hs", V), ("state", V[:, 0].copy())):
-        lk = {"hs": L.LOSS_HS, "state": L.LOSS_STATE}[kind]
-        need = anz.program.workspace_bytes(B, lk)
-        assert need >= (16 * B * anz.num_angles if kind == "hs" else 256)
-        ref = anz.program.adam_state(a.clone())
-        anz.program.adam_run(ref, Loss(kind, tgt), pen(), 0.1, 20)
-        st = anz.program.adam_state(a.clone())
-        st.workspace = torch.empty(need, dtype=torch.uint8, device=DEV)
-        anz.program.adam_run(st, Loss(kind, tgt), pen(), 0.1, 20)
-        assert torch.equal(st.angles, ref.angles) and torch.equal(st.best_regloss, ref.best_regloss)
-        st.workspace = torch.empty(max(need - 512, 16), dtype=torch.uint8, device=DEV)
+    cases = [  # (name, n, loss, number of targets (0: adam_run), penalty mask on the CP parameters)
+        ("hs_heis", 4, Loss("hs", V), 0, False),
+        ("hs_heis_cp_mask", 4, Loss("hs", V), 0, True),
+        ("state", 4, Loss("state", V[:, 0].copy()), 0, False),
+        ("relphase", 4, Loss("relphase", V), 0, False),
+        ("isometry_as_hs", 4, Loss("isometry", V[:, :8], ancillas=[0]), 0, False),
+        ("isometry_6q", 6, Loss("isometry", V64[:, :16], ancillas=[0, 1]), 0, False),
+        ("multi_hs", 4, MultiLoss("hs", np.stack([V, V.conj().T, np.eye(16)])), 3, False),
+        ("multi_state", 4, MultiLoss("state", np.stack([V[:, 0], V[:, 1], V[:, 2]])), 3, True),
+    ]
+    for name, n, loss, n_targets, masked in cases:
+        anz = Ansatz(n, "cp", fill_layers(chain_layer(n), 12))
+        a = anz.program.initial_angles(4, B)
+        p = pen()
+        if masked:      # every other CP parameter: the penalty mask takes its own scratch block
+            p.cp_mask = np.zeros(anz.num_angles, dtype=np.uint8)
+            p.cp_mask[np.flatnonzero(anz.cp_mask)[::2]] = 1
+        idx = np.arange(B) % n_targets if n_targets else None
+
+        def run(workspace):
+            st = anz.program.adam_state(a.clone())
+            st.workspace = workspace
+            if n_targets:
+                anz.program.adam_run_multi(st, loss, idx, p, 0.1, 20)
+            else:
+                anz.program.adam_run(st, loss, p, 0.1, 20)
+            return st
+
+        need = anz.program.workspace_bytes_multi(B, n_targets, Loss.KINDS[loss.kind]) if n_targets else \
+            anz.program.workspace_bytes(B, loss.code)
+        if name == "hs_heis":
+            assert need >= 16 * B * anz.num_angles           # the packed optimiser state
+        ref = run(None)
+        st = run(torch.empty(need, dtype=torch.uint8, device=DEV))
+        for f in ("angles", "m", "v", "best_params", "best_regloss", "best_reg", "init_regloss", "init_reg"):
+            assert torch.equal(getattr(st, f), getattr(ref, f)), (name, f)
         with pytest.raises(L.CpflowError, match="workspace too small"):
-            anz.program.adam_run(st, Loss(kind, tgt), pen(), 0.1, 2)
-    st.workspace = torch.empty(need + 64, dtype=torch.uint8, device=DEV)[8:]
-    with pytest.raises(L.CpflowError, match="aligned"):
-        anz.program.adam_run(st, Loss("state", V[:, 0].copy()), pen(), 0.1, 2)
+            run(torch.empty(need - 1, dtype=torch.uint8, device=DEV))
+        with pytest.raises(L.CpflowError, match="aligned"):
+            run(torch.empty(need + 256, dtype=torch.uint8, device=DEV)[8:])
 
 
 def test_packed_update_matches_the_scalar_update():
