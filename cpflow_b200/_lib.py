@@ -17,11 +17,18 @@ MAX_QUBITS = 8
 RX, RY, RZ, CP, CZ, CX = 0, 1, 2, 3, 4, 5
 F32, F64 = 0, 1
 LOSS_HS, LOSS_STATE, LOSS_RELPHASE, LOSS_ISOMETRY = 0, 1, 2, 3
+LOSS_ISOMETRY_RELPHASE = 5
 
 
 def isometry_kind(ancilla_mask):
     """CPF_ISOMETRY_KIND: the loss-kind argument of the query entry points for an isometry loss."""
     return LOSS_ISOMETRY | (int(ancilla_mask) << 8)
+
+
+def isometry_relphase_kind(ancilla_mask):
+    """CPF_ISOMETRY_RELPHASE_KIND: the loss-kind argument of the query entry points for a relative-phase isometry
+    loss."""
+    return LOSS_ISOMETRY_RELPHASE | (int(ancilla_mask) << 8)
 PEN_NONE, PEN_PIECEWISE, PEN_L1 = 0, 1, 2
 
 

@@ -241,8 +241,8 @@ void stage_heis_state(const cpf::Program* prog, cpf::KParams<R>& p, void* blk, s
   p.pk_stride = cpf::heis_pk_stride(prog->n_qubits, (1 << prog->n_qubits) / cpt, (int)prog->su2.size(), (int)prog->cp.size());
 }
 
-// ---- isometry loss (CPF_LOSS_ISOMETRY) ----
-// Largest number of input columns k of the 6-8 qubit kernel: a sample is k lane groups of 2^(n-RB) threads in one CTA.
+// ---- isometry losses (CPF_LOSS_ISOMETRY, CPF_LOSS_ISOMETRY_RELPHASE) ----
+// Largest number of input columns k of the isometry kernel: a sample is k lane groups of 2^(n-RB) threads in one CTA.
 constexpr int ISO_MAX_K = 32;
 
 // k input columns; the ancilla qubits as amplitude-index bits (qubit q is bit n - 1 - q, big-endian)
@@ -265,14 +265,15 @@ enum Block { BLK_MASK, BLK_V, BLK_INDEX, BLK_TARGET, BLK_HEIS, N_BLK };
 template <typename R>
 struct CallPlan {
   Route route;          // the state-adjoint kernels, the Heisenberg-picture kernel (HS on layered templates) or the
-                        // isometry kernel (n >= 6); each in a single- or a multi-target form
+                        // isometry kernel (the isometry loss on n >= 6, the relative-phase isometry loss on every n);
+                        // each in a single- or a multi-target form
   bool multi;           // sample b is scored against target target_index[b] of a table
   bool layered;         // ROUTE_ADJOINT: try the kernel compiled for the layer before the interpreter
   bool single;          // single-column kernels (state loss, isometry kernel)
   bool iso_as_hs;       // n <= 5 isometry: the HS call on V = 2^a [W at the columns s_c, 0 elsewhere] (iso_impl.cuh:
                         // pack_iso_hs_kernel), built in BLK_V
   int32_t kind;         // the loss the kernel sees
-  IsoSpec iso;          // isometry kinds
+  IsoSpec iso;          // isometry kinds (CPF_LOSS_ISOMETRY, CPF_LOSS_ISOMETRY_RELPHASE)
   int n_stage;          // ROUTE_HEIS: SWP::NSTAGE of the kernel chosen
   int cpt, words;       // not ROUTE_ISO: columns per thread and words of one packed target
   size_t heis_aux;      // ROUTE_HEIS: per-gate scratch at the start of BLK_HEIS (the packed state follows, 256-byte aligned)
@@ -294,15 +295,21 @@ int plan_call(const cpf::Program* prog, int32_t kind, int32_t mask, int64_t batc
               const cpf_penalty_spec* pen, CallPlan<R>* pl) {
   const int n = prog->n_qubits;
   *pl = CallPlan<R>();
-  if (kind < CPF_LOSS_HS || kind > CPF_LOSS_ISOMETRY) return fail(CPF_ERR_INVALID, "unknown loss kind");
+  const bool phases = kind == CPF_LOSS_ISOMETRY_RELPHASE;
+  if ((kind < CPF_LOSS_HS || kind > CPF_LOSS_ISOMETRY) && !phases) return fail(CPF_ERR_INVALID, "unknown loss kind");
   if (table && kind == CPF_LOSS_ISOMETRY)
     return fail(CPF_ERR_UNSUPPORTED, "multi-target tables do not take the isometry loss (one target per call)");
+  if (table && phases)
+    return fail(CPF_ERR_UNSUPPORTED,
+                "multi-target tables do not take the relative-phase isometry loss (one target per call)");
   if (table && table->n_targets < 1) return fail(CPF_ERR_INVALID, "target table: n_targets must be >= 1");
-  // HS, relative phase and an isometry without ancillas run on the full-unitary kernels, which stop at 5 qubits
-  if (kind == CPF_LOSS_ISOMETRY) {
+  // HS, relative phase and an isometry without ancillas run on the full-unitary kernels, which stop at 5 qubits.  The
+  // relative-phase isometry loss runs on the isometry kernel on every n, so only its k is limited (k <= 32 always
+  // holds on n <= 5).
+  if (kind == CPF_LOSS_ISOMETRY || phases) {
     if (mask < 0 || (mask >> n) != 0)
       return fail(CPF_ERR_INVALID, "ancilla_mask " + std::to_string(mask) + " names a qubit >= n = " + std::to_string(n));
-    if (n > 5 && mask == 0) return fail(CPF_ERR_UNSUPPORTED, cpf::FULL_UNITARY_LIMIT);
+    if (n > 5 && mask == 0 && !phases) return fail(CPF_ERR_UNSUPPORTED, cpf::FULL_UNITARY_LIMIT);
     pl->iso = iso_spec(prog, mask);
     if (n > 5 && pl->iso.k > ISO_MAX_K)
       return fail(CPF_ERR_UNSUPPORTED, "isometry losses on 6-8 qubits take at most k = " + std::to_string(ISO_MAX_K) +
@@ -322,7 +329,7 @@ int plan_call(const cpf::Program* prog, int32_t kind, int32_t mask, int64_t batc
   pl->multi = table != nullptr;
   pl->iso_as_hs = kind == CPF_LOSS_ISOMETRY && n <= 5;
   pl->kind = pl->iso_as_hs ? CPF_LOSS_HS : kind;
-  pl->single = pl->kind == CPF_LOSS_STATE || pl->kind == CPF_LOSS_ISOMETRY;
+  pl->single = pl->kind == CPF_LOSS_STATE || pl->kind == CPF_LOSS_ISOMETRY || phases;
   pl->layered = layered_kernels(prog);
   // The Heisenberg-picture kernel keeps parameter and slot indices in 16 bits of shared memory (heis_impl.cuh: HSu2,
   // HCp) and B * P below 2^32.  CPF_ENGINE=adjoint forces the state-adjoint kernels (tests cover both engines).
@@ -336,7 +343,7 @@ int plan_call(const cpf::Program* prog, int32_t kind, int32_t mask, int64_t batc
     int rc = 0;
     heis = cpf::launch_heis<R>(dummy, *prog, nullptr, err, rc, true, &pl->n_stage);
   }
-  pl->route = pl->kind == CPF_LOSS_ISOMETRY ? ROUTE_ISO : heis ? ROUTE_HEIS : ROUTE_ADJOINT;
+  pl->route = pl->kind == CPF_LOSS_ISOMETRY || phases ? ROUTE_ISO : heis ? ROUTE_HEIS : ROUTE_ADJOINT;
 
   pl->bytes[BLK_MASK] = prog->cp.empty() ? 1 : prog->cp.size();
   pl->pen_mask = pl->pen.kind != CPF_PEN_NONE && pen->cp_mask && !prog->cp.empty();
@@ -451,7 +458,8 @@ int run_staged(const cpf::Program* prog, const CallPlan<R>& pl, const void* targ
 
   std::string err;
   if (pl.route == ROUTE_ISO) {
-    rc = cpf::launch_iso<R>(p, n, st, err);
+    rc = pl.kind == CPF_LOSS_ISOMETRY_RELPHASE ? cpf::launch_iso_phase<R>(p, n, st, err)
+                                               : cpf::launch_iso<R>(p, n, st, err);
   } else if (pl.route == ROUTE_HEIS) {
     if (!(pl.multi ? cpf::launch_heis_multi<R>(p, *prog, st, err, rc) : cpf::launch_heis<R>(p, *prog, st, err, rc, false))) {
       rc = CPF_ERR_UNSUPPORTED;
@@ -567,10 +575,12 @@ int run_adam(const cpf::Program* prog, int32_t kind, int32_t mask, const void* t
 }
 
 // The plan behind a query entry point's loss-kind argument: an isometry kind carries its ancilla mask in bits 8-15
-// (CPF_ISOMETRY_KIND); any other use of bits 8-31 makes an unknown kind.
+// (CPF_ISOMETRY_KIND, CPF_ISOMETRY_RELPHASE_KIND); any other use of bits 8-31 makes an unknown kind.
 template <typename R>
 int plan_query(const cpf::Program* prog, int32_t arg, int64_t batch, CallPlan<R>* pl) {
-  const int32_t kind = (arg & ~0xff00) == CPF_LOSS_ISOMETRY || (arg >> 8) == 0 ? arg & 0xff : -1;
+  const int32_t base = arg & ~0xff00;
+  const int32_t kind =
+      base == CPF_LOSS_ISOMETRY || base == CPF_LOSS_ISOMETRY_RELPHASE || (arg >> 8) == 0 ? arg & 0xff : -1;
   return plan_call<R>(prog, kind, (arg >> 8) & 0xff, batch, nullptr, nullptr, pl);
 }
 
@@ -836,7 +846,7 @@ static int launch_plan_t(const cpf::Program* prog, int32_t loss_kind, int64_t ba
     out->block_threads = g.block;
     out->samples_per_cta = g.spb;
     out->threads_per_sample = g.spt;
-    out->max_block_threads = n == 6 ? 512 : 1024;          // __launch_bounds__ of iso_kernel
+    out->max_block_threads = n <= 6 ? 512 : 1024;          // __launch_bounds__ of iso_kernel
     out->words_per_sample = cpf::iso_sample_words(cpf::coef_stride_words(n_su2, n_cp), k, cpf::iso_sum_stride(n_su2, n_cp));
     out->time_slices = 1;
     out->grid = (batch + g.spb - 1) / g.spb;
@@ -869,7 +879,7 @@ static int eval_cost_t(const cpf::Program* p, int32_t loss_kind, double* flops, 
   CallPlan<R> pl;
   if (int rc = plan_query<R>(p, loss_kind, 1, &pl)) return rc;
   const double N = (double)(1 << p->n_qubits);
-  const double C = pl.kind == CPF_LOSS_STATE ? 1.0 : pl.iso.k ? (double)pl.iso.k : N;     // isometry: C = k
+  const double C = pl.kind == CPF_LOSS_STATE ? 1.0 : pl.iso.k ? (double)pl.iso.k : N;     // isometry kinds: C = k
   const double rs = (double)sizeof(R);
   if (flops) *flops = C * N * (16.0 * p->n_rot + 4.0 * p->n_phase + 8.0);
   if (bytes) *bytes = 6.0 * p->n_params * rs + 2.0 * rs;
@@ -894,7 +904,8 @@ static int executed_cost_t(const cpf::Program* p, int32_t loss_kind, double* flo
   } else {
     // state-adjoint kernels: the credited count plus the uncompute of phi (6 flop per amplitude and rotation on
     // fused gates, 1.5 per phase gate), with fused gates instead of primitive rotations: C N (22 G + 5.5 K + 8);
-    // an isometry runs as an HS call on n <= 5 and on the isometry kernel with C = k on n >= 6
+    // an isometry runs as an HS call on n <= 5 and on the isometry kernel with C = k on n >= 6, the relative-phase
+    // isometry on the isometry kernel on every n
     const double C = pl.kind == CPF_LOSS_STATE ? 1.0 : pl.route == ROUTE_ISO ? (double)pl.iso.k : N;
     *flops = C * N * (22.0 * G + 5.5 * K + 8.0) + 232.0 * G + 80.0 * K;
   }

@@ -11,6 +11,9 @@
 // the parameter phase adds the k groups' sums in a fixed order.  No floating-point atomics: a sample's results do not
 // depend on its batch position or on how a run is split.  Barriers are CTA-wide (__syncthreads): a sample is more than
 // a warp, and the samples of a CTA run the same number of steps.
+//
+// The relative-phase isometry loss (InterpSweepIsoPhase, 2-8 qubits) runs the same kernel with one change: the loss is
+// 1 - sum_c |t_c|^2 / k, and each group seeds its adjoint with its own partial t_c (the HS seed with NN = k).
 #pragma once
 #include <string>
 
@@ -21,15 +24,21 @@ namespace cpf {
 // Register bits of the isometry kernel on NQ qubits: those of the single-column kernels (engine_rb(NQ, true)), whose
 // decoded schedule it runs; a lane group (one column) stays within one warp.
 template <int NQ> constexpr int iso_rb() { return NQ == 8 ? 3 : 2; }
+// engine_rb(NQ, true) on 2-8 qubits (inst_f32.cu: single_rb_f32, the same in float64): the register bits of the
+// relative-phase isometry kernel, which also runs 2-5 qubits
+template <int NQ> constexpr int iso_phase_rb() { return NQ == 8 ? 3 : NQ == 4 || NQ == 5 ? 1 : 2; }
 
-template <typename R, int NQ>
-struct InterpSweepIso : InterpSweep<R, NQ, iso_rb<NQ>(), 1, true> {
-  using Base = InterpSweep<R, NQ, iso_rb<NQ>(), 1, true>;
+// The sweep of iso_kernel with RB_ register bits.  The kernels' sweep types derive from it; they only set RB_ and the
+// mode flags: ISOMETRY (always), COTANGENT (InterpSweepIsoCot) and PHASES (InterpSweepIsoPhase).
+template <typename R, int NQ, int RB_>
+struct InterpSweepIsoRB : InterpSweep<R, NQ, RB_, 1, true> {
+  using Base = InterpSweep<R, NQ, RB_, 1, true>;
   using CO = typename Base::CO;
   using V = typename Base::V;
-  static constexpr int NA = Base::NA, LB = Base::LB, TPS = Base::TPS, RB = iso_rb<NQ>();
+  static constexpr int NA = Base::NA, LB = Base::LB, TPS = Base::TPS, RB = RB_;
   static constexpr bool ISOMETRY = true;
   static constexpr bool COTANGENT = false;
+  static constexpr bool PHASES = false;
   // InterpSweep::backward with the reduced sums stored at `sums` (this group's slots, reduce table re-pointed) instead
   // of over the coefficients, which the other groups of the sample may still be reading.
   static __device__ __forceinline__ void backward_into(const KParams<R>& p, const R* coef, R* sums, const uint2* s_dec,
@@ -104,6 +113,10 @@ struct InterpSweepIso : InterpSweep<R, NQ, iso_rb<NQ>(), 1, true> {
   }
 };
 
+// The isometry loss (one global phase) on 6-8 qubits.
+template <typename R, int NQ>
+struct InterpSweepIso : InterpSweepIsoRB<R, NQ, iso_rb<NQ>()> {};
+
 // The cotangent mode of iso_kernel (cpf_adjoint_from_cotangent on 6-8 qubits, DESIGN.md section 2.4): a launch item
 // is (sample b / n_chunks, column chunk b % n_chunks) with n_chunks = N / k; group c runs input column
 // (b % n_chunks) * k + c and seeds its adjoint with that column of the caller's cotangent instead of the loss seed.
@@ -112,6 +125,15 @@ struct InterpSweepIso : InterpSweep<R, NQ, iso_rb<NQ>(), 1, true> {
 template <typename R, int NQ>
 struct InterpSweepIsoCot : InterpSweepIso<R, NQ> {
   static constexpr bool COTANGENT = true;
+};
+
+// The relative-phase isometry loss (CPF_LOSS_ISOMETRY_RELPHASE, DESIGN.md section 2.4), on 2-8 qubits:
+// L = 1 - sum_c |t_c|^2 / k with t_c = <W e_c| U |s_c>, W up to a phase per input column.  Group c seeds its adjoint
+// with its own t_c / k instead of the shared t / k^2.  The register bits are those of the single-column split on every
+// n (iso_phase_rb), so on 4-5 qubits they differ from iso_rb.
+template <typename R, int NQ>
+struct InterpSweepIsoPhase : InterpSweepIsoRB<R, NQ, iso_phase_rb<NQ>()> {
+  static constexpr bool PHASES = true;
 };
 
 // words per group of the per-group gradient sums (odd: the groups of a sample store the same slot in distinct banks)
@@ -263,7 +285,7 @@ __host__ __device__ inline int iso_sample_words(int coef_stride, int k, int sum_
 }
 
 template <typename R, int NQ, typename SW>
-__global__ void __launch_bounds__(NQ == 6 ? 512 : 1024, 1) iso_kernel(const KParams<R> p) {
+__global__ void __launch_bounds__(NQ <= 6 ? 512 : 1024, 1) iso_kernel(const KParams<R> p) {
   constexpr int RB = SW::RB;
   using C = Cfg<R, NQ, RB, 1, true>;
   using T = VT<R, 1>;
@@ -350,12 +372,31 @@ __global__ void __launch_bounds__(NQ == 6 ? 512 : 1024, 1) iso_kernel(const KPar
       if (la == 0) { part[3 * grp] = tr_c; part[3 * grp + 1] = ti_c; part[3 * grp + 2] = reg_c; }
     }
     __syncthreads();
-    R tr = part[0], ti = part[1], reg = part[2];
-    for (int c = 1; c < k; ++c) { tr += part[3 * c]; ti += part[3 * c + 1]; reg += part[3 * c + 2]; }
-    const R ab = sqrt_r(tr * tr + ti * ti);
-    const R loss = R(1) - mul_rn(ab, ab) / NN;
+    R tr = part[0], ti = part[1], reg = part[2], loss;
     V lr[NA], li[NA];
-    {
+    if constexpr (SW::PHASES) {
+      // a phase per column: every thread adds sum_c |t_c|^2 and the penalty shares in group order; group grp seeds
+      // with its own t_c / k
+      R s2 = tr * tr + ti * ti;
+      for (int c = 1; c < k; ++c) {
+        const R xr = part[3 * c], xi = part[3 * c + 1];
+        s2 += xr * xr + xi * xi;
+        reg += part[3 * c + 2];
+      }
+      const R kk = R(k);
+      loss = R(1) - s2 / kk;
+      const R tr_c = part[3 * grp], ti_c = part[3 * grp + 1];
+      const V a = T::bc(-tr_c / kk), bq = T::bc(ti_c / kk), nb = T::bc(-ti_c / kk);
+#pragma unroll
+      for (int j = 0; j < NA; ++j) {
+        const V vr = tv[2 * j], vi = tv[2 * j + 1];
+        lr[j] = T::fma(bq, vi, T::mul(a, vr));
+        li[j] = T::fma(nb, vr, T::mul(a, vi));
+      }
+    } else {
+      for (int c = 1; c < k; ++c) { tr += part[3 * c]; ti += part[3 * c + 1]; reg += part[3 * c + 2]; }
+      const R ab = sqrt_r(tr * tr + ti * ti);
+      loss = R(1) - mul_rn(ab, ab) / NN;
       const V a = T::bc(-tr / NN), bq = T::bc(ti / NN), nb = T::bc(-ti / NN);
 #pragma unroll
       for (int j = 0; j < NA; ++j) {
@@ -495,6 +536,8 @@ int launch_iso_sized(KParams<R> p, cudaStream_t st, std::string& err) {
 
 // inst_iso_f32.cu / inst_iso_f64.cu
 template <typename R> int launch_iso(const KParams<R>& p, int n_qubits, cudaStream_t st, std::string& err);
+// inst_iso_phase_f32.cu / inst_iso_phase_f64.cu: the relative-phase isometry loss on 2-8 qubits
+template <typename R> int launch_iso_phase(const KParams<R>& p, int n_qubits, cudaStream_t st, std::string& err);
 // cotangent mode: p.B launch items of p.iso_k columns (p.B = batch * N / p.iso_k), gradients to p.grad_out [p.B][P]
 template <typename R> int launch_iso_cot(const KParams<R>& p, int n_qubits, cudaStream_t st, std::string& err);
 template <typename R> int launch_cot_reduce(const R* partial, R* grad, long long batch, int P, int n_chunks,

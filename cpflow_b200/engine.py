@@ -286,23 +286,31 @@ class AdamState:
 
 
 class Loss:
-    """Declarative loss spec (cpf_loss_spec): 'hs' | 'state' | 'relphase' | 'isometry' and a target array.
+    """Declarative loss spec (cpf_loss_spec): 'hs' | 'state' | 'relphase' | 'isometry' | 'isometry_relphase' and a
+    target array.
 
     'isometry' takes `ancillas`, the qubits that start in |0>: with k = 2^(n - len(ancillas)) and s_0 < ... < s_{k-1}
     the basis states whose ancilla qubits are 0, the target W is N x k (column c = the wanted image of |s_c>) and the
-    loss is 1 - |sum_c <W e_c| U |s_c>|^2 / k^2 (one global phase, like 'hs')."""
-    KINDS = {"hs": L.LOSS_HS, "state": L.LOSS_STATE, "relphase": L.LOSS_RELPHASE, "isometry": L.LOSS_ISOMETRY}
+    loss is 1 - |sum_c <W e_c| U |s_c>|^2 / k^2 (one global phase, like 'hs').
+
+    'isometry_relphase' takes the same `ancillas` and W, and keeps a phase per input column:
+    1 - sum_c |<W e_c| U |s_c>|^2 / k.  It is 0 exactly when U|s_c> = e^{i phi_c} W e_c for every c (relative-phase
+    gates with clean ancillas, states each prepared up to its own phase, a unitary up to a diagonal on the input
+    side), and runs fused on 2-8 qubits with k <= 32."""
+    KINDS = {"hs": L.LOSS_HS, "state": L.LOSS_STATE, "relphase": L.LOSS_RELPHASE, "isometry": L.LOSS_ISOMETRY,
+             "isometry_relphase": L.LOSS_ISOMETRY_RELPHASE}
+    ISOMETRY_KINDS = ("isometry", "isometry_relphase")
 
     def __init__(self, kind, target, ancillas=None):
         if kind not in self.KINDS:
             raise ValueError(f"unknown loss kind {kind!r}")
-        if ancillas is not None and kind != "isometry":
+        if ancillas is not None and kind not in self.ISOMETRY_KINDS:
             raise ValueError(f"ancillas are an argument of the 'isometry' loss, not of {kind!r}")
         self.kind = kind
         self.target = np.asarray(target.detach().cpu().numpy() if isinstance(target, torch.Tensor) else target,
                                  dtype=np.complex128)
         self.ancillas = ()
-        if kind == "isometry":
+        if kind in self.ISOMETRY_KINDS:
             self.ancillas = _check_isometry(self.target, ancillas)
         self._dev = {}
 
@@ -312,7 +320,8 @@ class Loss:
 
     @property
     def columns(self):
-        """Basis indices s_0 < ... < s_{k-1} of the input columns ('isometry'): ancilla qubits (big-endian) are 0."""
+        """Basis indices s_0 < ... < s_{k-1} of the input columns (the isometry kinds): ancilla qubits (big-endian) are
+        0."""
         n = int(self.target.shape[0]).bit_length() - 1
         bits = sum(1 << (n - 1 - q) for q in self.ancillas)
         return tuple(s for s in range(2 ** n) if s & bits == 0)
@@ -320,7 +329,11 @@ class Loss:
     @property
     def code(self):
         """The loss-kind argument of the query entry points (workspace_bytes, launch_plan, eval_cost, executed_cost)."""
-        return L.isometry_kind(self.ancilla_mask) if self.kind == "isometry" else self.KINDS[self.kind]
+        if self.kind == "isometry":
+            return L.isometry_kind(self.ancilla_mask)
+        if self.kind == "isometry_relphase":
+            return L.isometry_relphase_kind(self.ancilla_mask)
+        return self.KINDS[self.kind]
 
     def spec(self, dtype, device):
         key = (dtype, str(device))
@@ -348,11 +361,14 @@ class Loss:
         if self.kind == "isometry":
             k = self.target.shape[1]
             return float(1 - np.abs((self.target.conj() * u[:, list(self.columns)]).sum()) ** 2 / k ** 2)
+        if self.kind == "isometry_relphase":
+            t = (self.target.conj() * u[:, list(self.columns)]).sum(0)
+            return float(1 - (np.abs(t) ** 2).sum() / self.target.shape[1])
         return float(1 - (np.abs(self.target.conj() * u) ** 2).sum() / n)
 
     def __repr__(self):
-        if self.kind == "isometry":
-            return f"Loss('isometry', target{tuple(self.target.shape)}, ancillas={list(self.ancillas)})"
+        if self.kind in self.ISOMETRY_KINDS:
+            return f"Loss({self.kind!r}, target{tuple(self.target.shape)}, ancillas={list(self.ancillas)})"
         return f"Loss({self.kind!r}, target{tuple(self.target.shape)})"
 
 

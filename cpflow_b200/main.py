@@ -55,6 +55,10 @@ def batched_unitary_loss(unitary_loss_func, U):
             k = tgt.shape[1]
             t = (tgt.conj() * U[:, :, list(unitary_loss_func.columns)]).sum((-1, -2))
             return (1 - t.abs() ** 2 / k ** 2).cpu().numpy()
+        if unitary_loss_func.kind == 'isometry_relphase':
+            k = tgt.shape[1]
+            t = (tgt.conj() * U[:, :, list(unitary_loss_func.columns)]).sum(-2)
+            return (1 - (t.abs() ** 2).sum(-1) / k).cpu().numpy()
         return (1 - ((tgt.conj() * U).abs() ** 2).sum((-1, -2)) / n).cpu().numpy()
     if isinstance(unitary_loss_func, TorchLoss):
         with torch.no_grad():

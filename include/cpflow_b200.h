@@ -82,7 +82,8 @@ typedef enum cpf_loss_kind {
   CPF_LOSS_HS = 0,       /* 1 - |sum_ij U_ij conj(V_ij)|^2 / N^2   matrix_utils.py:35-42 */
   CPF_LOSS_STATE = 1,    /* 1 - |<psi| U |0>|^2                    tutorial ipynb:1318    */
   CPF_LOSS_RELPHASE = 2, /* 1 - sum_ij |conj(V_ij) U_ij|^2 / N     tutorial ipynb:1507    */
-  CPF_LOSS_ISOMETRY = 3  /* 1 - |sum_c <W e_c| U |s_c>|^2 / k^2     (ancilla qubits start in |0>) */
+  CPF_LOSS_ISOMETRY = 3, /* 1 - |sum_c <W e_c| U |s_c>|^2 / k^2     (ancilla qubits start in |0>) */
+  CPF_LOSS_ISOMETRY_RELPHASE = 5 /* 1 - sum_c |<W e_c| U |s_c>|^2 / k  (ancillas in |0>, a phase per column) */
 } cpf_loss_kind;
 
 /* ISOMETRY: the qubits of `ancilla_mask` (bit q = qubit q) start in |0>, so only the images of the k = 2^(n - popcount)
@@ -90,16 +91,28 @@ typedef enum cpf_loss_kind {
  * image of |s_c>.  One global phase, like HS: ancilla_mask = 0 is the HS loss, all qubits (k = 1) the state loss.
  * n <= 5 runs on the HS kernels (target 2^a [W at the columns s_c, 0 elsewhere], N = 2^a k: exact scaling); n = 6-8
  * on the isometry kernel with k <= 32 (k > 32 and ancilla_mask = 0 are CPF_ERR_UNSUPPORTED).  Not for multi-target
- * tables.  A mask bit at a position >= n is CPF_ERR_INVALID. */
+ * tables.  A mask bit at a position >= n is CPF_ERR_INVALID.
+ *
+ * ISOMETRY_RELPHASE: the same ancilla_mask, k, s_c and N x k target W, but W up to a phase per input column:
+ * L = 1 - (1/k) sum_c |t_c|^2 with t_c = <W e_c| U |s_c>.  L = 0 exactly when U|s_c> = e^{i phi_c} W e_c for every c
+ * (unit-norm columns), and L does not change under W -> W D for a diagonal phase matrix D: relative-phase gates with
+ * clean ancillas, sets of states each prepared up to its own phase, a unitary up to a diagonal on the input side.
+ * ancilla_mask = 0 with a W of one unit-modulus entry per column is the RELPHASE loss; k = 1 is the state loss.  Runs
+ * on the isometry kernel on 2-8 qubits (group c seeds its adjoint with its own t_c / k), with k <= 32 on every n:
+ * k > 32 (ancilla_mask = 0 on 6-8 qubits included) is CPF_ERR_UNSUPPORTED, as are multi-target tables; a mask bit
+ * at a position >= n is CPF_ERR_INVALID.  (The value 5 leaves 4 unassigned.) */
 typedef struct cpf_loss_spec {
   int32_t kind;       /* cpf_loss_kind */
-  const void* target; /* device: N*N complex row-major (HS, RELPHASE), N complex (STATE), N*k row-major (ISOMETRY) */
-  int32_t ancilla_mask; /* ISOMETRY only (ignored for the other kinds) */
+  const void* target; /* device: N*N complex row-major (HS, RELPHASE), N complex (STATE), N*k row-major (ISOMETRY,
+                         ISOMETRY_RELPHASE) */
+  int32_t ancilla_mask; /* ISOMETRY and ISOMETRY_RELPHASE only (ignored for the other kinds) */
 } cpf_loss_spec;
 
 /* cpf_workspace_bytes, cpf_eval_cost, cpf_executed_cost and cpf_launch_plan take a loss kind only: for the isometry
- * loss pass CPF_ISOMETRY_KIND(ancilla_mask), which carries the mask in bits 8-15. */
+ * losses pass CPF_ISOMETRY_KIND(ancilla_mask) or CPF_ISOMETRY_RELPHASE_KIND(ancilla_mask), which carry the mask in
+ * bits 8-15. */
 #define CPF_ISOMETRY_KIND(ancilla_mask) ((int32_t)CPF_LOSS_ISOMETRY | ((int32_t)(ancilla_mask) << 8))
+#define CPF_ISOMETRY_RELPHASE_KIND(ancilla_mask) ((int32_t)CPF_LOSS_ISOMETRY_RELPHASE | ((int32_t)(ancilla_mask) << 8))
 
 typedef enum cpf_penalty_kind {
   CPF_PEN_NONE = 0,
@@ -275,7 +288,7 @@ int cpf_initial_angles(const cpf_program* prog, int32_t dtype, uint64_t seed,
 
 /* Algorithmic work of one loss+grad evaluation, SURVEY.md §8(d):
  * flops = C*N*(16*G1 + 4*K + 8), bytes = 6*P*sizeof(real) + 2*sizeof(real); C = N columns (HS, RELPHASE), 1 (STATE),
- * k (ISOMETRY). */
+ * k (ISOMETRY, ISOMETRY_RELPHASE). */
 int cpf_eval_cost(const cpf_program* prog, int32_t loss_kind, int32_t dtype, double* flops,
                   double* bytes);
 
