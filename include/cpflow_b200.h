@@ -160,7 +160,9 @@ typedef struct cpf_program_info {
 typedef struct cpf_adam_buffers {
   void* angles;            /* [B,P] in: theta at step `step0`; out: theta after the last step */
   void* m;                 /* [B,P] first moment  (ignored on input when step0 == 0) */
-  void* v;                 /* [B,P] second moment (ignored on input when step0 == 0) */
+  void* v;                 /* [B,P] second moment (ignored on input when step0 == 0).  After a fresh run the
+                              moments of frozen parameters and of parameters that feed no gate are 0; a resumed
+                              run (step0 > 0) leaves them unchanged */
   const uint8_t* freeze;   /* [B,P] nullable; nonzero = parameter is frozen (never updated):
                               the reduced vector of cp_utils.py:100-108 */
   void* best_params;       /* [B,P] params at the lowest regloss so far (optimization.py:70-73) */

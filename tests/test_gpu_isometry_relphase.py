@@ -1,14 +1,13 @@
 """Relative-phase isometry loss on the device: parity with a float64 autograd reference, the fused Adam loop,
 cross-checks with the relphase and isometry kernels, bitwise determinism and end-to-end synthesis with known optima.
 
-The reference, L = 1 - (1/k) sum_c |<W e_c| U |s_c>|^2, is built here on the oracle's program unitary, penalty and
-optax Adam, as tests/isometry_ref.py does for the isometry loss."""
+The float64 reference, L = 1 - (1/k) sum_c |<W e_c| U |s_c>|^2, is tests/isometry_ref.py's (relphase=True)."""
 import numpy as np
 import pytest
 import torch
 from scipy.stats import unitary_group
 
-from isometry_ref import columns
+import isometry_ref as R
 from cpflow_b200 import ansatz as A
 from cpflow_b200 import _lib as L
 from cpflow_b200.engine import Loss, Penalty, Program, clean_ancilla_isometry
@@ -21,29 +20,6 @@ from oracle import cpflow_oracle as O
 pytestmark = pytest.mark.gpu
 DEV = "cuda"
 TOL = {torch.float64: 1e-12, torch.float32: 1e-5}
-
-
-# ---------------- float64 reference ----------------
-def ref_loss_batched(u, W, cols):
-    t = (W.conj()[None] * u[:, :, cols]).sum(-2)                  # [B, k]: t_c = <W e_c| U |s_c>
-    return 1 - (torch.abs(t) ** 2).sum(-1) / W.shape[1]
-
-
-def ref_loss_and_grad(n, ops, angles, W, ancillas, cp_mask=None, r=0.0, penalty_func=None):
-    W = torch.as_tensor(W, dtype=torch.complex128)
-    a = angles.clone().double().requires_grad_(True)
-    u = O.program_unitary_batched(n, ops, a)
-    loss = ref_loss_batched(u, W, columns(n, ancillas))
-    reg = O.regularization_value(a, cp_mask, r, penalty_func) if penalty_func is not None else torch.zeros_like(loss)
-    (loss + reg).sum().backward()
-    return loss.detach(), reg.detach(), a.grad.detach()
-
-
-def ref_adam(n, ops, W, ancillas, x0, lr, T, cp_mask, r, penalty_func):
-    def lg(p):
-        loss, reg, g = ref_loss_and_grad(n, ops, p, W, ancillas, cp_mask, r, penalty_func)
-        return loss + reg, g
-    return O.adam_minimize_batched(lg, torch.as_tensor(x0).double(), lr, T)
 
 
 # ---------------- helpers ----------------
@@ -73,8 +49,8 @@ def _check(prog, cp_mask, loss, a, dt):
     pf = make_regularization_function(RegularizationOptions)
     pen = Penalty("piecewise", 0.002, pf.segments, pf.period, cp_mask=sub)
     lo, rg, gr = prog.loss_grad(a.to(dt).contiguous(), loss, pen)
-    ol, orr, og = ref_loss_and_grad(prog.n_qubits, prog.ops, a.cpu().double(), loss.target, loss.ancillas,
-                                    torch.as_tensor(sub), 0.002, O.make_regularization_function())
+    ol, orr, og = R.loss_and_grad_batched(prog.n_qubits, prog.ops, a.cpu().double(), loss.target, loss.ancillas,
+                                          torch.as_tensor(sub), 0.002, O.make_regularization_function(), relphase=True)
     assert float(orr.abs().max()) > 0                               # the penalty takes part
     for x, y in ((lo, ol), (rg, orr), (gr, og)):
         assert _rel(x.cpu().double().numpy(), y.numpy()) < TOL[dt]
@@ -135,8 +111,8 @@ def test_adam_against_reference(n, anc):
     a0 = torch.rand(B, anz.num_angles, dtype=torch.float64) * 6
     st = anz.program.adam_state(a0.to(DEV).clone())
     anz.program.adam_run(st, loss, _penalty(), 0.1, T)
-    params, regloss = ref_adam(n, anz.program.ops, loss.target, anc, a0, 0.1, T, torch.as_tensor(anz.cp_mask), 0.002,
-                               O.make_regularization_function())
+    params, regloss = R.mynimize_repeated(n, anz.program.ops, loss.target, anc, a0, 0.1, T, torch.as_tensor(anz.cp_mask),
+                                          0.002, O.make_regularization_function(), relphase=True)
     assert _rel(st.best_regloss.cpu().numpy(), regloss[:, 1].numpy()) < 1e-9
     assert _rel(st.init_regloss.cpu().numpy(), regloss[:, 0].numpy()) < 1e-9
     assert _rel(st.best_params.cpu().numpy(), params[:, 1].numpy()) < 1e-9

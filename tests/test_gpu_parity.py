@@ -14,13 +14,14 @@ from oracle import cpflow_oracle as O
 from conftest import hst
 from cpflow_b200 import _lib as L
 from cpflow_b200.ansatz import Ansatz
-from cpflow_b200.engine import Loss, Penalty, Program
+from cpflow_b200.engine import Loss, MultiLoss, Penalty, Program
 from cpflow_b200.gates import u_toff3, u_toff4
 from cpflow_b200.topology import chain_layer, connected_layer, fill_layers
 
 pytestmark = pytest.mark.gpu
 DEV = "cuda"
-from parity_lib import CONFIGS, KITE4, PF, SQUARE4, STAR4, TOL, measure_adam_loop, measure_loss_grad, pen, rel, setup  # noqa: E402
+from parity_lib import (CONFIGS, KITE4, PF, SQUARE4, STAR4, TOL, host_loss, host_steps, measure_adam_loop,  # noqa: E402
+                        measure_loss_grad, pen, poisoned_state, rel, setup, with_dispatch_env)
 
 
 @pytest.mark.parametrize("n,layer,K,rg", CONFIGS)
@@ -722,22 +723,86 @@ def test_large_angles_leave_the_fast_range_reduction():
     assert float((lo.cpu().double() - ol).abs().max()) < 1e-5
 
 
+# Routes of the Adam loop for test_parameters_that_feed_no_gate: (qubits, layer, CP gates, loss kind, ancillas,
+# number of targets (0: single-target run), dispatch switches, samples)
+NO_GATE_ROUTES = {
+    "heis": (3, chain_layer(3), 6, "hs", None, 0, {}, 33),
+    "heis_any": (4, KITE4, 10, "hs", None, 0, {"CPF_HEIS_ANY": "1"}, 33),
+    "heis_mt": (3, chain_layer(3), 6, "hs", None, 3, {}, 33),
+    "layered": (5, chain_layer(5), 8, "state", None, 0, {}, 33),
+    "interp": (6, chain_layer(6), 7, "state", None, 0, {}, 33),
+    "interp_mt": (6, chain_layer(6), 7, "state", None, 3, {}, 33),
+    "iso6": (6, chain_layer(6), 7, "isometry", [0, 2, 4], 0, {}, 33),
+    "iso7": (7, chain_layer(7), 7, "isometry", [1, 5], 0, {}, 20),
+    "iso8": (8, chain_layer(8), 7, "isometry", [0, 3, 7], 0, {}, 12),
+    "isorel3": (3, chain_layer(3), 6, "isometry_relphase", [], 0, {}, 33),
+    "isorel8": (8, chain_layer(8), 7, "isometry_relphase", [1, 4, 6], 0, {}, 12),
+    "iso_as_hs": (4, chain_layer(4), 8, "isometry", [0], 0, {}, 33),
+    "host": (4, chain_layer(4), 8, "hs", None, 0, {}, 33),
+}
+_NO_GATE_STATE = ("angles", "m", "v", "best_params", "best_regloss", "best_reg", "init_regloss", "init_reg")
+_PER_PARAMETER = ("angles", "m", "v", "best_params", "hist_params")
+
+
 def test_parameters_that_feed_no_gate():
-    """A program whose parameter vector is longer than its gates use (the packed optimiser state holds referenced
-    parameters only): the unused entries keep their angles, get zero moments and their own value as best parameter."""
-    from cpflow_b200.engine import Program
-    anz = Ansatz(3, "cp", fill_layers(chain_layer(3), 6))
-    ops, P = anz.program.ops, anz.num_angles
-    prog = Program(3, ops, P + 3)
-    ref = Program(3, ops, P)
-    V = unitary_group.rvs(8, random_state=1)
-    a = torch.tensor(np.random.default_rng(2).uniform(0, 6.28, (33, P + 3)), dtype=torch.float32, device=DEV)
-    for hist in (False, True):
-        st = prog.adam_state(a.clone(), hist_len=7 if hist else 0)
-        prog.adam_run(st, Loss("hs", V), None, 0.1, 7)
-        rf = ref.adam_state(a[:, :P].contiguous().clone(), hist_len=7 if hist else 0)
-        ref.adam_run(rf, Loss("hs", V), None, 0.1, 7)
-        assert torch.equal(st.angles[:, :P], rf.angles) and torch.equal(st.best_regloss, rf.best_regloss)
-        assert torch.equal(st.best_params[:, :P], rf.best_params) and torch.equal(st.m[:, :P], rf.m)
-        assert torch.equal(st.angles[:, P:], a[:, P:]) and torch.equal(st.best_params[:, P:], a[:, P:])
-        assert float(st.m[:, P:].abs().max()) == 0.0 and float(st.v[:, P:].abs().max()) == 0.0
+    """A program whose parameter vector is longer than its gates use (3 parameters feed no gate), on every route of the
+    Adam loop (NO_GATE_ROUTES; 'host': the host-driven loop of callable losses, cpf_adam_step), with and without a
+    freeze mask and a history.  After a fresh 7-step run from NaN-filled buffers no entry of the state is NaN; frozen
+    and unreferenced entries keep their angles and come back with zero moments (cpf_adam_buffers: a fresh run starts
+    the moments at zero); the referenced entries are bit-identical to the same run of the program without the extra
+    parameters (the Heisenberg kernel's packed optimiser state holds referenced parameters only, the other kernels
+    never visit the extra entries).  Every route is run; the failure lists each route that failed."""
+    failed = []
+    for route in NO_GATE_ROUTES:
+        try:
+            _check_no_gate_route(route)
+        except AssertionError as e:
+            failed.append(f"{route}: {str(e).splitlines()[0]}")
+    assert not failed, "routes that failed:\n" + "\n".join(failed)
+
+
+def _check_no_gate_route(route):
+    n, layer, K, kind, anc, nt, env, B = NO_GATE_ROUTES[route]
+    anz = Ansatz(n, "cp", fill_layers(layer, K))
+    ops, P, N = anz.program.ops, anz.num_angles, 2 ** n
+    prog, ref = Program(n, ops, P + 3), Program(n, ops, P)
+    V = unitary_group.rvs(N, random_state=1)
+    tgt = V[:, 0].copy() if kind == "state" else (V[:, :2 ** (n - len(anc))] if anc is not None else V)
+    if nt:
+        loss = MultiLoss(kind, np.stack([tgt, tgt.conj(), np.roll(tgt, 1, axis=0)]))
+        idx = np.arange(B) % nt
+    else:
+        loss = host_loss(kind, tgt) if route == "host" else Loss(kind, tgt, ancillas=anc)
+    rng = np.random.default_rng(2)
+    a = torch.tensor(rng.uniform(0, 6.28, (B, P + 3)), dtype=torch.float32, device=DEV)
+    fm = torch.tensor(rng.random((B, P + 3)) < 0.2, dtype=torch.uint8, device=DEV)
+
+    def run(pr, angles, freeze, hist):
+        st = poisoned_state(pr, angles.clone(), freeze=freeze, hist_len=7 if hist else 0)
+        if route == "host":
+            host_steps(pr, st, loss, None, 0.1, 7)
+        elif nt:
+            pr.adam_run_multi(st, loss, idx, None, 0.1, 7)
+        else:
+            pr.adam_run(st, loss, None, 0.1, 7)
+        torch.cuda.synchronize()
+        return st
+
+    for freeze in (None, fm):
+        for hist in (False, True):
+            where = (route, "freeze" if freeze is not None else "no freeze", "history" if hist else "no history")
+            st = with_dispatch_env(env, lambda: run(prog, a, freeze, hist))
+            rf = with_dispatch_env(env, lambda: run(ref, a[:, :P].contiguous(),
+                                                    None if freeze is None else freeze[:, :P].contiguous(), hist))
+            names = _NO_GATE_STATE + (("hist_params", "hist_regloss") if hist else ())
+            for name in names:
+                x, y = getattr(st, name), getattr(rf, name)
+                assert not torch.isnan(x).any(), where + (name,)
+                assert torch.equal(x[..., :P] if name in _PER_PARAMETER else x, y), where + (name,)
+            still = torch.zeros_like(fm, dtype=torch.bool) if freeze is None else freeze.bool()
+            still[:, P:] = True
+            assert torch.equal(st.angles[still], a[still]), where
+            assert bool((st.m[still] == 0).all()) and bool((st.v[still] == 0).all()), where
+            assert torch.equal(st.best_params[:, P:], a[:, P:]), where
+            if hist:
+                assert torch.equal(st.hist_params[:, :, P:], a[:, None, P:].expand(B, 7, 3)), where

@@ -1,7 +1,7 @@
 """Measured parity maxima of the CUDA engine against the CPU oracle (run on the GPU box):
 
     python tools/parity_report.py > profiles/parity_r2.txt
-    python tools/parity_report.py --steps > profiles/adam_steps_r1.txt
+    python tools/parity_report.py --steps > profiles/adam_steps_r2.txt
 
 Same measurement functions as tests/test_gpu_parity.py (tests/parity_lib.py); the tests assert the contract's
 tolerances (1e-5 complex64, 1e-12 complex128), this prints what was actually measured per configuration."""
