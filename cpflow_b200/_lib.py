@@ -18,6 +18,7 @@ RX, RY, RZ, CP, CZ, CX = 0, 1, 2, 3, 4, 5
 F32, F64 = 0, 1
 LOSS_HS, LOSS_STATE, LOSS_RELPHASE, LOSS_ISOMETRY = 0, 1, 2, 3
 LOSS_ISOMETRY_RELPHASE = 5
+LOSS_SUBSPACE, LOSS_SUBSPACE_RELPHASE = 6, 7
 
 
 def isometry_kind(ancilla_mask):
@@ -29,6 +30,17 @@ def isometry_relphase_kind(ancilla_mask):
     """CPF_ISOMETRY_RELPHASE_KIND: the loss-kind argument of the query entry points for a relative-phase isometry
     loss."""
     return LOSS_ISOMETRY_RELPHASE | (int(ancilla_mask) << 8)
+
+
+def subspace_kind(k):
+    """CPF_SUBSPACE_KIND: the loss-kind argument of the query entry points for a subspace loss on k input states."""
+    return LOSS_SUBSPACE | (int(k) << 8)
+
+
+def subspace_relphase_kind(k):
+    """CPF_SUBSPACE_RELPHASE_KIND: the loss-kind argument of the query entry points for a relative-phase subspace loss
+    on k input states."""
+    return LOSS_SUBSPACE_RELPHASE | (int(k) << 8)
 PEN_NONE, PEN_PIECEWISE, PEN_L1 = 0, 1, 2
 
 

@@ -245,11 +245,12 @@ void stage_heis_state(const cpf::Program* prog, cpf::KParams<R>& p, void* blk, s
 // Largest number of input columns k of the isometry kernel: a sample is k lane groups of 2^(n-RB) threads in one CTA.
 constexpr int ISO_MAX_K = 32;
 
-// k input columns; the ancilla qubits as amplitude-index bits (qubit q is bit n - 1 - q, big-endian)
-struct IsoSpec { int k, amask; };
+// k input columns (lane groups of the isometry kernel); the ancilla qubits as amplitude-index bits (qubit q is bit
+// n - 1 - q, big-endian); the subspace kinds' caller k (0 for the isometry kinds), of which k is the next power of two
+struct IsoSpec { int k, amask, sub_k; };
 IsoSpec iso_spec(const cpf::Program* prog, int32_t mask) {
   const int n = prog->n_qubits;
-  IsoSpec s{1 << (n - __builtin_popcount((unsigned)mask)), 0};
+  IsoSpec s{1 << (n - __builtin_popcount((unsigned)mask)), 0, 0};
   for (int q = 0; q < n; ++q)
     if ((mask >> q) & 1) s.amask |= 1 << (n - 1 - q);
   return s;
@@ -272,8 +273,10 @@ struct CallPlan {
   bool single;          // single-column kernels (state loss, isometry kernel)
   bool iso_as_hs;       // n <= 5 isometry: the HS call on V = 2^a [W at the columns s_c, 0 elsewhere] (iso_impl.cuh:
                         // pack_iso_hs_kernel), built in BLK_V
+  bool sub_as_hs;       // n <= 5 subspace loss (one global phase): the HS call on V = (N/k) B A^dag (iso_impl.cuh:
+                        // pack_subspace_hs_kernel), built in BLK_V
   int32_t kind;         // the loss the kernel sees
-  IsoSpec iso;          // isometry kinds (CPF_LOSS_ISOMETRY, CPF_LOSS_ISOMETRY_RELPHASE)
+  IsoSpec iso;          // isometry and subspace kinds (the subspace kinds: k = k', the padded group count)
   int n_stage;          // ROUTE_HEIS: SWP::NSTAGE of the kernel chosen
   int cpt, words;       // not ROUTE_ISO: columns per thread and words of one packed target
   size_t heis_aux;      // ROUTE_HEIS: per-gate scratch at the start of BLK_HEIS (the packed state follows, 256-byte aligned)
@@ -295,18 +298,34 @@ int plan_call(const cpf::Program* prog, int32_t kind, int32_t mask, int64_t batc
               const cpf_penalty_spec* pen, CallPlan<R>* pl) {
   const int n = prog->n_qubits;
   *pl = CallPlan<R>();
-  const bool phases = kind == CPF_LOSS_ISOMETRY_RELPHASE;
-  if ((kind < CPF_LOSS_HS || kind > CPF_LOSS_ISOMETRY) && !phases) return fail(CPF_ERR_INVALID, "unknown loss kind");
+  const bool sub = kind == CPF_LOSS_SUBSPACE || kind == CPF_LOSS_SUBSPACE_RELPHASE;
+  const bool phases = kind == CPF_LOSS_ISOMETRY_RELPHASE || kind == CPF_LOSS_SUBSPACE_RELPHASE;
+  if ((kind < CPF_LOSS_HS || kind > CPF_LOSS_ISOMETRY) && !phases && !sub)
+    return fail(CPF_ERR_INVALID, "unknown loss kind");
   if (table && kind == CPF_LOSS_ISOMETRY)
     return fail(CPF_ERR_UNSUPPORTED, "multi-target tables do not take the isometry loss (one target per call)");
-  if (table && phases)
+  if (table && kind == CPF_LOSS_ISOMETRY_RELPHASE)
     return fail(CPF_ERR_UNSUPPORTED,
                 "multi-target tables do not take the relative-phase isometry loss (one target per call)");
+  if (table && sub)
+    return fail(CPF_ERR_UNSUPPORTED, "multi-target tables do not take the subspace losses (one target per call)");
   if (table && table->n_targets < 1) return fail(CPF_ERR_INVALID, "target table: n_targets must be >= 1");
   // HS, relative phase and an isometry without ancillas run on the full-unitary kernels, which stop at 5 qubits.  The
   // relative-phase isometry loss runs on the isometry kernel on every n, so only its k is limited (k <= 32 always
   // holds on n <= 5).
-  if (kind == CPF_LOSS_ISOMETRY || phases) {
+  if (sub) {
+    // ancilla_mask carries k; the isometry kernel runs k' = the next power of two groups
+    const int N = 1 << n;
+    if (mask < 1 || mask > N)
+      return fail(CPF_ERR_INVALID, "subspace losses take 1 <= k <= N = " + std::to_string(N) + " input states (k = " +
+                                       std::to_string(mask) + ")");
+    if (mask > ISO_MAX_K)
+      return fail(CPF_ERR_UNSUPPORTED, "subspace losses take at most k = " + std::to_string(ISO_MAX_K) +
+                                       " input states (k = " + std::to_string(mask) + ")");
+    int kp = 1;
+    while (kp < mask) kp <<= 1;
+    pl->iso = IsoSpec{kp, 0, mask};
+  } else if (kind == CPF_LOSS_ISOMETRY || phases) {
     if (mask < 0 || (mask >> n) != 0)
       return fail(CPF_ERR_INVALID, "ancilla_mask " + std::to_string(mask) + " names a qubit >= n = " + std::to_string(n));
     if (n > 5 && mask == 0 && !phases) return fail(CPF_ERR_UNSUPPORTED, cpf::FULL_UNITARY_LIMIT);
@@ -328,8 +347,10 @@ int plan_call(const cpf::Program* prog, int32_t kind, int32_t mask, int64_t batc
 
   pl->multi = table != nullptr;
   pl->iso_as_hs = kind == CPF_LOSS_ISOMETRY && n <= 5;
-  pl->kind = pl->iso_as_hs ? CPF_LOSS_HS : kind;
-  pl->single = pl->kind == CPF_LOSS_STATE || pl->kind == CPF_LOSS_ISOMETRY || phases;
+  pl->sub_as_hs = kind == CPF_LOSS_SUBSPACE && n <= 5;
+  pl->kind = pl->iso_as_hs || pl->sub_as_hs ? CPF_LOSS_HS : kind;
+  const bool iso_route = pl->kind == CPF_LOSS_ISOMETRY || phases || pl->kind == CPF_LOSS_SUBSPACE;
+  pl->single = pl->kind == CPF_LOSS_STATE || iso_route;
   pl->layered = layered_kernels(prog);
   // The Heisenberg-picture kernel keeps parameter and slot indices in 16 bits of shared memory (heis_impl.cuh: HSu2,
   // HCp) and B * P below 2^32.  CPF_ENGINE=adjoint forces the state-adjoint kernels (tests cover both engines).
@@ -343,13 +364,14 @@ int plan_call(const cpf::Program* prog, int32_t kind, int32_t mask, int64_t batc
     int rc = 0;
     heis = cpf::launch_heis<R>(dummy, *prog, nullptr, err, rc, true, &pl->n_stage);
   }
-  pl->route = pl->kind == CPF_LOSS_ISOMETRY || phases ? ROUTE_ISO : heis ? ROUTE_HEIS : ROUTE_ADJOINT;
+  pl->route = iso_route ? ROUTE_ISO : heis ? ROUTE_HEIS : ROUTE_ADJOINT;
 
   pl->bytes[BLK_MASK] = prog->cp.empty() ? 1 : prog->cp.size();
   pl->pen_mask = pl->pen.kind != CPF_PEN_NONE && pen->cp_mask && !prog->cp.empty();
-  if (pl->iso_as_hs) pl->bytes[BLK_V] = ((size_t)2 << (2 * n)) * sizeof(R);
+  if (pl->iso_as_hs || pl->sub_as_hs) pl->bytes[BLK_V] = ((size_t)2 << (2 * n)) * sizeof(R);
   if (pl->route == ROUTE_ISO) {
-    pl->bytes[BLK_TARGET] = ((size_t)pl->iso.k << (n + 1)) * sizeof(R);      // W packed column by column
+    // W packed column by column; the subspace kinds: B and then A, each packed to k' columns
+    pl->bytes[BLK_TARGET] = ((size_t)pl->iso.k << (n + 1)) * sizeof(R) * (sub ? 2 : 1);
     return CPF_OK;
   }
   pl->cpt = heis ? cpf::heis_cpt<R>(n) : pl->single ? 1 : cpf::cpt_for<R>(n);
@@ -428,6 +450,10 @@ int run_staged(const cpf::Program* prog, const CallPlan<R>& pl, const void* targ
     rc = cpf::launch_pack_iso<R>((const R*)target, (R*)blk[BLK_V], n, pl.iso.k, pl.iso.amask, true, st);
     if (rc) return fail(rc, "pack_iso launch failed");
     target = blk[BLK_V];
+  } else if (pl.sub_as_hs) {
+    rc = cpf::launch_pack_subspace_hs<R>((const R*)target, (R*)blk[BLK_V], n, pl.iso.sub_k, st);
+    if (rc) return fail(rc, "pack_subspace_hs launch failed");
+    target = blk[BLK_V];
   }
   R* packed = (R*)blk[BLK_TARGET];
   p.target_packed = packed;
@@ -441,6 +467,17 @@ int run_staged(const cpf::Program* prog, const CallPlan<R>& pl, const void* targ
              : cpf::launch_pack_targets<R>((const R*)target, packed, n, pl.cpt, pl.single, table->n_targets, st);
     if (rc) return fail(rc, "pack_targets launch failed");
     p.target_index = (const int32_t*)blk[BLK_INDEX];
+  } else if (pl.route == ROUTE_ISO && pl.iso.sub_k) {
+    // B and A, each packed column by column to k' columns; the k' - k padding columns are zero
+    const int k = pl.iso.sub_k, kp = pl.iso.k;
+    const size_t col = (size_t)2 << n;                // reals per packed column
+    if (k != kp) CPF_CUDA(cudaMemsetAsync(packed, 0, pl.bytes[BLK_TARGET], st));
+    rc = cpf::launch_pack_iso<R>((const R*)target, packed, n, k, 0, false, st);
+    if (!rc) rc = cpf::launch_pack_iso<R>((const R*)target + col * k, packed + col * kp, n, k, 0, false, st);
+    if (rc) return fail(rc, "pack_iso launch failed");
+    p.iso_k = kp;
+    p.inputs_packed = packed + col * kp;
+    p.sub_k = k;
   } else if (pl.route == ROUTE_ISO) {
     rc = cpf::launch_pack_iso<R>((const R*)target, packed, n, pl.iso.k, pl.iso.amask, false, st);
     if (rc) return fail(rc, "pack_iso launch failed");
@@ -468,7 +505,9 @@ int run_staged(const cpf::Program* prog, const CallPlan<R>& pl, const void* targ
   std::string err;
   if (pl.route == ROUTE_ISO) {
     rc = pl.kind == CPF_LOSS_ISOMETRY_RELPHASE ? cpf::launch_iso_phase<R>(p, n, st, err)
-                                               : cpf::launch_iso<R>(p, n, st, err);
+         : pl.kind == CPF_LOSS_SUBSPACE        ? cpf::launch_sub<R>(p, n, st, err)
+         : pl.kind == CPF_LOSS_SUBSPACE_RELPHASE ? cpf::launch_sub_phase<R>(p, n, st, err)
+                                                 : cpf::launch_iso<R>(p, n, st, err);
   } else if (pl.route == ROUTE_HEIS) {
     if (!(pl.multi ? cpf::launch_heis_multi<R>(p, *prog, st, err, rc) : cpf::launch_heis<R>(p, *prog, st, err, rc, false))) {
       rc = CPF_ERR_UNSUPPORTED;
@@ -584,12 +623,15 @@ int run_adam(const cpf::Program* prog, int32_t kind, int32_t mask, const void* t
 }
 
 // The plan behind a query entry point's loss-kind argument: an isometry kind carries its ancilla mask in bits 8-15
-// (CPF_ISOMETRY_KIND, CPF_ISOMETRY_RELPHASE_KIND); any other use of bits 8-31 makes an unknown kind.
+// (CPF_ISOMETRY_KIND, CPF_ISOMETRY_RELPHASE_KIND), a subspace kind its k (CPF_SUBSPACE_KIND,
+// CPF_SUBSPACE_RELPHASE_KIND); any other use of bits 8-31 makes an unknown kind.
 template <typename R>
 int plan_query(const cpf::Program* prog, int32_t arg, int64_t batch, CallPlan<R>* pl) {
   const int32_t base = arg & ~0xff00;
-  const int32_t kind =
-      base == CPF_LOSS_ISOMETRY || base == CPF_LOSS_ISOMETRY_RELPHASE || (arg >> 8) == 0 ? arg & 0xff : -1;
+  const int32_t kind = base == CPF_LOSS_ISOMETRY || base == CPF_LOSS_ISOMETRY_RELPHASE || base == CPF_LOSS_SUBSPACE ||
+                               base == CPF_LOSS_SUBSPACE_RELPHASE || (arg >> 8) == 0
+                           ? arg & 0xff
+                           : -1;
   return plan_call<R>(prog, kind, (arg >> 8) & 0xff, batch, nullptr, nullptr, pl);
 }
 
@@ -836,6 +878,13 @@ template <typename R>
 static int workspace_t(const cpf::Program* prog, int32_t loss_kind, int64_t batch, const cpf_target_table* table,
                        int64_t* bytes) {
   CallPlan<R> pl;
+  // cpf_workspace_bytes_multi is a query entry point too: a subspace kind carries its k in bits 8-15 there, and a k
+  // out of range (a bare kind 6 or 7 is k = 0) is refused as in cpf_workspace_bytes before the table is
+  const int32_t base = loss_kind & ~0xff00;
+  if (table && (base == CPF_LOSS_SUBSPACE || base == CPF_LOSS_SUBSPACE_RELPHASE)) {
+    if (int rc = plan_query<R>(prog, loss_kind, batch, &pl)) return rc;
+    loss_kind = base;
+  }
   const int rc = table ? plan_call<R>(prog, loss_kind, 0, batch, table, nullptr, &pl)
                        : plan_query<R>(prog, loss_kind, batch, &pl);
   if (!rc) *bytes = pl.workspace();
@@ -890,7 +939,8 @@ static int eval_cost_t(const cpf::Program* p, int32_t loss_kind, double* flops, 
   CallPlan<R> pl;
   if (int rc = plan_query<R>(p, loss_kind, 1, &pl)) return rc;
   const double N = (double)(1 << p->n_qubits);
-  const double C = pl.kind == CPF_LOSS_STATE ? 1.0 : pl.iso.k ? (double)pl.iso.k : N;     // isometry kinds: C = k
+  // isometry kinds: C = k; subspace kinds: C = the caller's k on either route
+  const double C = pl.kind == CPF_LOSS_STATE ? 1.0 : pl.iso.sub_k ? (double)pl.iso.sub_k : pl.iso.k ? (double)pl.iso.k : N;
   const double rs = (double)sizeof(R);
   if (flops) *flops = C * N * (16.0 * p->n_rot + 4.0 * p->n_phase + 8.0);
   if (bytes) *bytes = 6.0 * p->n_params * rs + 2.0 * rs;
@@ -916,7 +966,9 @@ static int executed_cost_t(const cpf::Program* p, int32_t loss_kind, double* flo
     // state-adjoint kernels: the credited count plus the uncompute of phi (6 flop per amplitude and rotation on
     // fused gates, 1.5 per phase gate), with fused gates instead of primitive rotations: C N (22 G + 5.5 K + 8);
     // an isometry runs as an HS call on n <= 5 and on the isometry kernel with C = k on n >= 6, the relative-phase
-    // isometry on the isometry kernel on every n
+    // isometry on the isometry kernel on every n.  The subspace losses: C = N on the HS route, and on the isometry kernel
+    // C = k', the padded group count, not the caller's k: the zero groups run full sweeps too, and this entry point
+    // counts executed work (cpf_eval_cost credits C = k)
     const double C = pl.kind == CPF_LOSS_STATE ? 1.0 : pl.route == ROUTE_ISO ? (double)pl.iso.k : N;
     *flops = C * N * (22.0 * G + 5.5 * K + 8.0) + 232.0 * G + 80.0 * K;
   }

@@ -81,6 +81,10 @@ struct KParams {
   const int32_t* target_index;
   // isometry kernels (iso_impl.cuh): k input columns per sample, and the ancilla qubits as amplitude-index bits
   int iso_k, iso_amask;
+  // subspace kernels (iso_impl.cuh: sweep types with INPUTS): the input states packed like the target ([iso_k][N]
+  // complex, columns >= sub_k zero) and the caller's k, which normalises the loss.  Appended last, so the kernels
+  // without inputs keep their parameter layout.
+  const R* inputs_packed; int sub_k;
 };
 
 // ------------------------------------------------------------------------------------------

@@ -14,6 +14,11 @@
 //
 // The relative-phase isometry loss (InterpSweepIsoPhase, 2-8 qubits) runs the same kernel with one change: the loss is
 // 1 - sum_c |t_c|^2 / k, and each group seeds its adjoint with its own partial t_c (the HS seed with NN = k).
+//
+// The subspace losses (InterpSweepSub on 6-8 qubits, InterpSweepSubPhase on 2-8) run it with arbitrary input states:
+// group c starts its forward sweep from a_c (column c of the packed inputs) instead of e_{s_c}, and the target holds the
+// wanted images b_c.  A sample has k' = the next power of two >= k groups, so a CTA stays a whole number of warps; the
+// packed columns c >= k of both are zero, so those groups add exactly 0 to every sum, and the loss is normalised by k.
 #pragma once
 #include <string>
 
@@ -29,7 +34,8 @@ template <int NQ> constexpr int iso_rb() { return NQ == 8 ? 3 : 2; }
 template <int NQ> constexpr int iso_phase_rb() { return NQ == 8 ? 3 : NQ == 4 || NQ == 5 ? 1 : 2; }
 
 // The sweep of iso_kernel with RB_ register bits.  The kernels' sweep types derive from it; they only set RB_ and the
-// mode flags: ISOMETRY (always), COTANGENT (InterpSweepIsoCot) and PHASES (InterpSweepIsoPhase).
+// mode flags: ISOMETRY (always), COTANGENT (InterpSweepIsoCot), PHASES (InterpSweepIsoPhase) and INPUTS
+// (InterpSweepSub, InterpSweepSubPhase).
 template <typename R, int NQ, int RB_>
 struct InterpSweepIsoRB : InterpSweep<R, NQ, RB_, 1, true> {
   using Base = InterpSweep<R, NQ, RB_, 1, true>;
@@ -39,6 +45,7 @@ struct InterpSweepIsoRB : InterpSweep<R, NQ, RB_, 1, true> {
   static constexpr bool ISOMETRY = true;
   static constexpr bool COTANGENT = false;
   static constexpr bool PHASES = false;
+  static constexpr bool INPUTS = false;   // forward sweeps start from p.inputs_packed, not from basis states
   // InterpSweep::backward with the reduced sums stored at `sums` (this group's slots, reduce table re-pointed) instead
   // of over the coefficients, which the other groups of the sample may still be reading.
   static __device__ __forceinline__ void backward_into(const KParams<R>& p, const R* coef, R* sums, const uint2* s_dec,
@@ -134,6 +141,18 @@ struct InterpSweepIsoCot : InterpSweepIso<R, NQ> {
 template <typename R, int NQ>
 struct InterpSweepIsoPhase : InterpSweepIsoRB<R, NQ, iso_phase_rb<NQ>()> {
   static constexpr bool PHASES = true;
+};
+
+// The subspace loss (CPF_LOSS_SUBSPACE, one global phase) on 6-8 qubits: L = 1 - |sum_c <b_c| U |a_c>|^2 / k^2.
+template <typename R, int NQ>
+struct InterpSweepSub : InterpSweepIso<R, NQ> {
+  static constexpr bool INPUTS = true;
+};
+
+// The relative-phase subspace loss (CPF_LOSS_SUBSPACE_RELPHASE) on 2-8 qubits: L = 1 - sum_c |<b_c| U |a_c>|^2 / k.
+template <typename R, int NQ>
+struct InterpSweepSubPhase : InterpSweepIsoPhase<R, NQ> {
+  static constexpr bool INPUTS = true;
 };
 
 // words per group of the per-group gradient sums (odd: the groups of a sample store the same slot in distinct banks)
@@ -329,7 +348,8 @@ __global__ void __launch_bounds__(NQ <= 6 ? 512 : 1024, 1) iso_kernel(const KPar
   R* mom = p.m ? p.m + b * P : nullptr;
   R* vel = p.v ? p.v + b * P : nullptr;
   const uint8_t* frz = p.freeze ? p.freeze + b * P : nullptr;
-  const R NN = R(k) * R(k);
+  const R kn = SW::INPUTS ? R(p.sub_k) : R(k);     // the loss's k: the caller's, not the padded group count
+  const R NN = kn * kn;
 
   R best = R(0), best_reg_v = R(0);
   if (p.mode == M_ADAM && p.step0 > 0) { best = p.best_regloss[b]; best_reg_v = p.best_reg[b]; }
@@ -342,8 +362,15 @@ __global__ void __launch_bounds__(NQ <= 6 ? 512 : 1024, 1) iso_kernel(const KPar
     __syncthreads();
     if (it == p.nsteps) break;
     V pr[NA], pi[NA];
+    if constexpr (SW::INPUTS) {
+      // this group's amplitudes of a_grp (column-major packed, like the target)
+      const R* av = p.inputs_packed + 2 * ((size_t)grp * N + (la << RB));
 #pragma unroll
-    for (int r = 0; r < NA; ++r) { pr[r] = T::onehot((la << RB) | r, col0); pi[r] = T::bc(R(0)); }
+      for (int r = 0; r < NA; ++r) { pr[r] = T::bc(av[2 * r]); pi[r] = T::bc(av[2 * r + 1]); }
+    } else {
+#pragma unroll
+      for (int r = 0; r < NA; ++r) { pr[r] = T::onehot((la << RB) | r, col0); pi[r] = T::bc(R(0)); }
+    }
     SW::forward(p, coef, s_dec, la, pr, pi);
 
     if constexpr (SW::COTANGENT) {
@@ -383,7 +410,7 @@ __global__ void __launch_bounds__(NQ <= 6 ? 512 : 1024, 1) iso_kernel(const KPar
         s2 += xr * xr + xi * xi;
         reg += part[3 * c + 2];
       }
-      const R kk = R(k);
+      const R kk = kn;
       loss = R(1) - s2 / kk;
       const R tr_c = part[3 * grp], ti_c = part[3 * grp + 1];
       const V a = T::bc(-tr_c / kk), bq = T::bc(ti_c / kk), nb = T::bc(-ti_c / kk);
@@ -473,6 +500,28 @@ __global__ void pack_iso_hs_kernel(const R* __restrict__ src, R* __restrict__ ds
   }
 }
 
+// The n <= 5 subspace loss as an HS loss: V = (N/k) B A^dag (N x N; src = B then A, each N x k row-major), so
+// Tr(V^dag U) = (N/k) sum_c <b_c| U |a_c> and the HS kernels compute 1 - |sum_c t_c|^2 / k^2 and its gradient.  The sum
+// over c starts from +0, so with A = the basis columns e_{s_c} and a power-of-two k every entry is bit for bit the one
+// pack_iso_hs_kernel writes.
+template <typename R>
+__global__ void pack_subspace_hs_kernel(const R* __restrict__ src, R* __restrict__ dst, int N, int k) {
+  const R scale = R(N) / R(k);
+  const R* A = src + (size_t)2 * N * k;
+  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < N * N; i += gridDim.x * blockDim.x) {
+    const int j = i / N, s = i % N;
+    const R* b = src + (size_t)2 * j * k;
+    const R* a = A + (size_t)2 * s * k;
+    R re = R(0), im = R(0);
+    for (int c = 0; c < k; ++c) {           // b_c[j] conj(a_c[s])
+      re += b[2 * c] * a[2 * c] + b[2 * c + 1] * a[2 * c + 1];
+      im += b[2 * c + 1] * a[2 * c] - b[2 * c] * a[2 * c + 1];
+    }
+    dst[2 * i] = scale * re;
+    dst[2 * i + 1] = scale * im;
+  }
+}
+
 // grad[b, i] = sum over h of partial[b * n_chunks + h, i], in increasing h (the cotangent mode's chunk sum)
 template <typename R>
 __global__ void cot_reduce_kernel(const R* __restrict__ partial, R* __restrict__ grad, long long B, int P,
@@ -544,5 +593,11 @@ template <typename R> int launch_cot_reduce(const R* partial, R* grad, long long
                                             cudaStream_t st);
 template <typename R> int launch_pack_iso(const R* src, R* dst, int n_qubits, int k, int amask, bool as_hs,
                                           cudaStream_t st);
+// inst_sub_f32.cu / inst_sub_f64.cu: the subspace losses on the isometry kernel (p.iso_k = k' groups, p.sub_k = k),
+// CPF_LOSS_SUBSPACE on 6-8 qubits and CPF_LOSS_SUBSPACE_RELPHASE on 2-8
+template <typename R> int launch_sub(const KParams<R>& p, int n_qubits, cudaStream_t st, std::string& err);
+template <typename R> int launch_sub_phase(const KParams<R>& p, int n_qubits, cudaStream_t st, std::string& err);
+// V = (N/k) B A^dag into dst (N x N row-major) from src = B then A (pack_subspace_hs_kernel)
+template <typename R> int launch_pack_subspace_hs(const R* src, R* dst, int n_qubits, int k, cudaStream_t st);
 
 }  // namespace cpf

@@ -296,26 +296,41 @@ class Loss:
     'isometry_relphase' takes the same `ancillas` and W, and keeps a phase per input column:
     1 - sum_c |<W e_c| U |s_c>|^2 / k.  It is 0 exactly when U|s_c> = e^{i phi_c} W e_c for every c (relative-phase
     gates with clean ancillas, states each prepared up to its own phase, a unitary up to a diagonal on the input
-    side), and runs fused on 2-8 qubits with k <= 32."""
-    KINDS = {"hs": L.LOSS_HS, "state": L.LOSS_STATE, "relphase": L.LOSS_RELPHASE, "isometry": L.LOSS_ISOMETRY,
-             "isometry_relphase": L.LOSS_ISOMETRY_RELPHASE}
-    ISOMETRY_KINDS = ("isometry", "isometry_relphase")
+    side), and runs fused on 2-8 qubits with k <= 32.
 
-    def __init__(self, kind, target, ancillas=None):
+    'subspace' and 'subspace_relphase' take `inputs`, an N x k matrix A of input states a_c, and the target B, the
+    N x k matrix of their wanted images b_c, with 1 <= k <= min(N, 32) and unit-norm columns.  With t_c = <b_c| U |a_c>:
+    'subspace' is 1 - |sum_c t_c|^2 / k^2, 0 exactly when U a_c = e^{i phi} b_c for every c (one global phase: logical
+    gates on a code space, state-to-state maps), and 'subspace_relphase' is 1 - sum_c |t_c|^2 / k, 0 exactly when
+    U a_c = e^{i phi_c} b_c for every c.  Both run fused on 2-8 qubits."""
+    KINDS = {"hs": L.LOSS_HS, "state": L.LOSS_STATE, "relphase": L.LOSS_RELPHASE, "isometry": L.LOSS_ISOMETRY,
+             "isometry_relphase": L.LOSS_ISOMETRY_RELPHASE, "subspace": L.LOSS_SUBSPACE,
+             "subspace_relphase": L.LOSS_SUBSPACE_RELPHASE}
+    ISOMETRY_KINDS = ("isometry", "isometry_relphase")
+    SUBSPACE_KINDS = ("subspace", "subspace_relphase")
+
+    def __init__(self, kind, target, ancillas=None, inputs=None):
         if kind not in self.KINDS:
             raise ValueError(f"unknown loss kind {kind!r}")
         if ancillas is not None and kind not in self.ISOMETRY_KINDS:
             raise ValueError(f"ancillas are an argument of the 'isometry' loss, not of {kind!r}")
+        if inputs is not None and kind not in self.SUBSPACE_KINDS:
+            raise ValueError(f"inputs are an argument of the 'subspace' losses, not of {kind!r}")
         self.kind = kind
-        self.target = np.asarray(target.detach().cpu().numpy() if isinstance(target, torch.Tensor) else target,
-                                 dtype=np.complex128)
+        self.target = _host_complex(target)
         self.ancillas = ()
+        self.inputs = None
         if kind in self.ISOMETRY_KINDS:
             self.ancillas = _check_isometry(self.target, ancillas)
+        if kind in self.SUBSPACE_KINDS:
+            self.inputs = _check_subspace(kind, self.target, inputs)
         self._dev = {}
 
     @property
     def ancilla_mask(self):
+        """cpf_loss_spec.ancilla_mask: the ancilla qubits' bits (the isometry kinds) or k (the subspace kinds)."""
+        if self.kind in self.SUBSPACE_KINDS:
+            return self.target.shape[1]
         return sum(1 << q for q in self.ancillas)
 
     @property
@@ -333,20 +348,27 @@ class Loss:
             return L.isometry_kind(self.ancilla_mask)
         if self.kind == "isometry_relphase":
             return L.isometry_relphase_kind(self.ancilla_mask)
+        if self.kind == "subspace":
+            return L.subspace_kind(self.ancilla_mask)
+        if self.kind == "subspace_relphase":
+            return L.subspace_relphase_kind(self.ancilla_mask)
         return self.KINDS[self.kind]
 
     def spec(self, dtype, device):
         key = (dtype, str(device))
         if key not in self._dev:
-            self._dev[key] = torch.as_tensor(self.target, dtype=_CDT[dtype]).contiguous().to(device)
+            # the subspace kinds: B and then A (each N x k row-major) in one buffer
+            host = self.target if self.inputs is None else np.concatenate([self.target.ravel(), self.inputs.ravel()])
+            self._dev[key] = torch.as_tensor(host, dtype=_CDT[dtype]).contiguous().to(device)
         return L.CpfLossSpec(self.KINDS[self.kind], self._dev[key].data_ptr(), self.ancilla_mask)
 
     def __getstate__(self):
-        return {"kind": self.kind, "target": self.target, "ancillas": self.ancillas}
+        return {"kind": self.kind, "target": self.target, "ancillas": self.ancillas, "inputs": self.inputs}
 
     def __setstate__(self, st):
         self.kind, self.target, self._dev = st["kind"], st["target"], {}
         self.ancillas = tuple(st.get("ancillas", ()))
+        self.inputs = st.get("inputs")
 
     def __call__(self, u):
         """Value of the loss at an explicit unitary `u` (host utility with the formulas of
@@ -364,12 +386,46 @@ class Loss:
         if self.kind == "isometry_relphase":
             t = (self.target.conj() * u[:, list(self.columns)]).sum(0)
             return float(1 - (np.abs(t) ** 2).sum() / self.target.shape[1])
+        if self.kind in self.SUBSPACE_KINDS:
+            k = self.target.shape[1]
+            t = (self.target.conj() * (u @ self.inputs)).sum(0)          # t_c = <b_c| U |a_c>
+            if self.kind == "subspace":
+                return float(1 - np.abs(t.sum()) ** 2 / k ** 2)
+            return float(1 - (np.abs(t) ** 2).sum() / k)
         return float(1 - (np.abs(self.target.conj() * u) ** 2).sum() / n)
 
     def __repr__(self):
         if self.kind in self.ISOMETRY_KINDS:
             return f"Loss({self.kind!r}, target{tuple(self.target.shape)}, ancillas={list(self.ancillas)})"
+        if self.kind in self.SUBSPACE_KINDS:
+            return f"Loss({self.kind!r}, target{tuple(self.target.shape)}, inputs{tuple(self.inputs.shape)})"
         return f"Loss({self.kind!r}, target{tuple(self.target.shape)})"
+
+
+def _host_complex(x):
+    return np.asarray(x.detach().cpu().numpy() if isinstance(x, torch.Tensor) else x, dtype=np.complex128)
+
+
+def _check_subspace(kind, B, inputs):
+    """Checks of a subspace loss: B (target) and A (inputs) are both N x k with N = 2^n, n >= 1, and
+    1 <= k <= min(N, 32), and every column of both has unit norm.  Returns A as a complex128 array."""
+    if inputs is None:
+        raise ValueError(f"the {kind!r} loss needs `inputs` (the N x k matrix of input states)")
+    A = _host_complex(inputs)
+    if B.ndim != 2 or B.shape[0] < 2 or B.shape[0] & (B.shape[0] - 1):
+        raise ValueError(f"a {kind!r} target is N x k with N = 2^n rows, got shape {B.shape}")
+    if A.shape != B.shape:
+        raise ValueError(f"{kind!r}: inputs and target must have the same shape N x k, got {A.shape} and {B.shape}")
+    N, k = B.shape
+    if not 1 <= k <= min(N, 32):
+        raise ValueError(f"{kind!r} takes 1 <= k <= min(N, 32) = {min(N, 32)} columns, got k = {k}")
+    for name, M in (("target", B), ("inputs", A)):
+        norms = np.linalg.norm(M, axis=0)
+        bad = np.flatnonzero(np.abs(norms - 1) > 1e-6)
+        if bad.size:
+            raise ValueError(f"{kind!r}: column {int(bad[0])} of {name} has norm {norms[bad[0]]:.6g}; the columns "
+                             "must be unit vectors")
+    return A
 
 
 def _check_isometry(W, ancillas):
@@ -416,6 +472,8 @@ class MultiLoss:
     def __init__(self, kind, targets):
         if kind not in Loss.KINDS:
             raise ValueError(f"unknown loss kind {kind!r}")
+        if kind in Loss.SUBSPACE_KINDS:
+            raise ValueError(f"MultiLoss does not take the {kind!r} loss (one target per call)")
         t = np.asarray(targets.detach().cpu().numpy() if isinstance(targets, torch.Tensor) else targets,
                        dtype=np.complex128)
         want = 2 if kind == "state" else 3

@@ -59,6 +59,13 @@ def batched_unitary_loss(unitary_loss_func, U):
             k = tgt.shape[1]
             t = (tgt.conj() * U[:, :, list(unitary_loss_func.columns)]).sum(-2)
             return (1 - (t.abs() ** 2).sum(-1) / k).cpu().numpy()
+        if unitary_loss_func.kind in ('subspace', 'subspace_relphase'):
+            A = torch.as_tensor(unitary_loss_func.inputs).to(U.device, U.dtype)
+            k = tgt.shape[1]
+            t = (tgt.conj() * (U @ A)).sum(-2)                          # [B, k]: t_c = <b_c| U |a_c>
+            if unitary_loss_func.kind == 'subspace':
+                return (1 - t.sum(-1).abs() ** 2 / k ** 2).cpu().numpy()
+            return (1 - (t.abs() ** 2).sum(-1) / k).cpu().numpy()
         return (1 - ((tgt.conj() * U).abs() ** 2).sum((-1, -2)) / n).cpu().numpy()
     if isinstance(unitary_loss_func, TorchLoss):
         with torch.no_grad():

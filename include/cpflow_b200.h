@@ -83,7 +83,9 @@ typedef enum cpf_loss_kind {
   CPF_LOSS_STATE = 1,    /* 1 - |<psi| U |0>|^2                    tutorial ipynb:1318    */
   CPF_LOSS_RELPHASE = 2, /* 1 - sum_ij |conj(V_ij) U_ij|^2 / N     tutorial ipynb:1507    */
   CPF_LOSS_ISOMETRY = 3, /* 1 - |sum_c <W e_c| U |s_c>|^2 / k^2     (ancilla qubits start in |0>) */
-  CPF_LOSS_ISOMETRY_RELPHASE = 5 /* 1 - sum_c |<W e_c| U |s_c>|^2 / k  (ancillas in |0>, a phase per column) */
+  CPF_LOSS_ISOMETRY_RELPHASE = 5, /* 1 - sum_c |<W e_c| U |s_c>|^2 / k  (ancillas in |0>, a phase per column) */
+  CPF_LOSS_SUBSPACE = 6,         /* 1 - |sum_c <b_c| U |a_c>|^2 / k^2   (k given input states, one global phase) */
+  CPF_LOSS_SUBSPACE_RELPHASE = 7 /* 1 - sum_c |<b_c| U |a_c>|^2 / k     (k given input states, a phase per pair) */
 } cpf_loss_kind;
 
 /* ISOMETRY: the qubits of `ancilla_mask` (bit q = qubit q) start in |0>, so only the images of the k = 2^(n - popcount)
@@ -100,19 +102,38 @@ typedef enum cpf_loss_kind {
  * ancilla_mask = 0 with a W of one unit-modulus entry per column is the RELPHASE loss; k = 1 is the state loss.  Runs
  * on the isometry kernel on 2-8 qubits (group c seeds its adjoint with its own t_c / k), with k <= 32 on every n:
  * k > 32 (ancilla_mask = 0 on 6-8 qubits included) is CPF_ERR_UNSUPPORTED, as are multi-target tables; a mask bit
- * at a position >= n is CPF_ERR_INVALID.  (The value 5 leaves 4 unassigned.) */
+ * at a position >= n is CPF_ERR_INVALID.  (The value 5 leaves 4 unassigned.)
+ *
+ * SUBSPACE and SUBSPACE_RELPHASE: arbitrary input states.  `target` holds B (N x k, row-major: column c = the wanted
+ * image b_c) immediately followed by A (N x k, row-major: column c = the input state a_c), 2 N k complex values of the
+ * call's dtype, and `ancilla_mask` carries k, with 1 <= k <= min(N, 32).  With t_c = <b_c| U |a_c>:
+ *   SUBSPACE          L = 1 - |sum_c t_c|^2 / k^2, 0 exactly when U a_c = e^{i phi} b_c for every c (one global phase);
+ *                     invariant under (A, B) -> (A Q, B Q) for a k x k unitary Q.
+ *   SUBSPACE_RELPHASE L = 1 - (1/k) sum_c |t_c|^2, 0 exactly when U a_c = e^{i phi_c} b_c for every c; invariant
+ *                     under B -> B D for a diagonal phase matrix D.
+ * The columns are assumed to have unit norm (not checked here).  With A = the isometry's basis columns e_{s_c} they
+ * are the ISOMETRY and ISOMETRY_RELPHASE losses.  SUBSPACE on n <= 5 runs on the HS kernels with the target
+ * V = (N/k) B A^dag (Tr(V^dag U) = (N/k) sum_c t_c); SUBSPACE on 6-8 qubits and SUBSPACE_RELPHASE on 2-8 qubits run on
+ * the isometry kernel, group c starting its forward sweep from a_c, with k rounded up to a power of two k' (the
+ * columns c >= k are zero and add exactly 0).  k < 1 or k > N is CPF_ERR_INVALID, 32 < k <= N CPF_ERR_UNSUPPORTED.
+ * Multi-target tables do not take them (CPF_ERR_UNSUPPORTED, one target per call); cpf_workspace_bytes_multi reads
+ * its loss kind as the other query entry points do, so a subspace kind with a k out of range there (a bare 6 or 7 is
+ * k = 0) is CPF_ERR_INVALID first. */
 typedef struct cpf_loss_spec {
   int32_t kind;       /* cpf_loss_kind */
   const void* target; /* device: N*N complex row-major (HS, RELPHASE), N complex (STATE), N*k row-major (ISOMETRY,
-                         ISOMETRY_RELPHASE) */
-  int32_t ancilla_mask; /* ISOMETRY and ISOMETRY_RELPHASE only (ignored for the other kinds) */
+                         ISOMETRY_RELPHASE), B then A, each N*k row-major (SUBSPACE, SUBSPACE_RELPHASE) */
+  int32_t ancilla_mask; /* ISOMETRY and ISOMETRY_RELPHASE: the ancilla mask; SUBSPACE and SUBSPACE_RELPHASE: k
+                           (ignored for the other kinds) */
 } cpf_loss_spec;
 
 /* cpf_workspace_bytes, cpf_eval_cost, cpf_executed_cost and cpf_launch_plan take a loss kind only: for the isometry
  * losses pass CPF_ISOMETRY_KIND(ancilla_mask) or CPF_ISOMETRY_RELPHASE_KIND(ancilla_mask), which carry the mask in
- * bits 8-15. */
+ * bits 8-15, and for the subspace losses CPF_SUBSPACE_KIND(k) or CPF_SUBSPACE_RELPHASE_KIND(k), which carry k there. */
 #define CPF_ISOMETRY_KIND(ancilla_mask) ((int32_t)CPF_LOSS_ISOMETRY | ((int32_t)(ancilla_mask) << 8))
 #define CPF_ISOMETRY_RELPHASE_KIND(ancilla_mask) ((int32_t)CPF_LOSS_ISOMETRY_RELPHASE | ((int32_t)(ancilla_mask) << 8))
+#define CPF_SUBSPACE_KIND(k) ((int32_t)CPF_LOSS_SUBSPACE | ((int32_t)(k) << 8))
+#define CPF_SUBSPACE_RELPHASE_KIND(k) ((int32_t)CPF_LOSS_SUBSPACE_RELPHASE | ((int32_t)(k) << 8))
 
 typedef enum cpf_penalty_kind {
   CPF_PEN_NONE = 0,
@@ -290,7 +311,7 @@ int cpf_initial_angles(const cpf_program* prog, int32_t dtype, uint64_t seed,
 
 /* Algorithmic work of one loss+grad evaluation, SURVEY.md §8(d):
  * flops = C*N*(16*G1 + 4*K + 8), bytes = 6*P*sizeof(real) + 2*sizeof(real); C = N columns (HS, RELPHASE), 1 (STATE),
- * k (ISOMETRY, ISOMETRY_RELPHASE). */
+ * k (ISOMETRY, ISOMETRY_RELPHASE, SUBSPACE, SUBSPACE_RELPHASE). */
 int cpf_eval_cost(const cpf_program* prog, int32_t loss_kind, int32_t dtype, double* flops,
                   double* bytes);
 
